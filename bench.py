@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- element-assembly throughput of libpetiga_cuda on BASELINE.json's headline configuration.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--path auto|quadrature] [--mesh 128]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--path auto|quadrature] [--mesh 128] [--dump-outputs DIR]
 
 Workload (config.workload): demo/Poisson3D of the reference, p=3 C2, 128^3 elements, dof=1, AIJ, Dirichlet 1.0 on
 all six faces, one `IGAComputeSystem` per step (zero -> integrate -> fix-up -> scatter -> fully assembled).
@@ -11,6 +11,11 @@ beside it.  N > 1 (torchrun, one rank per GPU): the same global mesh split by th
 
 --impl reference times the CPU restatement of the reference's assembly (oracle/, "port": the reference needs
 PETSc+MPI+gfortran and cannot be built here) on all host cores, one emulated MPI rank per core.
+
+--dump-outputs DIR (one process) writes what the last timed step computed, so that two builds can be compared output for
+output on identical inputs: DIR/rhs.npy + rhs_index.npy (right-hand side at a fixed seeded sample of 2^21 positions, all of
+them when it is shorter) and DIR/matrix_values.npy + matrix_rows.npy + matrix_cols.npy (2^20 sampled nonzeros of the
+assembled matrix with their row and column), all float64: 56 MiB at most.
 """
 import argparse
 import json
@@ -151,10 +156,16 @@ def main():
     ap.add_argument("--no-solve", action="store_true", help="skip the assemble + device CG solve figure (e2e_solve)")
     ap.add_argument("--no-parity", action="store_true", help="skip the golden-vector parity cases run before the timed region")
     ap.add_argument("--no-configs", action="store_true", help="skip the secondary BASELINE configurations (N=1 only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the last timed step's matrix and right-hand side "
+                                                           "as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the outputs of the GPU path, not of --impl reference")
         return main_reference(args)
 
     import ctypes as C
@@ -167,6 +178,8 @@ def main():
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: libpetiga_cuda has no CPU fallback")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes the outputs of one process: run it with --gpus 1")
     torch.cuda.set_device(local)
     L = pb.load_cuda()
     nccl = None
@@ -262,12 +275,16 @@ def main():
         g.SetOption("async", 0)
         ms = e0.elapsed_time(e1) / args.steps
         launches = int(g.GetStat("launches") - l0)
+        snapshot = snapshot_outputs(g, A, B) if args.dump_outputs else None     # before the calls below overwrite A and B
         if t1 - t0 < 1.0:      # too short for nvidia-smi to see: keep the same kernel busy ~1.5 s for the clock record only
             tend = time.time() + 1.5
             while time.time() < tend:
                 g.ComputeSystem(A, B)
             t1 = time.time()
         clocks = sampler.stop(t0, t1)
+    if snapshot is not None:
+        write_outputs(args.dump_outputs, snapshot)
+        snapshot = None
 
     # -------- the per-element quadrature path on the same workload (reported beside the headline, not as it) --------
     quad = None
@@ -562,6 +579,55 @@ def _bc_struct(case):
         bc.vvalue[a][s][k] = v
         bc.vcount[a][s] = k + 1
     return bc
+
+
+DUMP_SEED = 20261017
+DUMP_MATRIX_ENTRIES, DUMP_RHS_ENTRIES = 1 << 20, 1 << 21      # 3 x 8 MiB + 2 x 16 MiB of float64
+
+
+def _sample(n, k):
+    """Sorted positions of a fixed seeded sample of k of n entries (all of them when n <= k)."""
+    import numpy as np
+    if n <= k:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=k, replace=False))
+
+
+def _device_array(ptr, n, typestr):
+    """Zero-copy torch view of n elements of device memory owned by libpetiga_cuda."""
+    import types
+    import torch
+    cai = {"shape": (n,), "typestr": typestr, "data": (ptr, False), "version": 2}
+    return torch.as_tensor(types.SimpleNamespace(__cuda_array_interface__=cai), device="cuda")
+
+
+def snapshot_outputs(g, A, B):
+    """Device copies of a seeded sample of what the last ComputeSystem left in A and B: right-hand side entries with their
+    positions, matrix values with their row and column (the AIJ pattern of IGACreateMat)."""
+    import ctypes as C
+    import torch
+    import petiga_b200 as pb
+    g.Synchronize()
+    L = pb.load_cuda()
+    L.petiga_cuda_plan_pattern.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 4
+    nrows, nnz, rp, ci = C.c_int(), C.c_int64(), C.c_void_p(), C.c_void_p()
+    assert L.petiga_cuda_plan_pattern(g.plan(), 0, C.byref(nrows), C.byref(nnz), C.byref(rp), C.byref(ci)) == 0, L.petiga_cuda_last_error()
+    assert not A.baij and nnz.value == A.nnz
+    pos = torch.from_numpy(_sample(A.nnz, DUMP_MATRIX_ENTRIES)).cuda()
+    rowptr = _device_array(rp.value, nrows.value + 1, "<i4").long()
+    idx = torch.from_numpy(_sample(B.size, DUMP_RHS_ENTRIES)).cuda()
+    return {"matrix_values": _device_array(A.device_ptr(), A.nnz, "<f8")[pos],
+            "matrix_rows": torch.searchsorted(rowptr, pos, right=True) - 1,
+            "matrix_cols": _device_array(ci.value, A.nnz, "<i4")[pos],
+            "rhs": _device_array(B.device_ptr(), B.size, "<f8")[idx], "rhs_index": idx}
+
+
+def write_outputs(out_dir, snapshot):
+    """DIR/<name>.npy, float64 throughout (row, column and position indices are exact in it)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in snapshot.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy().astype(np.float64))
 
 
 if __name__ == "__main__":

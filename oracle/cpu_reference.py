@@ -5,7 +5,7 @@ gfortran, none of which exist in the image) run the way `mpiexec -n T` runs PetI
 box partition, one host thread each (ctypes releases the GIL), every rank looping over its element box
 (src/petigaksp.c:149-202), adding the rows it owns straight into the global CSR and the rows of other ranks into its stash;
 then the receiving side of MatAssemblyEnd/VecAssemblyEnd adds the stashes (src/petigaksp.c:197-200).  The library is
-rebuilt with -march=native on the box it runs on (oracle.build(native=True) tags the binary with the CPU)."""
+rebuilt with -march=native on the box it runs on (oracle.build(native=True), in a temporary directory)."""
 import os
 import threading
 import time

@@ -5,7 +5,9 @@ The product package petiga_b200 never does.
 """
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -24,24 +26,6 @@ _dp = C.POINTER(C.c_double)
 _ip = C.POINTER(C.c_int)
 
 
-def _cpu_tag():
-    """Short hash of this host's CPU model + ISA flags: a -march=native binary is only valid on the CPU it was built for,
-    so the native library carries the tag in its name and is rebuilt on a box with a different CPU (VERDICT r1 weak #5)."""
-    import hashlib
-    model = flags = ""
-    try:
-        for line in open("/proc/cpuinfo"):
-            if line.startswith("model name") and not model:
-                model = line.split(":", 1)[1].strip()
-            elif line.startswith("flags") and not flags:
-                flags = line.split(":", 1)[1].strip()
-            if model and flags:
-                break
-    except OSError:
-        pass
-    return hashlib.sha1((model + "|" + flags).encode()).hexdigest()[:8]
-
-
 def cpu_model():
     try:
         for line in open("/proc/cpuinfo"):
@@ -53,17 +37,25 @@ def cpu_model():
 
 
 def build(native=False):
-    """Compile the oracle with gcc (a few seconds; mtime-guarded, so calling it every time is cheap).
-    native=True adds -march=native (CPU-baseline timing) and tags the file with the CPU it was built on."""
-    name = ("libpetiga_oracle_native_%s.so" % _cpu_tag()) if native else "libpetiga_oracle.so"
-    out = os.path.join(_HERE, name)
+    """Compile the oracle with gcc (a few seconds).  The portable library sits beside the source, mtime-guarded, so calling
+    this every time is cheap.  native=True adds -march=native (CPU-baseline timing): that binary is only valid on the CPU it
+    was built for and the tree may be read-only where the benchmark runs, so it goes to a fresh temporary directory."""
     src = os.path.join(_HERE, "petiga_oracle.c")
     hdr = os.path.join(_HERE, "gauss_tables.h")
+    if native:
+        tmpdir = tempfile.mkdtemp(prefix="petiga_oracle_")
+        out = os.path.join(tmpdir, "libpetiga_oracle_native.so")
+        try:
+            subprocess.check_call(["gcc", "-O2", "-march=native", "-fPIC", "-shared", "-o", out, src, "-lm"], cwd=_HERE)
+        except Exception:
+            shutil.rmtree(tmpdir)
+            raise
+        return out
+    out = os.path.join(_HERE, "libpetiga_oracle.so")
     if os.path.exists(out) and os.path.getmtime(out) >= max(os.path.getmtime(src), os.path.getmtime(hdr)):
         return out
-    march = "native" if native else "x86-64-v2"
     tmp = out + ".tmp%d" % os.getpid()      # several ranks / xdist workers may build at once: write aside, then rename
-    cmd = ["gcc", "-O2", "-march=" + march, "-fPIC", "-shared", "-o", tmp, src, "-lm"]
+    cmd = ["gcc", "-O2", "-march=x86-64-v2", "-fPIC", "-shared", "-o", tmp, src, "-lm"]
     subprocess.check_call(cmd, cwd=_HERE)
     os.replace(tmp, out)
     return out
@@ -85,6 +77,8 @@ def lib(native=False):
             return lib(False)
         raise
     L = C.CDLL(path)
+    if native:
+        shutil.rmtree(os.path.dirname(path))     # the loaded mapping outlives the file: nothing is left behind
     L.oiga_create.restype = C.c_void_p
     L.oiga_create.argtypes = [C.c_int, C.c_int]
     L.oiga_destroy.argtypes = [C.c_void_p]
