@@ -214,16 +214,7 @@ int launch_boundary_pass(petiga_cuda_plan* P, int slot, int form, const double* 
       int nqf = 1;
       for (int i = 0; i < L.dim; i++) if (i != d) nqf *= L.ax[i].nqp;
       if (nqf > kMaxFaceQ) { set_error("boundary form: more than 100 quadrature points per face element"); return PETIGA_CUDA_ERR_SUP; }
-      if (apply_fix && P->has_bc)
-        for (int dd = 0; dd < L.dim; dd++)
-          for (int ss = 0; ss < 2; ss++) {
-            FixSide& fs = bp.bc[dd][ss];
-            for (int k = 0; k < P->bc.vcount[dd][ss]; k++) {
-              const int c = P->bc.vfield[dd][ss][k];
-              if (c >= L.dof || fs.vcount >= kMaxDof) continue;
-              fs.vfield[fs.vcount] = c; fs.vvalue[fs.vcount] = P->bc.vvalue[dd][ss][k]; fs.vcount++;
-            }
-          }
+      if (apply_fix) fill_fix_sides(P, false, bp.bc);
       const int nfe = bp.n0 * bp.n1, blocks = (nfe + kWarps - 1) / kWarps;
       if (L.dim == 1) bnd_vec_kernel<1><<<blocks, kWarps * 32, 0, P->stream>>>(bp);
       else if (L.dim == 2) bnd_vec_kernel<2><<<blocks, kWarps * 32, 0, P->stream>>>(bp);

@@ -942,22 +942,12 @@ int launch_kronecker(petiga_cuda_plan* P, int slot, int block, double* values, d
       if ((kp.rsmask_ij[ij] >> rs) & 1) { if (n == 0) kp.slotA[ij] = (signed char)rs; else if (n == 1) kp.slotB[ij] = (signed char)rs; n++; }
     if (n > 2) kp.two_slot = 0;
   }
-  if (slot == PETIGA_SLOT_SYSTEM && P->has_bc)
+  if (slot == PETIGA_SLOT_SYSTEM) {
+    fill_fix_sides(P, true, kp.bc);
     for (int d = 0; d < L.dim; d++)
-      for (int s = 0; s < 2; s++) {
-        FixSide& fs = kp.bc[d][s];
-        for (int k = 0; k < P->bc.vcount[d][s]; k++) {
-          int c = P->bc.vfield[d][s][k];
-          if (c >= L.dof || fs.vcount >= kMaxDof) continue;
-          fs.vfield[fs.vcount] = c; fs.vvalue[fs.vcount] = P->bc.vvalue[d][s][k]; fs.vcount++;
-        }
-        for (int k = 0; k < P->bc.lcount[d][s]; k++) {
-          int c = P->bc.lfield[d][s][k];
-          if (c >= L.dof || fs.lcount >= kMaxDof) continue;
-          fs.lfield[fs.lcount] = c; fs.lvalue[fs.lcount] = P->bc.lvalue[d][s][k]; fs.lcount++;
-        }
-        if (!L.ax[d].periodic && (fs.vcount || fs.lcount)) kp.any_bc = 1;
-      }
+      for (int s = 0; s < 2; s++)
+        if (!L.ax[d].periodic && (kp.bc[d][s].vcount || kp.bc[d][s].lcount)) kp.any_bc = 1;
+  }
   {  // longest run of axis-0 rows that are full-width, in storage order and free of Dirichlet rows/columns
     const AxisLayout& a0 = L.ax[0];
     const bool fixing0 = kp.any_bc && slot == PETIGA_SLOT_SYSTEM && !a0.periodic;

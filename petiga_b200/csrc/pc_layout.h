@@ -15,6 +15,12 @@
 
 #include "../../include/petiga_cuda.h"
 
+#ifdef __CUDACC__
+#define PC_HOST_DEVICE __host__ __device__ __forceinline__
+#else
+#define PC_HOST_DEVICE inline
+#endif
+
 namespace pc {
 
 constexpr int kMaxP = 8;              // tuned kernels are instantiated for p = 1..4, the generic kernel (pc_quadg.cuh) runs p <= 8
@@ -59,16 +65,20 @@ struct Layout {
 // Builds the layout; returns 0 or a PETIGA_CUDA_ERR_* code with L.error set.
 int build_layout(const petiga_cuda_space& sp, int rank, int nranks, Layout& L);
 
-// closed-form position (in blocks, relative to the row base) of the column with per-axis offsets c[d]
-// (c = unwrapped column coordinate - first(row)) inside the row with per-axis ghost coordinates g[d].
+// closed-form position (in blocks, relative to the row base) of a column inside its row from the seg entries s0, s1, s2 of
+// the column's per-axis offsets and the row widths W0, W1 of axes 0 and 1.  Shared by the host and the quadrature kernels.
+PC_HOST_DEVICE int seg_position(uint32_t s0, uint32_t s1, uint32_t s2, int W0, int W1) {
+  const int Bi = s0 & 255, Si = (s0 >> 8) & 255, Li = (s0 >> 16) & 255;
+  const int Bj = s1 & 255, Sj = (s1 >> 8) & 255, Lj = (s1 >> 16) & 255;
+  const int Bk = s2 & 255, Sk = (s2 >> 8) & 255, Lk = (s2 >> 16) & 255;
+  return Bk * W1 * W0 + Sk * (Bj * W0 + Sj * Bi) + (Lk * Sj + Lj) * Si + Li;
+}
+
+// seg_position of the column with per-axis offsets c[d] (c = unwrapped column coordinate - first(row)) inside the row with
+// per-axis ghost coordinates g[d].
 inline int64_t col_position(const Layout& L, const int g[3], const int c[3]) {
-  uint32_t s0 = L.ax[0].seg[g[0] * kMaxW + c[0]], s1 = L.ax[1].seg[g[1] * kMaxW + c[1]],
-           s2 = L.ax[2].seg[g[2] * kMaxW + c[2]];
-  int Bi = s0 & 255, Si = (s0 >> 8) & 255, Li = (s0 >> 16) & 255;
-  int Bj = s1 & 255, Sj = (s1 >> 8) & 255, Lj = (s1 >> 16) & 255;
-  int Bk = s2 & 255, Sk = (s2 >> 8) & 255, Lk = (s2 >> 16) & 255;
-  int Wi = L.ax[0].W[g[0]], Wj = L.ax[1].W[g[1]];
-  return (int64_t)Bk * Wj * Wi + (int64_t)Sk * (Bj * Wi + Sj * Bi) + (int64_t)(Lk * Sj + Lj) * Si + Li;
+  return seg_position(L.ax[0].seg[g[0] * kMaxW + c[0]], L.ax[1].seg[g[1] * kMaxW + c[1]], L.ax[2].seg[g[2] * kMaxW + c[2]],
+                      L.ax[0].W[g[0]], L.ax[1].W[g[1]]);
 }
 
 // Host generation of the owned-row pattern (tests, small meshes).  block=0 expands to scalar AIJ rows.

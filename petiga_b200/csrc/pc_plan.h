@@ -121,6 +121,9 @@ int nccl_load();
 int allgather_owned(petiga_cuda_plan* P, const double* owned, double* full);
 int allreduce_sum(petiga_cuda_plan* P, double* d_buf, int n);
 void nvtx_push(const char* name);
+// IGAFormBC of every face as the element fix-up reads it: the values and, with loads, the Neumann loads of fields < dof
+// (pc_api.cu).  out must be zeroed; it stays so when no boundary condition is set.  Each caller derives its own any_bc.
+void fill_fix_sides(const petiga_cuda_plan* P, bool loads, FixSide out[3][2]);
 // boundary-integral pass (pc_bnd.cu)
 int launch_boundary_pass(petiga_cuda_plan* P, int slot, int form, const double* prm, double* rhs, bool apply_fix);
 }  // namespace pc

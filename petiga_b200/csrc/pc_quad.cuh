@@ -12,7 +12,7 @@
 //   IGAElementFix{System,Function,Jacobian} src/petigaelem.c:1360-1501 -> applied on the register tiles
 //   IGAElementAssembleMat/Vec (MatSetValuesLocal ADD_VALUES) :1525-1559 -> closed-form CSR position + red.global.add.f64
 #pragma once
-#include "pc_device.h"
+#include "pc_element.cuh"
 
 namespace pc {
 
@@ -93,15 +93,7 @@ quad_kernel(const __grid_constant__ KParams prm) {
   const bool transient = (prm.slot == PETIGA_SLOT_IFUNCTION || prm.slot == PETIGA_SLOT_IJACOBIAN);
 
   int ID[3] = {0, 0, 0}, nq1[3] = {1, 1, 1}, nqp = 1;
-  if (valid) {  // IGANextElement: index -> ID, i fastest (src/petigaelem.c:388-395)
-    int idx = elem;
-#pragma unroll
-    for (int d = 0; d < 3; d++) {
-      int c = idx % prm.ax[d].ew;
-      idx /= prm.ax[d].ew;
-      ID[d] = c + prm.ax[d].es;
-    }
-  }
+  if (valid) element_id(prm.ax, elem, ID);
 #pragma unroll
   for (int d = 0; d < 3; d++) { nq1[d] = prm.ax[d].nqp; nqp *= nq1[d]; }
 
@@ -109,10 +101,8 @@ quad_kernel(const __grid_constant__ KParams prm) {
   if (valid) {
     for (int a = lt; a < M; a += G) {
       int ia = a % NEN1, ja = (DIM > 1) ? (a / NEN1) % NEN1 : 0, ka = (DIM > 2) ? a / (NEN1 * NEN1) : 0;
-      int g0 = prm.ax[0].offset[ID[0]] + ia - prm.ax[0].gs;
-      int g1 = (DIM > 1) ? prm.ax[1].offset[ID[1]] + ja - prm.ax[1].gs : 0;
-      int g2 = (DIM > 2) ? prm.ax[2].offset[ID[2]] + ka - prm.ax[2].gs : 0;
-      int gidx = g0 + prm.ax[0].gw * (g1 + prm.ax[1].gw * g2);   // element->mapping[a] (petigaelem.c:703-719)
+      const int ai[3] = {ia, ja, ka};
+      int gidx = closure_index<DIM>(prm.ax, ID, ai);
       int lr = prm.localrow[gidx];
       lrow[a] = lr;
       if (mapped) {
@@ -126,7 +116,6 @@ quad_kernel(const __grid_constant__ KParams prm) {
 #pragma unroll
       for (int c = 0; c < DOF; c++) { onfix[c] = 0; vfix[c] = 0.0; vflux[c] = 0.0; }
       if (prm.any_bc) {
-        const int ai[3] = {ia, ja, ka};
 #pragma unroll
         for (int d = 0; d < DIM; d++) {
           if (prm.ax[d].periodic) continue;
@@ -472,16 +461,8 @@ quad_kernel(const __grid_constant__ KParams prm) {
         const int n = Cfg::col(tx, j);
         const int b = n / (DOF * DOF), jj = (n / DOF) % DOF, ii = n % DOF;
         const int ib = b % NEN1, jb = (DIM > 1) ? (b / NEN1) % NEN1 : 0, kb = (DIM > 2) ? b / (NEN1 * NEN1) : 0;
-        const uint32_t s0 = segs[ia * NEN1 + ib], s1 = segs[NEN1 * NEN1 + ja * NEN1 + jb], s2 = segs[2 * NEN1 * NEN1 + ka * NEN1 + kb];
-        const int Bi = s0 & 255, Si = (s0 >> 8) & 255, Li = (s0 >> 16) & 255;
-        const int Bj = s1 & 255, Sj = (s1 >> 8) & 255, Lj = (s1 >> 16) & 255;
-        const int Bk = s2 & 255, Sk = (s2 >> 8) & 255, Lk = (s2 >> 16) & 255;
-        const int pos = Bk * W1 * W0 + Sk * (Bj * W0 + Sj * Bi) + (Lk * Sj + Lj) * Si + Li;
-        size_t off;
-        if (DOF == 1) off = (size_t)(base + pos);
-        else if (prm.block) off = (size_t)(base + pos) * DOF * DOF + jj * DOF + ii;     // BAIJ: column-major blocks
-        else off = (size_t)base * DOF * DOF + (size_t)ii * (W0 * W1 * W2) * DOF + (size_t)pos * DOF + jj;
-        atomicAdd(dst + off, v);
+        const int pos = seg_position(segs[ia * NEN1 + ib], segs[NEN1 * NEN1 + ja * NEN1 + jb], segs[2 * NEN1 * NEN1 + ka * NEN1 + kb], W0, W1);
+        atomicAdd(dst + value_offset(base, pos, DOF, prm.block, ii, jj, W0 * W1 * W2), v);
       }
     }
   }

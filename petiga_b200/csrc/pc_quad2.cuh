@@ -16,7 +16,7 @@
 // which needs ~7x fewer FP64 operations than the pair loop at p=3 in 3-D (SURVEY 8d anticipates this).
 // Geometry, NURBS weights and state fields are evaluated at the points by the same axis-by-axis contraction.
 #pragma once
-#include "pc_device.h"
+#include "pc_element.cuh"
 
 namespace pc {
 
@@ -150,20 +150,13 @@ __global__ void __launch_bounds__(SFCfg<DIM, P, DOF>::THREADS, MINB) quad_sf_ker
   const bool transient = (prm.slot == PETIGA_SLOT_IFUNCTION || prm.slot == PETIGA_SLOT_IJACOBIAN);
 
   int ID[3] = {0, 0, 0};
-  if (valid) {
-    int idx = elem;
-#pragma unroll
-    for (int d = 0; d < 3; d++) { int c = idx % prm.ax[d].ew; idx /= prm.ax[d].ew; ID[d] = c + prm.ax[d].es; }
-  }
+  if (valid) element_id(prm.ax, elem, ID);
 
   // ---------------- header: closure, gathers, fix lists, position tables, 1-D tables ----------------
   if (valid) {
     for (int a = lt; a < NEN; a += G) {
-      const int ia = a % n0, ja = (a / n0) % n1, ka = a / (n0 * n1);
-      const int g0 = prm.ax[0].offset[ID[0]] + ia - prm.ax[0].gs;
-      const int g1 = (DIM > 1) ? prm.ax[1].offset[ID[1]] + ja - prm.ax[1].gs : 0;
-      const int g2 = (DIM > 2) ? prm.ax[2].offset[ID[2]] + ka - prm.ax[2].gs : 0;
-      const int gidx = g0 + prm.ax[0].gw * (g1 + prm.ax[1].gw * g2);
+      const int ai[3] = {a % n0, (a / n0) % n1, a / (n0 * n1)};
+      const int gidx = closure_index<DIM>(prm.ax, ID, ai);
       const int lr = prm.localrow[gidx];
       lrow[a] = lr;
       rbase[a] = want_mat ? prm.rowbase[lr] : 0;   // its L2 latency is paid here, under the header's other loads, not in the scatter
@@ -179,7 +172,6 @@ __global__ void __launch_bounds__(SFCfg<DIM, P, DOF>::THREADS, MINB) quad_sf_ker
 #pragma unroll
       for (int c = 0; c < DOF; c++) { onfix[c] = 0; vfix[c] = 0.0; vflux[c] = 0.0; }
       if (prm.any_bc) {   // BuildFix/AddFixa/AddFlux (petigaelem.c:1166-1283)
-        const int ai[3] = {ia, ja, ka};
 #pragma unroll
         for (int d = 0; d < DIM; d++) {
           if (prm.ax[d].periodic) continue;
@@ -321,19 +313,7 @@ __global__ void __launch_bounds__(SFCfg<DIM, P, DOF>::THREADS, MINB) quad_sf_ker
           for (int d = 0; d < DIM; d++) X1[i][d] = (ev(ls.f_x0 + i, ls.tG[d]) - X0[i] * wg[d]) * iw;   // quotient rule (K4) on W*X
           x[i] = X0[i];
         }
-        double det;
-        if (DIM == 1) { det = X1[0][0]; E[0][0] = 1.0 / det; }
-        else if (DIM == 2) {
-          det = X1[0][0] * X1[1][1] - X1[0][1] * X1[1][0];
-          E[0][0] = X1[1][1] / det; E[0][1] = -X1[0][1] / det; E[1][0] = -X1[1][0] / det; E[1][1] = X1[0][0] / det;
-        } else {
-          const double a00 = X1[0][0], a01 = X1[0][1], a02 = X1[0][2], a10 = X1[1][0], a11 = X1[1][1], a12 = X1[1][2], a20 = X1[2][0], a21 = X1[2][1], a22 = X1[2][2];
-          det = a00 * (a11 * a22 - a12 * a21) - a01 * (a10 * a22 - a12 * a20) + a02 * (a10 * a21 - a11 * a20);
-          E[0][0] = (a11 * a22 - a12 * a21) / det; E[0][1] = -(a01 * a22 - a02 * a21) / det; E[0][2] = (a01 * a12 - a02 * a11) / det;
-          E[1][0] = -(a10 * a22 - a12 * a20) / det; E[1][1] = (a00 * a22 - a02 * a20) / det; E[1][2] = -(a00 * a12 - a02 * a10) / det;
-          E[2][0] = (a10 * a21 - a11 * a20) / det; E[2][1] = -(a00 * a21 - a01 * a20) / det; E[2][2] = (a00 * a11 - a01 * a10) / det;
-        }
-        J *= det;                                            // detJac *= detX (petigaelem.c:1024-1029)
+        J *= inverse_map<DIM>(X1, E);                        // detJac *= detX (petigaelem.c:1024-1029)
       }
       JW[q] = J * w;
 #pragma unroll

@@ -173,8 +173,7 @@ __global__ void __launch_bounds__(64) sf3_geom_kernel(const __grid_constant__ SF
     pt[gt] = prm.ax[d].point[ID[d] * 4 + q];
   }
   const int a = gt, ai[3] = {a & 3, (a >> 2) & 3, a >> 4};
-  const int gidx = (prm.ax[0].offset[ID[0]] + ai[0] - prm.ax[0].gs) +
-                   prm.ax[0].gw * ((prm.ax[1].offset[ID[1]] + ai[1] - prm.ax[1].gs) + prm.ax[1].gw * (prm.ax[2].offset[ID[2]] + ai[2] - prm.ax[2].gs));
+  const int gidx = closure_index<3>(prm.ax, ID, ai);
   if (mapped) {
 #pragma unroll
     for (int i = 0; i < 3; i++) Xs[i * 64 + a] = prm.X[(size_t)gidx * 3 + i];

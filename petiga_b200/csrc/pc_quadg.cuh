@@ -22,7 +22,7 @@
 // K_e lives in shared memory; when (nen*dof)^2 doubles do not fit, the element is processed in column panels (the chunk
 // loop is repeated per panel).  It is a coverage kernel: correctness first, one element per CTA.
 #pragma once
-#include "pc_device.h"
+#include "pc_element.cuh"
 
 namespace pc {
 
@@ -109,10 +109,8 @@ __global__ void __launch_bounds__(kGenThreads) quad_gen_kernel(const __grid_cons
   int ID[3] = {0, 0, 0};
   {
     int idx = blockIdx.x;
-    if (!face) {
-#pragma unroll
-      for (int d = 0; d < 3; d++) { const int c = idx % prm.ax[d].ew; idx /= prm.ax[d].ew; ID[d] = c + prm.ax[d].es; }
-    } else {
+    if (!face) element_id(prm.ax, idx, ID);
+    else {
 #pragma unroll
       for (int d = 0; d < 3; d++) {
         if (d == fax) { ID[d] = fsd ? prm.ax[d].nel - 1 : 0; continue; }
@@ -317,17 +315,7 @@ __global__ void __launch_bounds__(kGenThreads) quad_gen_kernel(const __grid_cons
           for (int i = 0; i < DIM; i++)
 #pragma unroll
             for (int d = 0; d < DIM; d++) X1[i][d] = gq[10 + i * DIM + d];
-          if (DIM == 1) { det = X1[0][0]; E[0][0] = 1.0 / det; }
-          else if (DIM == 2) {
-            det = X1[0][0] * X1[1][1] - X1[0][1] * X1[1][0];
-            E[0][0] = X1[1][1] / det; E[0][1] = -X1[0][1] / det; E[1][0] = -X1[1][0] / det; E[1][1] = X1[0][0] / det;
-          } else {
-            const double a00 = X1[0][0], a01 = X1[0][1], a02 = X1[0][2], a10 = X1[1][0], a11 = X1[1][1], a12 = X1[1][2], a20 = X1[2][0], a21 = X1[2][1], a22 = X1[2][2];
-            det = a00 * (a11 * a22 - a12 * a21) - a01 * (a10 * a22 - a12 * a20) + a02 * (a10 * a21 - a11 * a20);
-            E[0][0] = (a11 * a22 - a12 * a21) / det; E[0][1] = -(a01 * a22 - a02 * a21) / det; E[0][2] = (a01 * a12 - a02 * a11) / det;
-            E[1][0] = -(a10 * a22 - a12 * a20) / det; E[1][1] = (a00 * a22 - a02 * a20) / det; E[1][2] = -(a00 * a12 - a02 * a10) / det;
-            E[2][0] = (a10 * a21 - a11 * a20) / det; E[2][1] = -(a00 * a21 - a01 * a20) / det; E[2][2] = (a00 * a11 - a01 * a10) / det;
-          }
+          det = inverse_map<DIM>(X1, E);
 #pragma unroll
           for (int i = 0; i < DIM; i++) x[i] = Xq[ql * 3 + i];
           if (face) {   // IGA_GetNormal (src/petigaval.F90:45-99)
@@ -544,22 +532,14 @@ __global__ void __launch_bounds__(kGenThreads) quad_gen_kernel(const __grid_cons
         if (v == 0.0) continue;
         const int ai[3] = {a % nA[0], (a / nA[0]) % nA[1], a / (nA[0] * nA[1])};
         const int bi[3] = {b % nA[0], (b / nA[0]) % nA[1], b / (nA[0] * nA[1])};
-        const uint32_t s0 = segs[ai[0] * kGenMaxN1 + bi[0]], s1 = segs[kGenMaxN1 * kGenMaxN1 + ai[1] * kGenMaxN1 + bi[1]],
-                       s2 = segs[2 * kGenMaxN1 * kGenMaxN1 + ai[2] * kGenMaxN1 + bi[2]];
-        const int Bi = s0 & 255, Si = (s0 >> 8) & 255, Li = (s0 >> 16) & 255;
-        const int Bj = s1 & 255, Sj = (s1 >> 8) & 255, Lj = (s1 >> 16) & 255;
-        const int Bk = s2 & 255, Sk = (s2 >> 8) & 255, Lk = (s2 >> 16) & 255;
         const int W0 = Wd[ai[0]], W1 = Wd[kGenMaxN1 + ai[1]], W2 = Wd[2 * kGenMaxN1 + ai[2]];
-        const int pos = Bk * W1 * W0 + Sk * (Bj * W0 + Sj * Bi) + (Lk * Sj + Lj) * Si + Li;
+        const int pos = seg_position(segs[ai[0] * kGenMaxN1 + bi[0]], segs[kGenMaxN1 * kGenMaxN1 + ai[1] * kGenMaxN1 + bi[1]],
+                                     segs[2 * kGenMaxN1 * kGenMaxN1 + ai[2] * kGenMaxN1 + bi[2]], W0, W1);
         const int lr = lrow[a];
         int64_t base = prm.rowbase[lr];
         double* dst = prm.values;
         if (lr >= prm.nown) { dst = prm.ghost_values; base -= prm.nnz_own; }
-        size_t off;
-        if (dof == 1) off = (size_t)(base + pos);
-        else if (prm.block) off = (size_t)(base + pos) * dof * dof + j * dof + i;          // BAIJ: column-major blocks
-        else off = (size_t)base * dof * dof + (size_t)i * (W0 * W1 * W2) * dof + (size_t)pos * dof + j;
-        atomicAdd(dst + off, v);
+        atomicAdd(dst + value_offset(base, pos, dof, prm.block, i, j, W0 * W1 * W2), v);
       }
     }
     __syncthreads();

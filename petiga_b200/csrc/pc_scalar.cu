@@ -16,6 +16,7 @@
 #include <cmath>
 #include <cstring>
 
+#include "pc_element.cuh"
 #include "pc_plan.h"
 
 namespace pc {
@@ -161,8 +162,8 @@ __global__ void __launch_bounds__(kThreads) scalar_kernel(const __grid_constant_
   for (int k = 0; k < kMaxS; k++) S[k] = 0.0;
 
   for (int elem = blockIdx.x; elem < sp.nelem; elem += gridDim.x) {
-    int ID[3], idx = elem;
-    for (int d = 0; d < 3; d++) { int c = idx % sp.ax[d].ew; idx /= sp.ax[d].ew; ID[d] = c + sp.ax[d].es; }   // IGANextElement, i fastest
+    int ID[3];
+    element_id(sp.ax, elem, ID);
     __syncthreads();
     for (int a = threadIdx.x; a < nen; a += blockDim.x) {   // closure + IGAElementGetValues (petigaelem.c:693-755,1074-1100)
       const int n0 = sp.ax[0].nen, n1 = sp.ax[1].nen;

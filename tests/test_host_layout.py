@@ -165,6 +165,13 @@ def test_hot_kernel_register_budget():
     assert regs("pc_kron.ptxas.log", "kron_rows_kernelILi1ELi3ELi4") <= 64      # short pencils: 4 CTAs per SM
     assert regs("pc_kron.ptxas.log", "kron_rows_kernelILi1ELi3ELi3") <= 85      # long pencils: 3 CTAs per SM
     assert regs("pc_kron.ptxas.log", "kron_rows_kernelILi3ELi0ELi2") <= 128     # cfg 4 (BAIJ bs=3): 2 CTAs per SM (each warp stages a whole row in shared memory)
+    # cfg 5, the third-generation kernels and cfg 3's vector kernel, held at their counts with CUDA 12.9
+    assert regs("pc_quad.ptxas.log", "quad_kernelILi2ELi2ELi1ELi3E") <= 124     # cfg 5
+    assert regs("pc_quad3.ptxas.log", "quad_sf3r_kernelILi0E") <= 168
+    assert regs("pc_quad3.ptxas.log", "quad_sf3r_kernelILi1E") <= 168
+    assert regs("pc_quad3.ptxas.log", "quad_sf3r_kernelILi2E") <= 162
+    assert regs("pc_quad3.ptxas.log", "sf3_geom_kernel") <= 72
+    assert regs("pc_quad3.ptxas.log", "quad_vec3_kernelILi4ELb0E") <= 48     # cfg 3
 
 
 def test_functional_and_boundary_form_argument_checks():
