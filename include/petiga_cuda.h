@@ -215,10 +215,27 @@ int petiga_cuda_finish(petiga_cuda_plan *plan);
    petiga_cuda_spmv      <- MatMult
    petiga_cuda_solve_cg  <- KSPSolve with KSPCG + PCJACOBI: x is the initial guess on entry; stops at |r| <= max(rtol |b|, atol)
                             or maxit; *iters and *relres (= |r| / |b|) report the outcome.  The matrix must be symmetric positive
-                            definite (Poisson, Laplace, mass, elasticity systems). */
+                            definite (Poisson, Laplace, mass, elasticity systems).
+   petiga_cuda_solve_gmres <- KSPSolve with KSPGMRES + PCJACOBI (-ksp_pc_side right; PETSc's default side for GMRES is left):
+                            restarted GMRES(restart), classical Gram-Schmidt without refinement, the Jacobi diagonal applied on the
+                            right (A D^-1 u = b, x = D^-1 u), so that rtol, atol and relres mean what they mean for CG.  Any square
+                            matrix with a nonzero diagonal: the IJacobians of the nonlinear and time-dependent forms are not
+                            symmetric.  x is the initial guess on entry; stops at |b - A x| <= max(rtol |b|, atol) or maxit.
+                            Convergence is decided on the true residual, recomputed at the end of every cycle; *iters, *relres
+                            (= |b - A x| / |b| at exit) and *reason (PETIGA_KSP_*, PETSc's KSPConvergedReason values) report the
+                            outcome.  Stopping at maxit, a breakdown or a non-finite value returns 0 with the reason set; x then holds
+                            the last finite iterate.  b = 0 gives x = 0, 0 iterations and PETIGA_KSP_CONVERGED_ATOL.
+                            PETIGA_CUDA_ERR_ARG: a NULL pointer, b == x, restart < 1 or maxit < 0; PETIGA_CUDA_ERR_SUP: BAIJ with
+                            dof > 4 (as petiga_cuda_spmv).  Deterministic: two solves of the same system give the same bits. */
+enum {
+  PETIGA_KSP_CONVERGED_ITERATING = 0, PETIGA_KSP_CONVERGED_RTOL = 2, PETIGA_KSP_CONVERGED_ATOL = 3,
+  PETIGA_KSP_DIVERGED_ITS = -3, PETIGA_KSP_DIVERGED_BREAKDOWN = -5, PETIGA_KSP_DIVERGED_NANORINF = -9
+};
 int petiga_cuda_spmv(petiga_cuda_plan *plan, int block, const double *values, const double *x, double *y);
 int petiga_cuda_solve_cg(petiga_cuda_plan *plan, int block, const double *values, const double *b, double *x,
                          double rtol, double atol, int maxit, int *iters, double *relres);
+int petiga_cuda_solve_gmres(petiga_cuda_plan *plan, int block, const double *values, const double *b, double *x, int restart,
+                            double rtol, double atol, int maxit, int *iters, double *relres, int *reason);
 
 /* IGAComputeScalar (src/petigacomp.c:35-96): S[k] = sum over all ranks, elements and quadrature points of
    detJac*weight * Scalar_k(point, U).  U: device [owned nodes * dof] or NULL (a NULL state evaluates as zero, which is how
@@ -239,6 +256,7 @@ int petiga_cuda_free(void *ptr);
 int petiga_cuda_memcpy_h2d(void *dst, const void *src, size_t bytes);
 int petiga_cuda_memcpy_d2h(void *dst, const void *src, size_t bytes);
 int petiga_cuda_memset(void *dst, int value, size_t bytes);
+int petiga_cuda_memset_async(petiga_cuda_plan *plan, void *dst, int value, size_t bytes);   /* enqueued on the plan's stream */
 int petiga_cuda_host_alloc(void **ptr, size_t bytes);   /* pinned */
 int petiga_cuda_host_free(void *ptr);
 /* sum (a-b)^2 and sum b^2 over n device doubles on the current device (deterministic; synchronous): lets a caller compare two

@@ -240,16 +240,34 @@ PetscErrorCode IGASetOption(IGA iga, const char *name, PetscReal value);     /* 
                                                                                  resident hand-off to a GPU solve, SURVEY 8f-4) */
 PetscErrorCode IGAGetStat(IGA iga, const char *name, PetscReal *value);
 /* ---- the step after the path (SURVEY.md 8 f-4): the assembled Mat stays on the device and is consumed there ----
-   IGACreateKSP: src/petiga.c:856-885; use as demo/Poisson3D.c:73-83 does.  The solver is conjugate gradients with the Jacobi
-   diagonal (-ksp_type cg -pc_type jacobi), for the symmetric positive definite systems of the linear demos; KSPGetResidualNorm
-   returns |r| / |b|.  MatMult is the product the solver iterates with. */
+   IGACreateKSP: src/petiga.c:856-885; use as demo/Poisson3D.c:73-83 does.  The preconditioner is always the Jacobi diagonal
+   (-pc_type jacobi).  Two Krylov methods (KSPSetType):
+     KSPCG     conjugate gradients, for the symmetric positive definite systems of the linear demos.  The default of
+               IGACreateKSP here (PETSc's default is GMRES).
+     KSPGMRES  restarted GMRES (KSPGMRESSetRestart, default 30; classical Gram-Schmidt) for any matrix with a nonzero diagonal,
+               e.g. the non-symmetric IJacobians of the nonlinear and time-dependent forms.  The diagonal is applied on the
+               right (-ksp_pc_side right; PETSc's default side for GMRES is left), so the residual tested is |b - A x|.
+   KSPGetResidualNorm returns |b - A x| / |b|; KSPGetConvergedReason says why the solve stopped.  For CG the reason is derived
+   from what the CG kernel returns: |r| / |b| <= rtol gives RTOL, else fewer than maxits iterations gives ATOL, else
+   DIVERGED_ITS; so a CG solve that meets atol in its last allowed burst of iterations is reported as DIVERGED_ITS.
+   MatMult is the product the solvers iterate with. */
+typedef const char *KSPType;
+#define KSPCG "cg"
+#define KSPGMRES "gmres"
+typedef enum {
+  KSP_CONVERGED_ITERATING = 0, KSP_CONVERGED_RTOL = 2, KSP_CONVERGED_ATOL = 3,
+  KSP_DIVERGED_ITS = -3, KSP_DIVERGED_BREAKDOWN = -5, KSP_DIVERGED_NANORINF = -9
+} KSPConvergedReason;
 PetscErrorCode MatMult(Mat A, Vec x, Vec y);
 PetscErrorCode IGACreateKSP(IGA iga, KSP *ksp);
+PetscErrorCode KSPSetType(KSP ksp, KSPType type);                   /* KSPCG or KSPGMRES; any other name: PETSC_ERR_SUP */
+PetscErrorCode KSPGMRESSetRestart(KSP ksp, PetscInt restart);       /* >= 1; ignored by CG */
 PetscErrorCode KSPSetOperators(KSP ksp, Mat A, Mat P);
 PetscErrorCode KSPSetTolerances(KSP ksp, PetscReal rtol, PetscReal abstol, PetscReal dtol, PetscInt maxits);
 PetscErrorCode KSPSolve(KSP ksp, Vec b, Vec x);
 PetscErrorCode KSPGetIterationNumber(KSP ksp, PetscInt *its);
 PetscErrorCode KSPGetResidualNorm(KSP ksp, PetscReal *rnorm);
+PetscErrorCode KSPGetConvergedReason(KSP ksp, KSPConvergedReason *reason);
 PetscErrorCode KSPDestroy(KSP *ksp);
 
 PetscErrorCode IGASynchronize(IGA iga);                                        /* wait for the IGA's stream (after IGASetOption(iga,"async",1)) */

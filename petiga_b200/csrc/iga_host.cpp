@@ -49,8 +49,9 @@ struct _p_Vec {
 struct _p_Mat {
   IGA iga; int baij; int bs; int nrows; int64_t nnz; const int* d_rowptr; const int* d_colidx; double* d_values; long gen; };
 
-struct _p_KSP {      // IGACreateKSP: conjugate gradients + Jacobi on the device (petiga_cuda_solve_cg)
-  IGA iga; Mat A; double rtol, abstol; int maxits, its; double rnorm; };
+struct _p_KSP {      // IGACreateKSP: conjugate gradients (petiga_cuda_solve_cg) or GMRES (petiga_cuda_solve_gmres) + Jacobi on the device
+  IGA iga; Mat A; double rtol, abstol; int maxits, its; double rnorm;
+  bool gmres = false; int restart = 30; KSPConvergedReason reason = KSP_CONVERGED_ITERATING; };
 
 struct _p_IGA {
   IGAComm comm;
@@ -869,8 +870,38 @@ PetscErrorCode KSPSolve(KSP ksp, Vec b, Vec x) {
   if (b == x) return fail(PETSC_ERR_ARG_IDN, "b and x must be different vectors");
   IGA g = ksp->iga;
   // KSPSolve starts from x = 0 unless KSPSetInitialGuessNonzero was called (not mirrored)
+  ksp->reason = KSP_CONVERGED_ITERATING;
+  if (ksp->gmres) {
+    if (int rc = petiga_cuda_memset_async(g->plan, x->d, 0, (size_t)x->n * sizeof(double))) return from_cuda(rc);
+    int reason = 0;
+    if (int rc = petiga_cuda_solve_gmres(g->plan, ksp->A->baij, ksp->A->d_values, b->d, x->d, ksp->restart, ksp->rtol, ksp->abstol, ksp->maxits,
+                                         &ksp->its, &ksp->rnorm, &reason)) return from_cuda(rc);
+    ksp->reason = (KSPConvergedReason)reason;
+    return 0;
+  }
   if (int rc = petiga_cuda_memset(x->d, 0, (size_t)x->n * sizeof(double))) return from_cuda(rc);
-  return from_cuda(petiga_cuda_solve_cg(g->plan, ksp->A->baij, ksp->A->d_values, b->d, x->d, ksp->rtol, ksp->abstol, ksp->maxits, &ksp->its, &ksp->rnorm));
+  if (int rc = petiga_cuda_solve_cg(g->plan, ksp->A->baij, ksp->A->d_values, b->d, x->d, ksp->rtol, ksp->abstol, ksp->maxits, &ksp->its, &ksp->rnorm))
+    return from_cuda(rc);
+  ksp->reason = ksp->rnorm <= ksp->rtol ? KSP_CONVERGED_RTOL : ksp->its < ksp->maxits ? KSP_CONVERGED_ATOL : KSP_DIVERGED_ITS;
+  return 0;
+}
+PetscErrorCode KSPSetType(KSP ksp, KSPType type) {
+  if (!ksp || !type) return fail(PETSC_ERR_ARG_NULL, "Null KSP/KSPType");
+  if (!strcmp(type, KSPCG)) ksp->gmres = false;
+  else if (!strcmp(type, KSPGMRES)) ksp->gmres = true;
+  else return fail(PETSC_ERR_SUP, std::string("KSPSetType: unsupported type \"") + type + "\" (the device provides \"cg\" and \"gmres\")");
+  return 0;
+}
+PetscErrorCode KSPGMRESSetRestart(KSP ksp, PetscInt restart) {
+  if (!ksp) return fail(PETSC_ERR_ARG_NULL, "Null KSP");
+  if (restart < 1) return fail(PETSC_ERR_ARG_OUTOFRANGE, "KSPGMRESSetRestart: restart must be at least 1");
+  ksp->restart = restart;
+  return 0;
+}
+PetscErrorCode KSPGetConvergedReason(KSP ksp, KSPConvergedReason* reason) {
+  if (!ksp || !reason) return fail(PETSC_ERR_ARG_NULL, "Null pointer");
+  *reason = ksp->reason;
+  return 0;
 }
 PetscErrorCode KSPGetIterationNumber(KSP ksp, PetscInt* its) { if (!ksp || !its) return fail(PETSC_ERR_ARG_NULL, "Null pointer"); *its = ksp->its; return 0; }
 PetscErrorCode KSPGetResidualNorm(KSP ksp, PetscReal* rnorm) { if (!ksp || !rnorm) return fail(PETSC_ERR_ARG_NULL, "Null pointer"); *rnorm = ksp->rnorm; return 0; }

@@ -364,7 +364,7 @@ int petiga_cuda_plan_destroy(petiga_cuda_plan* P) {
   for (void* d : P->allocs) cudaFree(d);
   for (int b = 0; b < 2; b++) { cudaFree(P->d_rowptr[b]); cudaFree(P->d_colidx[b]); }
   cudaFree(P->d_X); cudaFree(P->d_W); cudaFree(P->d_fixtable); cudaFree(P->d_ghost_values); cudaFree(P->d_recv);
-  cudaFree(P->d_scalar); cudaFree(P->d_sf3_dprime); cudaFree(P->d_solve_work); cudaFree(P->d_solve_xfull); cudaFree(P->d_values_own); cudaFree(P->d_rhs_own); cudaFree(P->d_U_own); cudaFree(P->d_V_own);
+  cudaFree(P->d_scalar); cudaFree(P->d_sf3_dprime); cudaFree(P->d_solve_work); cudaFree(P->d_solve_xfull); cudaFree(P->d_gmres_work); cudaFree(P->d_values_own); cudaFree(P->d_rhs_own); cudaFree(P->d_U_own); cudaFree(P->d_V_own);
   if (P->h_pinned) cudaFreeHost(P->h_pinned);
   if (P->ev0) cudaEventDestroy(P->ev0);
   if (P->ev1) cudaEventDestroy(P->ev1);
@@ -868,6 +868,12 @@ int petiga_cuda_free(void* ptr) { PC_CUDA(cudaFree(ptr)); return 0; }
 int petiga_cuda_memcpy_h2d(void* dst, const void* src, size_t bytes) { PC_CUDA(cudaMemcpy(dst, src, bytes, cudaMemcpyHostToDevice)); return 0; }
 int petiga_cuda_memcpy_d2h(void* dst, const void* src, size_t bytes) { PC_CUDA(cudaMemcpy(dst, src, bytes, cudaMemcpyDeviceToHost)); return 0; }
 int petiga_cuda_memset(void* dst, int value, size_t bytes) { PC_CUDA(cudaMemset(dst, value, bytes)); return 0; }
+int petiga_cuda_memset_async(petiga_cuda_plan* P, void* dst, int value, size_t bytes) {
+  if (!P || (!dst && bytes)) return PETIGA_CUDA_ERR_ARG;
+  PC_CUDA(cudaSetDevice(P->device));
+  PC_CUDA(cudaMemsetAsync(dst, value, bytes, P->stream));
+  return 0;
+}
 // Pinned host memory on the NUMA node of the current device: the pages are placed by first touch, so the calling thread is moved onto
 // the GPU's local CPUs (sysfs local_cpulist of its PCI function) for the allocation and the first touch, then moved back.  With eight
 // ranks copying results out at once, buffers that all sit on one socket share one memory controller and one inter-socket link

@@ -37,6 +37,7 @@ struct petiga_cuda_plan {
   double* d_sf3pp[3] = {nullptr, nullptr, nullptr};     // the same products in the fragment layout of the third-generation kernel
   double* d_solve_work = nullptr; size_t solve_work_cap = 0;     // pc_solve.cu: r, z, p, Ap, 1/diag, reduction partials, scalars
   double* d_solve_xfull = nullptr; size_t solve_xfull_cap = 0;   // full-length operand of a distributed matrix-vector product
+  double* d_gmres_work = nullptr; size_t gmres_work_cap = 0;     // pc_solve.cu GMRES: Krylov basis, w, z, 1/diag, partials, Hessenberg, rotations
   double* d_sf3_dprime = nullptr; size_t sf3_dprime_cap = 0;   // D'[element][pair][64] of the geometry pre-pass (mapped geometry)
 
   // pattern (owned by the plan), per block mode

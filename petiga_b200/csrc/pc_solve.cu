@@ -7,6 +7,8 @@
 //   petiga_cuda_spmv      y = A x          (MatMult)   AIJ scalar CSR or BAIJ block CSR with column-major blocks
 //   petiga_cuda_solve_cg  Jacobi-preconditioned conjugate gradients (KSPCG + PCJACOBI), scalars kept on the device:
 //                         one host read of the residual norm every `check` iterations, none otherwise
+//   petiga_cuda_solve_gmres  restarted GMRES with the Jacobi diagonal on the right (KSPGMRES + PCJACOBI, -ksp_pc_side right) for
+//                         the non-symmetric Jacobians; the same host-read cadence, convergence decided on the true residual
 // Multi-rank: rows are distributed as the matrix is (rank-major global numbering, src/petigagrid.c:98-171); the operand of
 // the product is gathered into a full-length device vector over NCCL (a grouped ncclBroadcast per owner: the VecScatter of
 // MatMult_MPIAIJ), dot products by ncclAllReduce.  Deterministic: every reduction is a fixed-shape tree.
@@ -99,9 +101,11 @@ __device__ __forceinline__ void block_fold(double (&v)[NV], double* part, int np
     part[threadIdx.x * nparts_stride + blockIdx.x] = a;
   }
 }
+// one block folds every quantity (CG), or one block per quantity (GMRES's batch of dot products); either way each sum has the
+// same fixed order
 __global__ void __launch_bounds__(256) fold_partials_kernel(const double* __restrict__ part, int nparts, int nv, double* __restrict__ out) {
   __shared__ double sh[256];
-  for (int q = 0; q < nv; q++) {
+  for (int q = blockIdx.x; q < nv; q += gridDim.x) {
     double a = 0.0;
     for (int i = threadIdx.x; i < nparts; i += 256) a += part[q * nparts + i];
     sh[threadIdx.x] = a;
@@ -144,6 +148,110 @@ __global__ void axpby_kernel(int n, double a, const double* __restrict__ x, doub
 }
 __global__ void mul_kernel(int n, const double* __restrict__ a, const double* __restrict__ b, double* __restrict__ y) {
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) y[i] = a[i] * b[i];
+}
+
+// ---- GMRES(m) with right Jacobi preconditioning ----
+// Scalars of a solve, kept on the device next to the Hessenberg matrix so that the host reads them with one copy.
+enum GmresState { kScale = 0, kEst, kFlag, kValid, kExec, kBeta2, kBnorm2, kWnorm2, kStateLen };
+// kFlag: why the Arnoldi burst stopped early (later kernels of the burst see it and return at once)
+enum GmresStop { kRunning = 0, kEstimateMet = 1, kHappy = 2, kSingular = 3, kNonFinite = 4 };
+
+// v_k = scale w (k >= 1; v_0 = r / beta), z = D^-1 v_k
+__global__ void __launch_bounds__(256) gmres_basis_kernel(int n, const double* __restrict__ st, const double* __restrict__ w,
+                                                          const double* __restrict__ dinv, double* __restrict__ vk, double* __restrict__ z) {
+  if (st[kFlag] != kRunning) return;
+  const double scale = st[kScale];
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const double v = w[i] * scale;
+    vk[i] = v; z[i] = dinv[i] * v;
+  }
+}
+// h_j = v_{j0+j} . w for j < nv <= KC: one pass over the basis, w read once per row, partials [KC][blocks]
+template <int KC>
+__global__ void __launch_bounds__(256) gmres_dot_kernel(int n, int nv, const double* __restrict__ st, const double* __restrict__ V, size_t ld,
+                                                        const double* __restrict__ w, double* __restrict__ part) {
+  if (st[kFlag] != kRunning) return;
+  double acc[KC];
+#pragma unroll
+  for (int j = 0; j < KC; j++) acc[j] = 0.0;
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    const double wi = w[i];
+#pragma unroll
+    for (int j = 0; j < KC; j++) if (j < nv) acc[j] = fma(V[j * ld + i], wi, acc[j]);
+  }
+  block_fold<KC>(acc, part, gridDim.x);
+}
+// w -= sum_j h_j v_j (j <= k, classical Gram-Schmidt) and the partials of |w|^2
+__global__ void __launch_bounds__(256) gmres_update_kernel(int n, int nv, const double* __restrict__ st, const double* __restrict__ V, size_t ld,
+                                                           const double* __restrict__ h, double* __restrict__ w, double* __restrict__ part) {
+  if (st[kFlag] != kRunning) return;
+  double v[1] = {0.0};
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    double s = 0.0;
+    for (int j = 0; j < nv; j++) s = fma(h[j], V[j * ld + i], s);
+    const double wi = w[i] - s;
+    w[i] = wi;
+    v[0] = fma(wi, wi, v[0]);
+  }
+  block_fold<1>(v, part, gridDim.x);
+}
+// start of a cycle: g = beta e_1, v_0 = r / beta
+__global__ void gmres_start_kernel(int m, double* __restrict__ st, double* __restrict__ g) {
+  if (threadIdx.x != 0) return;
+  const double beta = sqrt(st[kBeta2]);
+  for (int i = 0; i <= m; i++) g[i] = 0.0;
+  g[0] = beta;
+  st[kScale] = 1.0 / beta; st[kEst] = beta;
+  st[kFlag] = kRunning; st[kValid] = 0; st[kExec] = 0;
+}
+// Arnoldi tail of column k (one warp; the work is O(k)): store the column of H, apply the earlier Givens rotations, make the new one,
+// update g and the residual estimate |g_{k+1}|, and raise the stop flag.  Nothing non-finite is stored: such a column stops the
+// burst with kNonFinite before it counts, so the solution update only ever sees finite columns.
+__global__ void gmres_tail_kernel(int k, int m, double target, const double* __restrict__ hd, double* __restrict__ st, double* __restrict__ H,
+                                  double* __restrict__ cs, double* __restrict__ sn, double* __restrict__ g) {
+  if (threadIdx.x != 0 || st[kFlag] != kRunning) return;
+  st[kExec] = k + 1;
+  const double hn = sqrt(st[kWnorm2]);
+  bool finite = isfinite(hn);
+  for (int i = 0; i <= k; i++) finite = finite && isfinite(hd[i]);
+  if (!finite) { st[kFlag] = kNonFinite; return; }
+  double* col = H + (size_t)k * (m + 1);
+  for (int i = 0; i <= k; i++) col[i] = hd[i];
+  col[k + 1] = hn;
+  for (int i = 0; i < k; i++) {
+    const double a = col[i], b = col[i + 1];
+    col[i] = cs[i] * a + sn[i] * b;
+    col[i + 1] = -sn[i] * a + cs[i] * b;
+  }
+  const double r = hypot(col[k], hn);
+  if (!(r > 0.0)) { st[kFlag] = kSingular; return; }          // A D^-1 v_k = 0: the column cannot enter the least-squares solve
+  cs[k] = col[k] / r; sn[k] = hn / r;
+  col[k] = r; col[k + 1] = 0.0;
+  g[k + 1] = -sn[k] * g[k];
+  g[k] = cs[k] * g[k];
+  st[kValid] = k + 1;
+  st[kEst] = fabs(g[k + 1]);
+  st[kScale] = hn > 0.0 ? 1.0 / hn : 0.0;
+  if (hn == 0.0) st[kFlag] = kHappy;
+  else if (fabs(g[k + 1]) <= target) st[kFlag] = kEstimateMet;
+}
+// y = R^-1 g over the first kv columns (back substitution, one thread)
+__global__ void gmres_ysolve_kernel(int kv, int m, const double* __restrict__ H, const double* __restrict__ g, double* __restrict__ y) {
+  if (threadIdx.x != 0) return;
+  for (int i = kv - 1; i >= 0; i--) {
+    double s = g[i];
+    for (int j = i + 1; j < kv; j++) s -= H[(size_t)j * (m + 1) + i] * y[j];
+    y[i] = s / H[(size_t)i * (m + 1) + i];
+  }
+}
+// x += D^-1 V y
+__global__ void __launch_bounds__(256) gmres_xupdate_kernel(int n, int kv, const double* __restrict__ V, size_t ld, const double* __restrict__ y,
+                                                            const double* __restrict__ dinv, double* __restrict__ x) {
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+    double s = 0.0;
+    for (int j = 0; j < kv; j++) s = fma(y[j], V[j * ld + i], s);
+    x[i] = fma(dinv[i], s, x[i]);
+  }
 }
 
 struct Pattern { int nrows; int64_t nnz; const int* rowptr; const int* colidx; int bs; };
@@ -274,5 +382,123 @@ extern "C" int petiga_cuda_solve_cg(petiga_cuda_plan* P, int block, const double
   PC_CUDA(cudaGetLastError());
   if (iters_out) *iters_out = it;
   if (relres_out) *relres_out = bnorm > 0 ? rnorm / bnorm : rnorm;
+  return 0;
+}
+
+extern "C" int petiga_cuda_solve_gmres(petiga_cuda_plan* P, int block, const double* values, const double* b, double* x, int restart, double rtol,
+                                       double atol, int maxit, int* iters_out, double* relres_out, int* reason_out) {
+  if (!P || !values || !b || !x || !iters_out || !relres_out || !reason_out || b == x || restart < 1 || maxit < 0) return PETIGA_CUDA_ERR_ARG;
+  PC_CUDA(cudaSetDevice(P->device));
+  nvtx_push("petiga_cuda_solve_gmres");
+  struct Pop { ~Pop() { nvtx_pop(); } } pop;
+  const Layout& L = P->L;
+  Pattern pt;
+  int rc = get_pattern(P, block, pt);
+  if (rc) return rc;
+  if (pt.bs > 4) { set_error("solve_gmres: block size > 4 (use the AIJ layout)"); return PETIGA_CUDA_ERR_SUP; }
+  const int n = pt.nrows * pt.bs, m = restart;
+  const size_t ld = (size_t)std::max(n, 1);
+  const int kc = 32;                                           // basis vectors per pass of the multi-dot
+  const int npass = (m + 1 + kc - 1) / kc;
+  // basis V[m+1], w, z, 1/diag, partials [npass*32][blocks], H[m][m+1], cs, sn, g, y, h, state; kept with the plan
+  const size_t nsmall = (size_t)m * (m + 1) + 2 * (size_t)m + 2 * (size_t)(m + 1) + (size_t)npass * kc + kStateLen;
+  const size_t need = (size_t)(m + 4) * ld + (size_t)npass * kc * kDotBlocks + nsmall;
+  if (P->gmres_work_cap < need) {
+    cudaFree(P->d_gmres_work);
+    P->d_gmres_work = nullptr; P->gmres_work_cap = 0;
+    PC_CUDA(cudaMalloc(&P->d_gmres_work, need * sizeof(double)));
+    P->gmres_work_cap = need;
+  }
+  double *V = P->d_gmres_work, *w = V + (size_t)(m + 1) * ld, *z = w + ld, *dinv = z + ld, *part = dinv + ld;
+  double *H = part + (size_t)npass * kc * kDotBlocks, *cs = H + (size_t)m * (m + 1), *sn = cs + m, *g = sn + m, *y = g + m + 1;
+  double *hd = y + m + 1, *st = hd + (size_t)npass * kc;
+  cudaStream_t s = P->stream;
+  const int gb = std::max(1, std::min((n + 255) / 256, kDotBlocks));
+  const bool multi = L.nranks > 1;
+  auto reduce = [&](int nv, double* out) -> int {              // partials -> out[0..nv) (+ sum over ranks)
+    fold_partials_kernel<<<nv, 256, 0, s>>>(part, gb, nv, out);
+    PC_CUDA(cudaGetLastError());
+    P->launches++;
+    return multi ? allreduce_sum(P, out, nv) : 0;
+  };
+  auto true_residual = [&]() -> int {                          // w = b - A x, st[kBeta2] = |w|^2
+    if (int e = spmv(P, pt, values, x, w)) return e;
+    axpby_kernel<<<gb, 256, 0, s>>>(n, 1.0, b, -1.0, w);
+    dot2_kernel<<<gb, 256, 0, s>>>(n, w, w, w, w, part);
+    P->launches += 2;
+    return reduce(1, st + kBeta2);
+  };
+  double h[kStateLen];
+  auto read_state = [&]() -> int {
+    PC_CUDA(cudaMemcpyAsync(h, st, sizeof(h), cudaMemcpyDeviceToHost, s));
+    PC_CUDA(cudaStreamSynchronize(s));
+    return 0;
+  };
+
+  if (n > 0) diag_inv_kernel<<<(n + 255) / 256, 256, 0, s>>>(pt.nrows, pt.bs, L.rank_start[L.rank] * L.dof, pt.rowptr, pt.colidx, values, dinv);
+  dot2_kernel<<<gb, 256, 0, s>>>(n, b, b, b, b, part);
+  P->launches += 2;
+  if ((rc = reduce(1, st + kBnorm2))) return rc;
+  if ((rc = true_residual()) || (rc = read_state())) return rc;
+  const double bnorm = std::sqrt(h[kBnorm2]);
+  const double target = std::max(rtol * bnorm, atol);
+  *iters_out = 0; *relres_out = 0.0;
+  if (!std::isfinite(bnorm)) { *relres_out = bnorm; *reason_out = PETIGA_KSP_DIVERGED_NANORINF; return 0; }
+  if (bnorm == 0.0) {                                          // b = 0: the solution is x = 0 (KSPSolve does the same)
+    PC_CUDA(cudaMemsetAsync(x, 0, (size_t)n * sizeof(double), s));
+    PC_CUDA(cudaStreamSynchronize(s));
+    *reason_out = PETIGA_KSP_CONVERGED_ATOL;
+    return 0;
+  }
+  int its = 0, stop = kRunning;
+  const int check = 10;
+  for (;;) {
+    // convergence is decided on the true residual only, once per cycle
+    const double rnorm = std::sqrt(h[kBeta2]);
+    *relres_out = rnorm / bnorm;
+    if (!std::isfinite(rnorm)) { *reason_out = PETIGA_KSP_DIVERGED_NANORINF; break; }
+    if (rnorm <= target) { *reason_out = rnorm <= rtol * bnorm ? PETIGA_KSP_CONVERGED_RTOL : PETIGA_KSP_CONVERGED_ATOL; break; }
+    if (stop == kNonFinite) { *reason_out = PETIGA_KSP_DIVERGED_NANORINF; break; }
+    if (stop == kHappy || stop == kSingular) { *reason_out = PETIGA_KSP_DIVERGED_BREAKDOWN; break; }
+    if (its >= maxit) { *reason_out = PETIGA_KSP_DIVERGED_ITS; break; }
+    gmres_start_kernel<<<1, 32, 0, s>>>(m, st, g);
+    P->launches++;
+    int k = 0;
+    stop = kRunning;
+    while (stop == kRunning && k < m && its + k < maxit) {
+      const int burst = std::min(check, std::min(m - k, maxit - its - k));
+      for (int q = k; q < k + burst; q++) {
+        gmres_basis_kernel<<<gb, 256, 0, s>>>(n, st, w, dinv, V + q * ld, z);
+        if ((rc = spmv(P, pt, values, z, w))) return rc;
+        for (int p = 0; p * kc <= q; p++) {
+          const int nv = std::min(kc, q + 1 - p * kc);
+          const double* Vp = V + (size_t)p * kc * ld;
+          double* pp = part + (size_t)p * kc * gb;
+          if (nv <= 8) gmres_dot_kernel<8><<<gb, 256, 0, s>>>(n, nv, st, Vp, ld, w, pp);
+          else if (nv <= 16) gmres_dot_kernel<16><<<gb, 256, 0, s>>>(n, nv, st, Vp, ld, w, pp);
+          else gmres_dot_kernel<32><<<gb, 256, 0, s>>>(n, nv, st, Vp, ld, w, pp);
+          P->launches++;
+        }
+        if ((rc = reduce(q + 1, hd))) return rc;
+        gmres_update_kernel<<<gb, 256, 0, s>>>(n, q + 1, st, V, ld, hd, w, part);
+        if ((rc = reduce(1, st + kWnorm2))) return rc;
+        gmres_tail_kernel<<<1, 32, 0, s>>>(q, m, target, hd, st, H, cs, sn, g);
+        P->launches += 3;
+      }
+      if ((rc = read_state())) return rc;
+      stop = (int)h[kFlag];
+      k = (int)h[kExec];
+    }
+    its += k;
+    const int kv = (int)h[kValid];
+    if (kv > 0) {
+      gmres_ysolve_kernel<<<1, 32, 0, s>>>(kv, m, H, g, y);
+      gmres_xupdate_kernel<<<gb, 256, 0, s>>>(n, kv, V, ld, y, dinv, x);
+      P->launches += 2;
+    }
+    if ((rc = true_residual()) || (rc = read_state())) return rc;
+  }
+  PC_CUDA(cudaGetLastError());
+  *iters_out = its;
   return 0;
 }

@@ -40,6 +40,11 @@ _SETTERS = {"VECTOR": "IGASetFormVector", "MATRIX": "IGASetFormMatrix", "SYSTEM"
             "I2JACOBIAN": "IGASetFormI2Jacobian"}
 
 
+# KSPConvergedReason values (PETSc's; include/petiga_host.h)
+KSP_CONVERGED_ITERATING, KSP_CONVERGED_RTOL, KSP_CONVERGED_ATOL = 0, 2, 3
+KSP_DIVERGED_ITS, KSP_DIVERGED_BREAKDOWN, KSP_DIVERGED_NANORINF = -3, -5, -9
+
+
 class IGAComm(C.Structure):
     _fields_ = [("rank", C.c_int), ("size", C.c_int), ("nccl", C.c_void_p), ("device", C.c_int)]
 
@@ -431,18 +436,27 @@ class IGA:
     def MatMult(self, A, x, y):
         _chk(self.H.MatMult(A.h, x.h, y.h))
 
-    def Solve(self, A, b, x, rtol=1e-8, atol=1e-50, maxits=10000):
-        """IGACreateKSP + KSPSetOperators + KSPSetTolerances + KSPSolve (demo/Poisson3D.c:73-83) on the device: CG + Jacobi.
-        Returns (iterations, |r| / |b|)."""
+    def Solve(self, A, b, x, rtol=1e-8, atol=1e-50, maxits=10000, ksp_type="cg", restart=30, return_reason=False):
+        """IGACreateKSP + KSPSetType + KSPSetOperators + KSPSetTolerances + KSPSolve (demo/Poisson3D.c:73-83) on the device with
+        the Jacobi preconditioner: ksp_type "cg" (symmetric positive definite A) or "gmres" (GMRES(restart), any A with a nonzero
+        diagonal).  Returns (iterations, |b - A x| / |b|), or (iterations, |b - A x| / |b|, KSPConvergedReason value) with
+        return_reason=True."""
         ksp = C.c_void_p()
         _chk(self.H.IGACreateKSP(self.h, C.byref(ksp)))
         try:
+            if ksp_type != "cg":
+                _chk(self.H.KSPSetType(ksp, C.c_char_p(ksp_type.encode())))
+            if restart != 30:
+                _chk(self.H.KSPGMRESSetRestart(ksp, int(restart)))
             _chk(self.H.KSPSetOperators(ksp, A.h, A.h))
             _chk(self.H.KSPSetTolerances(ksp, C.c_double(rtol), C.c_double(atol), C.c_double(1e5), int(maxits)))
             _chk(self.H.KSPSolve(ksp, b.h, x.h))
-            its, rn = C.c_int(), C.c_double()
+            its, rn, reason = C.c_int(), C.c_double(), C.c_int()
             _chk(self.H.KSPGetIterationNumber(ksp, C.byref(its)))
             _chk(self.H.KSPGetResidualNorm(ksp, C.byref(rn)))
+            if return_reason:
+                _chk(self.H.KSPGetConvergedReason(ksp, C.byref(reason)))
+                return its.value, rn.value, reason.value
             return its.value, rn.value
         finally:
             self.H.KSPDestroy(C.byref(ksp))
