@@ -84,7 +84,12 @@ enum {
   PETIGA_FORM_ELASTICROD = 14,    /* demo/ElasticRodFJ.F90 I2Function/I2Jacobian; params = {rho, E}                        */
   PETIGA_FORM_NITSCHE = 15,       /* demo/NitscheMethod.c:70-119 System: Poisson inside, Nitsche matrix + vector terms on the
                                      faces enabled with petiga_cuda_set_boundary_form                                       */
-  PETIGA_NFORMS = 16              /* PETIGA_FORM_BRATU also provides RHSFunction/RHSJacobian (its explicit form)            */
+  /* isogeometric collocation (petiga_cuda_space.collocation = 1): the strong form at the Greville points; slots VECTOR, MATRIX,
+     SYSTEM, dof 1.  A Galerkin form on a collocation plan, or one of these on a Galerkin plan, is PETIGA_CUDA_ERR_SUP */
+  PETIGA_FORM_LAPLACE_COLLOCATION = 16,   /* demo/Laplace.c SystemCollocation: K[a] = -Lap N_a, F = 0                                 */
+  PETIGA_FORM_CONVTEST_COLLOCATION = 17,  /* strong form of test/ConvTest.c: K[a] = c N_a - k Lap N_a,
+                                             F = (c + k dim pi^2) prod sin(pi x_i); params = {c, k}                                 */
+  PETIGA_NFORMS = 18              /* PETIGA_FORM_BRATU also provides RHSFunction/RHSJacobian (its explicit form)            */
 };
 
 /* built-in Scalar callbacks of petiga_cuda_compute_scalar (IGAComputeScalar, src/petigacomp.c:35-96) */
@@ -102,7 +107,8 @@ enum {
 enum {
   PETIGA_PATH_AUTO = 0,           /* Kronecker row-gather when the form/geometry is separable, else quadrature     */
   PETIGA_PATH_QUADRATURE = 1,     /* always the per-element quadrature kernels (the reference's formulation)       */
-  PETIGA_PATH_KRONECKER = 2       /* force the separable path; PETIGA_CUDA_ERR_SUP when not applicable             */
+  PETIGA_PATH_KRONECKER = 2,      /* force the separable path; PETIGA_CUDA_ERR_SUP when not applicable             */
+  PETIGA_PATH_COLLOCATION = 3     /* stat "last_path" only: the collocation kernel of a collocation plan ran              */
 };
 /* quadrature kernel selection (petiga_cuda_set_option "quad_impl"): -1 = by element size; 0 = sum-factorised; 1 = pair loop;
    2 = generic runtime-degree kernel (mixed degrees, degree <= 8, dof <= 8, second derivatives on mapped / NURBS geometry,
@@ -125,6 +131,12 @@ typedef struct {
   int elem_start[3], elem_width[3];    /* this rank's element box       (src/petigapart.c:170-202)         */
   int node_lstart[3], node_lwidth[3];  /* owned node box                (src/petiga.c:1186-1209)           */
   int node_gstart[3], node_gwidth[3];  /* ghost node box                                                   */
+  int collocation;                     /* IGASetUseCollocation (0 = Galerkin).  The tables then hold one point per basis
+                                          function -- its Greville abscissa: nnp entries, nqp1 = 1, offset[i] = span - p,
+                                          weight = detJac = 1, value = the basis and its derivatives there -- and the element box
+                                          is the owned node box.  The partition and numbering stay the Galerkin ones (from the
+                                          knot spans); the ghost box is the union of the owned rows' stencils.  nel may be
+                                          the table length nnp (IGABasis.nel) or the axis's element count (IGAAxis.nel). */
 } petiga_cuda_space;   /* the boxes of the other ranks follow from (nel, offset, proc_sizes) by the same arithmetic */
 
 /* IGAFormBC tables (include/petiga.h:221-225) + the fix table */
@@ -156,6 +168,7 @@ int petiga_cuda_plan_destroy(petiga_cuda_plan *plan);
             1 shared-memory window always), "sf3_static" (1 use the compiled-in form structures when the run-time lists match),
             "kron_minb_rows" (scalar separable kernel: pencil length from which the 3-CTA build runs), "kron_bulk" (1: cp.async.bulk row
             stores, measured slower), "scatter" (99: integrate but skip the global reductions, profiling only)
+   A collocation plan (petiga_cuda_space.collocation) always runs the collocation kernel; "path" = 2 is PETIGA_CUDA_ERR_SUP there.
    stats:   "launches", "last_path", "last_impl", "last_sf3_variant", "last_sf3_static", "last_kernel_ms", "last_flops", "num_sms",
             "nghostrows", "nnz_loc" */
 int petiga_cuda_set_option(petiga_cuda_plan *plan, const char *name, double value);

@@ -93,6 +93,9 @@ PetscErrorCode IGADeviceForm_Mass_Vector(IGAPoint, PetscScalar *, void *);      
 PetscErrorCode IGADeviceForm_BoundaryIntegral_System(IGAPoint, PetscScalar *, PetscScalar *, void *);   /* demo/BoundaryIntegral.c:50-57 System (Laplace + face term) */
 PetscErrorCode IGADeviceForm_Neumann_SystemGalerkin(IGAPoint, PetscScalar *, PetscScalar *, void *);    /* demo/Neumann.c:28-45                                       */
 PetscErrorCode IGADeviceForm_ConvTest_Galerkin(IGAPoint, PetscScalar *, PetscScalar *, void *);         /* test/ConvTest.c:51-69; ctx: {c, k}                         */
+/* collocation forms (IGASetUseCollocation): the strong form at each Greville point, K[a] and F of one row per node */
+PetscErrorCode IGADeviceForm_Laplace_SystemCollocation(IGAPoint, PetscScalar *, PetscScalar *, void *);  /* demo/Laplace.c SystemCollocation: -Lap N_a */
+PetscErrorCode IGADeviceForm_ConvTest_Collocation(IGAPoint, PetscScalar *, PetscScalar *, void *);      /* c N_a - k Lap N_a, F = (c + k dim pi^2) prod sin(pi x_i); ctx: {c, k} */
 PetscErrorCode IGADeviceForm_Elasticity3D_System(IGAPoint, PetscScalar *, PetscScalar *, void *);       /* ctx: {lambda, mu}                   */
 PetscErrorCode IGADeviceForm_Elasticity_System(IGAPoint, PetscScalar *, PetscScalar *, void *);         /* ctx: {mu, lambda} as demo/Elasticity.c:10-13 */
 PetscErrorCode IGADeviceForm_CahnHilliard2D_Residual(IGAPoint, PetscReal, const PetscScalar *, PetscReal, const PetscScalar *, PetscScalar *, void *); /* ctx: {theta, alpha} */
@@ -136,6 +139,15 @@ PetscErrorCode IGASetProcessors(IGA iga, PetscInt i, PetscInt processors);
 PetscErrorCode IGAGetAxis(IGA iga, PetscInt i, IGAAxis *axis);
 PetscErrorCode IGASetRuleSize(IGA iga, PetscInt i, PetscInt nqp);
 PetscErrorCode IGASetMatType(IGA iga, const char *mattype);            /* "aij" or "baij" (petiga.c:1326-1330 default) */
+/* Isogeometric collocation instead of Galerkin (-iga_collocation).  Before IGASetUp; changing it afterwards is
+   PETSC_ERR_ARG_WRONGSTATE.  IGASetUp then tabulates one point per basis function (its Greville abscissa, nel = nnp, one
+   point, weight = detJac = 1), keeps the Galerkin partition and numbering, takes the owned node box as the element box and the
+   union of the owned rows' stencils as the ghost box.  Collocation runs the collocation forms (IGADeviceForm_*Collocation) in
+   the VECTOR, MATRIX and SYSTEM slots, dof 1, degree 2..8, non-periodic axes; IGAComputeSystem replaces the row of a node that
+   carries an IGASetBoundaryValue by an identity row with F = the value.  Boundary loads, boundary forms, fix tables and the
+   separable path are PETSC_ERR_SUP.  The matrix is not symmetric: solve it with KSPGMRES. */
+PetscErrorCode IGASetUseCollocation(IGA iga, PetscBool collocation);
+PetscErrorCode IGAGetUseCollocation(IGA iga, PetscBool *collocation);
 PetscErrorCode IGASetUp(IGA iga);
 /* geometry in natural ordering, i fastest, (n_d+1) control points per axis: X[..][nsd], W[..] or NULL.
    Stands in for IGALoadGeometry (src/petigaio.c:201-286), which reads the same arrays from a PETSc binary file. */

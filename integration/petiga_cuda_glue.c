@@ -45,6 +45,9 @@ static PetscErrorCode IGAGetCudaPlan(IGA iga, petiga_cuda_plan **plan)
       sp.node_lstart[i] = iga->node_lstart[i]; sp.node_lwidth[i] = iga->node_lwidth[i];
       sp.node_gstart[i] = iga->node_gstart[i]; sp.node_gwidth[i] = iga->node_gwidth[i];
     }
+    sp.collocation = iga->collocation;                                                  /* IGASetUseCollocation: the basis tables
+                                                                                           and boxes above are then the collocation ones
+                                                                                           (nnp entries; nel = ax->nel is accepted) */
     if (size > 1) {                                                                     /* one rank per GPU; the id travels over MPI */
       if (!rank) PetscCheck(!petiga_cuda_comm_unique_id(id), comm, PETSC_ERR_LIB, "%s", petiga_cuda_last_error());
       PetscCallMPI(MPI_Bcast(id, 128, MPI_BYTE, 0, comm));

@@ -35,7 +35,8 @@ typedef struct { struct { void *System, *Function, *Jacobian, *IFunction, *IJaco
                  IGAFormBC value[3][2], load[3][2]; PetscBool visit[3][2]; } *IGAForm;
 struct _p_IGA { PetscInt dim, dof, order; IGAAxis axis[3]; IGABasis basis[3]; IGAForm form;
                 PetscInt proc_sizes[3], proc_ranks[3], elem_start[3], elem_width[3], node_lstart[3], node_lwidth[3], node_gstart[3], node_gwidth[3];
-                PetscInt geometry; PetscBool rational, fixtable; PetscReal *geometryX, *rationalW; PetscScalar *fixtableU; };
+                PetscInt geometry; PetscBool rational, fixtable; PetscReal *geometryX, *rationalW; PetscScalar *fixtableU;
+                PetscBool collocation; };
 typedef struct _p_IGA *IGA;
 extern PetscLogEvent IGA_FormSystem, IGA_FormFunction, IGA_FormJacobian, IGA_FormIFunction, IGA_FormIJacobian, IGA_FormVector, IGA_FormMatrix, IGA_FormScalar;
 PetscErrorCode IGAGetComm(IGA, MPI_Comm *);

@@ -4,6 +4,7 @@
 //   knot vectors        IGAAxisInitUniform / IGAAxisSetKnots   (ref: src/petigaaxis.c:401-480)
 //   Gauss rule + 1-D basis tables  IGABasisInitQuadrature      (ref: src/petigabasis.c:83-219, petigabsb.f90.in)
 //   processor grid + boxes         IGA_Partition / Stage1      (ref: src/petigapart.c, src/petiga.c:1111-1209)
+//   collocation tables + boxes     IGASetUseCollocation: one point per basis function, its Greville abscissa
 // Everything per-element runs on the GPU through libpetiga_cuda; there is no CPU assembly path here.
 #include <cmath>
 #include <cstdint>
@@ -56,6 +57,7 @@ struct _p_KSP {      // IGACreateKSP: conjugate gradients (petiga_cuda_solve_cg)
 struct _p_IGA {
   IGAComm comm;
   int dim = -1, dof = -1, order = -1, setup = 0;
+  int collocation = 0;   // IGASetUseCollocation
   _n_IGAAxis axis[3];
   int rule_nqp[3] = {0, 0, 0};
   int proc_user[3] = {-1, -1, -1};
@@ -204,7 +206,7 @@ PetscErrorCode fill_space(IGA g, petiga_cuda_space& sp) {
   sp.dim = g->dim; sp.dof = g->dof; sp.order = g->order;
   for (int d = 0; d < 3; d++) {
     const _n_IGAAxis& ax = g->axis[d];
-    sp.p[d] = ax.p; sp.m[d] = ax.m; sp.nel[d] = ax.nel; sp.nnp[d] = ax.nnp; sp.periodic[d] = ax.periodic; sp.nqp1[d] = g->nqp[d];
+    sp.p[d] = ax.p; sp.m[d] = ax.m; sp.nel[d] = g->collocation ? ax.nnp : ax.nel; sp.nnp[d] = ax.nnp; sp.periodic[d] = ax.periodic; sp.nqp1[d] = g->nqp[d];
     sp.U[d] = ax.U.data(); sp.offset[d] = g->offset[d].data(); sp.detJac[d] = g->detJac[d].data();
     sp.weight[d] = g->weight[d].data(); sp.point[d] = g->point[d].data(); sp.value[d] = g->value[d].data();
     sp.proc_sizes[d] = g->proc_sizes[d]; sp.proc_ranks[d] = g->proc_ranks[d];
@@ -212,6 +214,7 @@ PetscErrorCode fill_space(IGA g, petiga_cuda_space& sp) {
     sp.node_lstart[d] = g->node_lstart[d]; sp.node_lwidth[d] = g->node_lwidth[d];
     sp.node_gstart[d] = g->node_gstart[d]; sp.node_gwidth[d] = g->node_gwidth[d];
   }
+  sp.collocation = g->collocation;
   return 0;
 }
 
@@ -286,6 +289,8 @@ const FormEntry* lookup_form(const void* fn, int slot) {
       {FN(IGADeviceForm_BoundaryIntegral_System), PETIGA_SLOT_SYSTEM, PETIGA_FORM_BOUNDARYINTEGRAL, 0, 0},
       {FN(IGADeviceForm_Neumann_SystemGalerkin), PETIGA_SLOT_SYSTEM, PETIGA_FORM_NEUMANN, 0, 0},
       {FN(IGADeviceForm_ConvTest_Galerkin), PETIGA_SLOT_SYSTEM, PETIGA_FORM_CONVTEST, 2, 0},
+      {FN(IGADeviceForm_Laplace_SystemCollocation), PETIGA_SLOT_SYSTEM, PETIGA_FORM_LAPLACE_COLLOCATION, 0, 0},
+      {FN(IGADeviceForm_ConvTest_Collocation), PETIGA_SLOT_SYSTEM, PETIGA_FORM_CONVTEST_COLLOCATION, 2, 0},
       {FN(IGADeviceForm_Mass_Matrix), PETIGA_SLOT_MATRIX, PETIGA_FORM_MASS, 0, 0},
       {FN(IGADeviceForm_Mass_Vector), PETIGA_SLOT_VECTOR, PETIGA_FORM_MASS, 0, 0},
       {FN(IGADeviceForm_Elasticity3D_System), PETIGA_SLOT_SYSTEM, PETIGA_FORM_ELASTICITY3D, 2, 0},
@@ -347,6 +352,7 @@ SENT4(IGADeviceForm_Poisson_System) SENTF(IGADeviceForm_Poisson_Function) SENTF(
 SENT4(IGADeviceForm_Laplace_System) SENT4(IGADeviceForm_L2Projection_System) SENT4(IGADeviceForm_Mass_System)
 SENT3(IGADeviceForm_Mass_Matrix) SENT3(IGADeviceForm_Mass_Vector)
 SENT4(IGADeviceForm_BoundaryIntegral_System) SENT4(IGADeviceForm_Neumann_SystemGalerkin) SENT4(IGADeviceForm_ConvTest_Galerkin)
+SENT4(IGADeviceForm_Laplace_SystemCollocation) SENT4(IGADeviceForm_ConvTest_Collocation)
 PetscErrorCode IGADeviceExact_ConvTest(IGAPoint, PetscInt, PetscScalar*, void*) { return host_sentinel(); }
 PetscErrorCode IGADeviceExact_Neumann(IGAPoint, PetscInt, PetscScalar*, void*) { return host_sentinel(); }
 SENT4(IGADeviceForm_Elasticity3D_System) SENT4(IGADeviceForm_Elasticity_System)
@@ -457,6 +463,20 @@ PetscErrorCode IGASetRuleSize(IGA g, PetscInt i, PetscInt nqp) {
   g->rule_nqp[i] = nqp;
   g->setup = 0;   // IGASetRuleSize resets the setup stage in the reference
   drop_plan(g);
+  return 0;
+}
+// include/petiga.h IGASetUseCollocation (src/petiga.c): chooses the discretisation before IGASetUp
+PetscErrorCode IGASetUseCollocation(IGA g, PetscBool flag) {
+  if (PetscErrorCode e = check(g)) return e;
+  const int c = flag ? 1 : 0;
+  if (g->setup && c != g->collocation) return fail(PETSC_ERR_ARG_WRONGSTATE, "Cannot change collocation after IGASetUp()");
+  g->collocation = c;
+  return 0;
+}
+PetscErrorCode IGAGetUseCollocation(IGA g, PetscBool* flag) {
+  if (PetscErrorCode e = check(g)) return e;
+  if (!flag) return fail(PETSC_ERR_ARG_NULL, "Null pointer");
+  *flag = g->collocation ? PETSC_TRUE : PETSC_FALSE;
   return 0;
 }
 PetscErrorCode IGASetMatType(IGA g, const char* t) {
@@ -593,7 +613,34 @@ PetscErrorCode IGASetUp(IGA g) {
     g->geom_sizes[d] = ax.span[nel - 1] + 1;
   }
   // Stage 3: rule + 1-D tables
-  for (int d = 0; d < 3; d++) {
+  for (int d = 0; d < 3 && g->collocation; d++) {   // collocation: one point per basis function, its Greville abscissa
+    const _n_IGAAxis& ax = g->axis[d];
+    const int p = ax.p, nnp = ax.nnp, nen = p + 1, n = ax.m - p - 1, nd = std::min(p, 4);
+    if (p > 8) return fail(PETSC_ERR_SUP, "degree > 8");
+    g->nqp[d] = 1;
+    g->offset[d].assign(nnp, 0); g->detJac[d].assign(nnp, 1.0);
+    g->weight[d].assign(nnp, 1.0); g->point[d].assign(nnp, 0.0);
+    g->value[d].assign((size_t)nnp * nen * 5, 0.0);
+    for (int i = 0; i < nnp; i++) {
+      double u = 0.0;
+      if (p > 0) {
+        for (int j = 1; j <= p; j++) u += ax.U[i + j];
+        u /= p;
+      }
+      int k = n;   // FindSpan (The NURBS Book A2.1): the largest k with U[k] <= u < U[k+1]; k = n at the right end
+      if (u < ax.U[n + 1]) { k = p; while (k < n && ax.U[k + 1] <= u) k++; }
+      g->offset[d][i] = k - p;
+      g->point[d][i] = u;
+      double ders[9][5];
+      bspline_ders(k, u, p, nd, ax.U.data(), ders);
+      for (int a = 0; a < nen; a++) for (int dd = 0; dd < 5; dd++) g->value[d][((size_t)i * nen + a) * 5 + dd] = ders[a][dd];
+    }
+    // element box = owned node box; ghost box = union of the owned rows' stencils [offset, offset + p]
+    g->elem_start[d] = g->node_lstart[d]; g->elem_width[d] = g->node_lwidth[d];
+    const int lo = g->offset[d][g->node_lstart[d]], hi = g->offset[d][g->node_lstart[d] + g->node_lwidth[d] - 1] + p + 1;
+    g->node_gstart[d] = lo; g->node_gwidth[d] = hi - lo;
+  }
+  for (int d = 0; d < 3 && !g->collocation; d++) {
     const _n_IGAAxis& ax = g->axis[d];
     const int p = ax.p, nel = ax.nel, nen = p + 1, nd = std::min(p, 4);
     int q = (d < g->dim) ? g->rule_nqp[d] : 0;
@@ -811,10 +858,34 @@ PetscErrorCode VecGetArrayHost(Vec v, PetscScalar* out) { if (!v || !out) return
 PetscErrorCode VecSetArrayHost(Vec v, const PetscScalar* in) { if (!v || !in) return fail(PETSC_ERR_ARG_NULL, "Null"); if (PetscErrorCode e = check_owner(v, nullptr, "Vec")) return e; if (v->iga->plan) petiga_cuda_plan_activate(v->iga->plan); return from_cuda(petiga_cuda_memcpy_h2d(v->d, in, (size_t)v->n * sizeof(double))); }
 PetscErrorCode VecGetArrayDevice(Vec v, PetscScalar** d) { if (!v || !d) return fail(PETSC_ERR_ARG_NULL, "Null"); *d = v->d; return 0; }
 
+// what the collocation kernel supports, checked before any device work (the library repeats the checks for direct callers)
+static PetscErrorCode check_collocation(IGA g, int slot) {
+  const int f = g->slots[slot].form;
+  const bool cform = f == PETIGA_FORM_LAPLACE_COLLOCATION || f == PETIGA_FORM_CONVTEST_COLLOCATION;
+  if (!g->collocation) {
+    if (cform) return fail(PETSC_ERR_SUP, "a collocation form needs IGASetUseCollocation(iga, PETSC_TRUE)");
+    return 0;
+  }
+  if (slot != PETIGA_SLOT_VECTOR && slot != PETIGA_SLOT_MATRIX && slot != PETIGA_SLOT_SYSTEM)
+    return fail(PETSC_ERR_SUP, "collocation: only IGAComputeVector/Matrix/System run on the device");
+  if (!cform) return fail(PETSC_ERR_SUP, "collocation: pass one of the IGADeviceForm_*Collocation sentinels (Galerkin forms integrate)");
+  if (g->dof != 1) return fail(PETSC_ERR_SUP, "collocation: the device forms have dof 1");
+  for (int d = 0; d < g->dim; d++)
+    for (int s = 0; s < 2; s++) {
+      if (g->bc.lcount[d][s]) return fail(PETSC_ERR_SUP, "collocation: IGASetBoundaryLoad is not supported");
+      if (g->visit[d][s]) return fail(PETSC_ERR_SUP, "collocation: IGASetBoundaryForm is not supported");
+    }
+  if (g->fixtable) return fail(PETSC_ERR_SUP, "collocation: IGASetFixTable is not supported");
+  for (auto& o : g->options)
+    if (o.first == "path" && (int)o.second == PETIGA_PATH_KRONECKER) return fail(PETSC_ERR_SUP, "collocation: the separable path does not apply");
+  return 0;
+}
+
 static PetscErrorCode run(IGA g, int slot, PetscReal a, Vec V, PetscReal t, Vec U, Mat A, Vec B, PetscReal a2 = 0, Vec W = nullptr, PetscReal t0 = 0) {
   if (PetscErrorCode e = check(g)) return e;
   if (!g->setup) return fail(PETSC_ERR_ARG_WRONGSTATE, "Must call IGASetUp() first");                     // IGACheckSetUp
   if (g->slots[slot].form < 0) return fail(PETSC_ERR_USER, "Must call IGASetForm*() first");
+  if (PetscErrorCode e = check_collocation(g, slot)) return e;
   if (PetscErrorCode e = ensure_plan(g)) return e;
   if (A) if (PetscErrorCode e = check_owner(A, g, "Mat")) return e;
   for (Vec x : {V, U, B, W}) if (x) if (PetscErrorCode e = check_owner(x, g, "Vec")) return e;
@@ -958,8 +1029,8 @@ PetscErrorCode IGAGetInfoArray(IGA g, PetscInt info[46]) {
   if (PetscErrorCode e = check(g)) return e;
   int k = 0;
   info[k++] = g->order;
-  for (int d = 0; d < 3; d++) {
-    info[k++] = g->axis[d].p; info[k++] = g->axis[d].m; info[k++] = g->axis[d].nnp; info[k++] = g->axis[d].nel;
+  for (int d = 0; d < 3; d++) {   // nel: entries of the basis tables (nnp under collocation, as IGABasis.nel)
+    info[k++] = g->axis[d].p; info[k++] = g->axis[d].m; info[k++] = g->axis[d].nnp; info[k++] = (g->collocation && g->setup) ? g->axis[d].nnp : g->axis[d].nel;
     info[k++] = g->nqp[d]; info[k++] = g->axis[d].p + 1; info[k++] = g->proc_sizes[d]; info[k++] = g->proc_ranks[d];
     info[k++] = g->elem_start[d]; info[k++] = g->elem_width[d]; info[k++] = g->node_lstart[d]; info[k++] = g->node_lwidth[d];
     info[k++] = g->node_gstart[d]; info[k++] = g->node_gwidth[d]; info[k++] = g->geom_sizes[d];

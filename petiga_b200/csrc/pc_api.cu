@@ -467,6 +467,7 @@ int petiga_cuda_set_bc(petiga_cuda_plan* P, const petiga_cuda_bc* bc) {
 
 int petiga_cuda_set_fixtable_device(petiga_cuda_plan* P, const double* table_own) {
   if (!P) return PETIGA_CUDA_ERR_ARG;
+  if (P->L.collocation && table_own) { set_error("set_fixtable_device: IGASetFixTable is not supported on a collocation plan"); return PETIGA_CUDA_ERR_SUP; }
   PC_CUDA(cudaSetDevice(P->device));
   PC_CUDA(cudaStreamSynchronize(P->stream));
   cudaFree(P->d_fixtable);
@@ -602,6 +603,28 @@ int petiga_cuda_compute_ext(petiga_cuda_plan* P, int slot, int block, double shi
   if (has_v && !V) { set_error("compute: V == NULL"); return PETIGA_CUDA_ERR_ARG; }
   if (has_w && !W) { set_error("compute: the third vector (U0 / A) == NULL"); return PETIGA_CUDA_ERR_ARG; }
   if (fi.order > P->order) { set_error("compute: form reads derivatives above IGASetOrder"); return PETIGA_CUDA_ERR_ARG; }
+  if (L.collocation || fi.colloc) {   // isogeometric collocation: its own kernel, nothing else runs on such a plan
+    if (!L.collocation) { set_error("compute: a collocation form needs a collocation plan (IGASetUseCollocation)"); return PETIGA_CUDA_ERR_SUP; }
+    if (!fi.colloc) { set_error("compute: a collocation plan runs the collocation forms only (IGADeviceForm_*Collocation)"); return PETIGA_CUDA_ERR_SUP; }
+    if (P->path == PETIGA_PATH_KRONECKER) { set_error("compute: the separable path does not apply to collocation"); return PETIGA_CUDA_ERR_SUP; }
+    for (int d = 0; d < L.dim; d++)
+      for (int s = 0; s < 2; s++) {
+        if (P->visit[d][s]) { set_error("compute: IGASetBoundaryForm is not supported with collocation"); return PETIGA_CUDA_ERR_SUP; }
+        if (P->has_bc && P->bc.lcount[d][s]) { set_error("compute: IGASetBoundaryLoad is not supported with collocation"); return PETIGA_CUDA_ERR_SUP; }
+      }
+    if (P->d_fixtable) { set_error("compute: IGASetFixTable is not supported with collocation"); return PETIGA_CUDA_ERR_SUP; }
+    PC_CUDA(cudaSetDevice(P->device));
+    nvtx_push(slot);
+    cudaEventRecord(P->ev0, P->stream);
+    const int rc = launch_collocation(P, slot, form, values, rhs);
+    cudaEventRecord(P->ev1, P->stream);
+    nvtx_pop();
+    if (rc) return rc;
+    P->last_path = PETIGA_PATH_COLLOCATION;
+    P->last_impl = -1;
+    P->last_flops = 0;
+    return 0;
+  }
   PC_CUDA(cudaSetDevice(P->device));
   const int bs2 = L.dof * L.dof;
   const size_t nval = (size_t)L.nnz_own * bs2, nvec = (size_t)L.nown * L.dof;

@@ -55,6 +55,7 @@ struct FormInfo {
   int constant_f;     // vector coefficient is a constant (eligible for the separable path)
   int mat_const;      // matrix coefficient tensor does not depend on the point
   int bnd_mat, bnd_vec;   // the callback has a p->atboundary branch that adds matrix / vector terms on visited faces
+  int colloc;         // a collocation form (pc_colloc.cu): runs on collocation plans only, and nothing else runs there
 };
 
 __host__ __device__ inline FormInfo form_info(int form, int slot, int dim, int dof) {
@@ -130,6 +131,14 @@ __host__ __device__ inline FormInfo form_info(int form, int slot, int dim, int d
       if (dof != 1) break;
       if (slot == PETIGA_SLOT_I2FUNCTION) { f.valid = 1; f.vc0 = 0; f.vc1 = 1 + dim; f.per_qp = 1; f.needs_state = 1; f.order = 1; }
       if (slot == PETIGA_SLOT_I2JACOBIAN) { f.valid = 1; f.mc0 = 0; f.mc1 = 1 + dim; f.order = 1; }
+      break;
+    case PETIGA_FORM_LAPLACE_COLLOCATION:    // demo/Laplace.c SystemCollocation
+      if (dof != 1 || !lin) break;
+      f.valid = 1; f.colloc = 1; f.order = 2; f.constant_f = 1;
+      break;
+    case PETIGA_FORM_CONVTEST_COLLOCATION:   // strong form of test/ConvTest.c
+      if (dof != 1 || !lin) break;
+      f.valid = 1; f.colloc = 1; f.order = 2; f.needs_x = 1;
       break;
     case PETIGA_FORM_NITSCHE:           // demo/NitscheMethod.c:70-119: interior Poisson (f = -2 dim) + face terms
       if (dof != 1 || slot != PETIGA_SLOT_SYSTEM) break;

@@ -21,8 +21,14 @@ static int next_knot(int m, const double* U, int k, int direction) {
   return 0;
 }
 
-// Stencil(): src/petigamat.c:197-233 (non-collocation branch)
-static void stencil(const AxisLayout& a, const double* U, int i, int& first, int& last) {
+// Stencil(): src/petigamat.c:197-233.  Collocation branch: the p+1 basis functions that do not vanish at the row's point,
+// [offset[i], offset[i] + p] of the collocation table.
+static void stencil(const AxisLayout& a, const double* U, const int* offset, int collocation, int i, int& first, int& last) {
+  if (collocation) {
+    first = offset[i];
+    last = offset[i] + a.p;
+    return;
+  }
   const int p = a.p, m = a.m, n = m - p - 1;
   first = next_knot(m, U, i, +1) - p - 1;
   last = next_knot(m, U, i + p + 1, -1);
@@ -49,6 +55,7 @@ int build_layout(const petiga_cuda_space& sp, int rank, int nranks, Layout& L) {
   L.dof = sp.dof;
   L.rank = rank;
   L.nranks = nranks;
+  L.collocation = sp.collocation ? 1 : 0;
   if (sp.dim < 1 || sp.dim > 3) return fail(L, PETIGA_CUDA_ERR_ARG, "dim must be in [1,3]");
   if (sp.dof < 1 || sp.dof > 64) return fail(L, PETIGA_CUDA_ERR_ARG, "dof must be in [1,64]");
   int nprocs = 1;
@@ -71,17 +78,40 @@ int build_layout(const petiga_cuda_space& sp, int rank, int nranks, Layout& L) {
     if (!sp.U[d] || !sp.offset[d]) return fail(L, PETIGA_CUDA_ERR_ARG, "missing axis tables");
     const double* U = sp.U[d];
     const int* off = sp.offset[d];
+    // The partition runs on the Galerkin elements (the knot spans).  A collocation table holds one entry per node instead, so
+    // the Galerkin offsets are recovered from the knot vector: span k of every nonzero knot interval, offset k - p.
+    std::vector<int> span_off;
+    if (L.collocation) {
+      if (a.periodic) return fail(L, PETIGA_CUDA_ERR_SUP, "collocation: periodic axes are not supported on the device path");
+      if (d < sp.dim && a.p < 2) return fail(L, PETIGA_CUDA_ERR_SUP, "collocation: degree must be in [2,8] (second derivatives at the points)");
+      for (int k = a.p; k <= a.m - a.p - 1; k++)
+        if (U[k] < U[k + 1]) span_off.push_back(k - a.p);
+      if (span_off.empty()) return fail(L, PETIGA_CUDA_ERR_ARG, "collocation: knot vector without a nonzero span");
+      // nel may be the table length (IGABasis.nel = nnp) or the axis's element count (IGAAxis.nel); the tables always hold nnp
+      if ((a.nel != a.nnp && a.nel != (int)span_off.size()) || a.nqp != 1)
+        return fail(L, PETIGA_CUDA_ERR_ARG, "collocation: nel must be nnp (table length) or the number of knot spans, and nqp 1");
+      a.nel = a.nnp;
+      for (int i = 0; i < a.nnp; i++)
+        if (off[i] < 0 || off[i] + a.p >= a.nnp) return fail(L, PETIGA_CUDA_ERR_ARG, "collocation: offset table out of range");
+    }
+    const int* eoff = L.collocation ? span_off.data() : off;
+    const int nelp = L.collocation ? (int)span_off.size() : a.nel;
     a.first.resize(a.nnp); a.last.resize(a.nnp); a.own.assign(a.nnp, -1);
-    for (int i = 0; i < a.nnp; i++) stencil(a, U, i, a.first[i], a.last[i]);
+    for (int i = 0; i < a.nnp; i++) stencil(a, U, off, L.collocation, i, a.first[i], a.last[i]);
     a.box_es.resize(a.P); a.box_ew.resize(a.P); a.box_ls.resize(a.P); a.box_lw.resize(a.P); a.box_gs.resize(a.P); a.box_gw.resize(a.P);
-    if (a.nel < a.P) return fail(L, PETIGA_CUDA_ERR_ARG, "partition too fine");
+    if (nelp < a.P) return fail(L, PETIGA_CUDA_ERR_ARG, "partition too fine");
     for (int r = 0; r < a.P; r++) {  // IGA_Dist1D (petigapart.c:170-176) + node boxes (petiga.c:1160-1209)
-      int N = a.nel, ew = N / a.P + ((N % a.P) > r), es = r * (N / a.P) + (((N % a.P) > r) ? r : (N % a.P));
+      int N = nelp, ew = N / a.P + ((N % a.P) > r), es = r * (N / a.P) + (((N % a.P) > r) ? r : (N % a.P));
       int efirst = es, elast = es + ew - 1;
-      int gs = off[efirst], ge = off[elast] + a.p + 1, ls = gs;
-      int le = (elast < N - 1) ? off[elast + 1] : off[elast] + a.p + 1;
+      int gs = eoff[efirst], ge = eoff[elast] + a.p + 1, ls = gs;
+      int le = (elast < N - 1) ? eoff[elast + 1] : eoff[elast] + a.p + 1;
       int lw = le - ls;
       if (r == a.P - 1) lw = a.nnp - ls;
+      if (L.collocation) {   // element box = owned node box; ghost box = the stencils of the owned rows
+        es = ls; ew = lw;
+        if (lw < 1) return fail(L, PETIGA_CUDA_ERR_SUP, "a rank owns no nodes along an axis");
+        gs = a.first[ls]; ge = a.last[ls + lw - 1] + 1;
+      }
       a.box_es[r] = es; a.box_ew[r] = ew; a.box_ls[r] = ls; a.box_lw[r] = lw; a.box_gs[r] = gs; a.box_gw[r] = ge - gs;
       for (int i = ls; i < ls + lw; i++)
         if (i >= 0 && i < a.nnp) a.own[i] = r;
@@ -150,11 +180,13 @@ int build_layout(const petiga_cuda_space& sp, int rank, int nranks, Layout& L) {
       }
   std::sort(ghosts.begin(), ghosts.end());
   ghosts.erase(std::unique(ghosts.begin(), ghosts.end()), ghosts.end());
+  if (L.collocation) ghosts.clear();   // every row is computed by the rank that owns its point
   L.nghostrows = (int)ghosts.size();
   L.nloc = L.nown + L.nghostrows;
   for (int g = 0; g < ng; g++) {
     int gid = L.lgmap[g];
     if (gid >= my_lo && gid < my_hi) L.localrow[g] = gid - my_lo;
+    else if (L.collocation) L.localrow[g] = -1;
     else L.localrow[g] = L.nown + (int)(std::lower_bound(ghosts.begin(), ghosts.end(), gid) - ghosts.begin());
   }
   // per-row node coordinates and widths, row bases
@@ -163,6 +195,7 @@ int build_layout(const petiga_cuda_space& sp, int rank, int nranks, Layout& L) {
     for (int j = 0; j < A1.gw; j++)
       for (int i = 0; i < A0.gw; i++, g++) {
         int r = L.localrow[g];
+        if (r < 0) continue;
         L.rowW[0][r] = A0.W[i]; L.rowW[1][r] = A1.W[j]; L.rowW[2][r] = A2.W[k];
         L.rowG[0][r] = A0.wrapped[i]; L.rowG[1][r] = A1.wrapped[j]; L.rowG[2][r] = A2.wrapped[k];
       }
@@ -186,7 +219,7 @@ int build_layout(const petiga_cuda_space& sp, int rank, int nranks, Layout& L) {
     t = t1;
   }
   // rows other ranks hold for me, in *their* order (ascending global id == ascending local index here)
-  for (int s = 0; s < nranks; s++) {
+  for (int s = 0; s < nranks && !L.collocation; s++) {
     if (s == rank) continue;
     int c[3] = {s % A0.P, (s / A0.P) % A1.P, s / (A0.P * A1.P)};
     std::vector<int> mine[3];

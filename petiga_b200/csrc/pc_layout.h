@@ -5,7 +5,8 @@
 // Reference semantics reproduced here (bit-exact integer work):
 //   * box partition            src/petigapart.c:170-202 (IGA_Distribute), src/petiga.c:1160-1209
 //   * global numbering / lgmap src/petigagrid.c:98-171,185-228
-//   * row stencil              src/petigamat.c:197-267 (Stencil, ColumnIndices)
+//   * row stencil              src/petigamat.c:197-267 (Stencil, ColumnIndices), both branches
+//   * collocation boxes        the element box is the owned node box, the ghost box the union of the owned rows' stencils
 // What is new: instead of searching a sorted row per inserted value (MatSetValues), the position of
 // column B inside row A is computed in closed form from three per-axis tables (see col_position()).
 #pragma once
@@ -43,13 +44,14 @@ struct AxisLayout {
 
 struct Layout {
   int dim = 1, dof = 1, rank = 0, nranks = 1;
+  int collocation = 0;                    // rows are the owned nodes only: no ghost rows, nothing to exchange
   AxisLayout ax[3];
   int nown = 0;                           // owned nodes
   int nghostrows = 0;                     // distinct nodes in the ghost box owned by other ranks
   int nloc = 0;                           // nown + nghostrows = rows of the unified local buffer
   int64_t nnz_own = 0, nnz_loc = 0;       // blocks in owned rows / in owned+ghost rows
   std::vector<int> rank_start;            // [nranks+1] first global node of every rank
-  std::vector<int> localrow;              // [gw0*gw1*gw2] ghost-box node -> local row id
+  std::vector<int> localrow;              // [gw0*gw1*gw2] ghost-box node -> local row id (collocation: -1 for nodes of other ranks)
   std::vector<int> lgmap;                 // [gw0*gw1*gw2] ghost-box node -> global node
   std::vector<int64_t> rowbase;           // [nloc+1] block offset of every local row (owned rows first)
   std::vector<int> rowW[3];               // [nloc] per-axis widths of every local row

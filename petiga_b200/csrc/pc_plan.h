@@ -125,6 +125,8 @@ void nvtx_push(const char* name);
 // IGAFormBC of every face as the element fix-up reads it: the values and, with loads, the Neumann loads of fields < dof
 // (pc_api.cu).  out must be zeroed; it stays so when no boundary condition is set.  Each caller derives its own any_bc.
 void fill_fix_sides(const petiga_cuda_plan* P, bool loads, FixSide out[3][2]);
+// collocation rows (pc_colloc.cu): every value of the owned rows and the owned right-hand side, written once
+int launch_collocation(petiga_cuda_plan* P, int slot, int form, double* values, double* rhs);
 // boundary-integral pass (pc_bnd.cu)
 int launch_boundary_pass(petiga_cuda_plan* P, int slot, int form, const double* prm, double* rhs, bool apply_fix);
 }  // namespace pc

@@ -310,6 +310,7 @@ extern "C" int petiga_cuda_compute_scalar(petiga_cuda_plan* P, int scalar_id, co
                                           double* S_host) {
   if (!P || !S_host || n < 1 || n > kMaxS || nparams < 0 || nparams > 8 || (nparams && !params)) { set_error("compute_scalar: bad argument"); return PETIGA_CUDA_ERR_ARG; }
   const Layout& L = P->L;
+  if (L.collocation) { set_error("compute_scalar: a collocation plan has no quadrature rule; integrate on the Galerkin plan of the same axes (same numbering)"); return PETIGA_CUDA_ERR_SUP; }
   ScalarParams sp;
   memset(&sp, 0, sizeof(sp));
   for (int k = 0; k < nparams; k++) sp.prm[k] = params[k];

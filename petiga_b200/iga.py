@@ -20,6 +20,9 @@ FORMS = {
     "BOUNDARYINTEGRAL": {"SYSTEM": "IGADeviceForm_BoundaryIntegral_System"},
     "NEUMANN": {"SYSTEM": "IGADeviceForm_Neumann_SystemGalerkin"},
     "CONVTEST": {"SYSTEM": "IGADeviceForm_ConvTest_Galerkin"},
+    # collocation forms (SetUseCollocation(True)): the strong form at the Greville points
+    "LAPLACE_COLLOCATION": {"SYSTEM": "IGADeviceForm_Laplace_SystemCollocation"},
+    "CONVTEST_COLLOCATION": {"SYSTEM": "IGADeviceForm_ConvTest_Collocation"},
     "MASS": {"SYSTEM": "IGADeviceForm_Mass_System", "MATRIX": "IGADeviceForm_Mass_Matrix", "VECTOR": "IGADeviceForm_Mass_Vector"},
     "ELASTICITY3D": {"SYSTEM": "IGADeviceForm_Elasticity3D_System"},
     "ELASTICITY": {"SYSTEM": "IGADeviceForm_Elasticity_System"},
@@ -213,6 +216,15 @@ class IGA:
 
     def SetMatType(self, t):
         _chk(self.H.IGASetMatType(self.h, t.encode()))
+
+    def SetUseCollocation(self, flag=True):
+        """IGASetUseCollocation: assemble by collocation at the Greville points instead of Galerkin (before SetUp)."""
+        _chk(self.H.IGASetUseCollocation(self.h, int(bool(flag))))
+
+    def GetUseCollocation(self):
+        f = C.c_int()
+        _chk(self.H.IGAGetUseCollocation(self.h, C.byref(f)))
+        return bool(f.value)
 
     def _axis(self, i):
         ax = C.c_void_p()
