@@ -84,12 +84,17 @@ enum {
   PETIGA_FORM_ELASTICROD = 14,    /* demo/ElasticRodFJ.F90 I2Function/I2Jacobian; params = {rho, E}                        */
   PETIGA_FORM_NITSCHE = 15,       /* demo/NitscheMethod.c:70-119 System: Poisson inside, Nitsche matrix + vector terms on the
                                      faces enabled with petiga_cuda_set_boundary_form                                       */
-  /* isogeometric collocation (petiga_cuda_space.collocation = 1): the strong form at the Greville points; slots VECTOR, MATRIX,
-     SYSTEM, dof 1.  A Galerkin form on a collocation plan, or one of these on a Galerkin plan, is PETIGA_CUDA_ERR_SUP */
+  /* isogeometric collocation (petiga_cuda_space.collocation = 1): the strong form at the Greville points, dof 1; the linear forms
+     in the slots VECTOR, MATRIX, SYSTEM, the Bratu form in FUNCTION, JACOBIAN, IFUNCTION, IJACOBIAN.  A Galerkin form on a
+     collocation plan, or one of these on a Galerkin plan, is PETIGA_CUDA_ERR_SUP */
   PETIGA_FORM_LAPLACE_COLLOCATION = 16,   /* demo/Laplace.c SystemCollocation: K[a] = -Lap N_a, F = 0                                 */
   PETIGA_FORM_CONVTEST_COLLOCATION = 17,  /* strong form of test/ConvTest.c: K[a] = c N_a - k Lap N_a,
                                              F = (c + k dim pi^2) prod sin(pi x_i); params = {c, k}                                 */
-  PETIGA_NFORMS = 18              /* PETIGA_FORM_BRATU also provides RHSFunction/RHSJacobian (its explicit form)            */
+  PETIGA_FORM_BRATU_COLLOCATION = 18,     /* strong form of PETIGA_FORM_BRATU at x_a, u = sum_b R_b U_b, v = sum_b R_b V_b; params = {lambda}:
+                                             Function F_a = -Lap u - lambda e^u,  Jacobian J_ab = -Lap R_b - lambda e^u R_b,
+                                             IFunction F_a = v - Lap u - lambda e^u,  IJacobian J_ab = shift R_b - Lap R_b - lambda e^u R_b;
+                                             a node with a boundary value has F_a = U_a - value and an identity row              */
+  PETIGA_NFORMS = 19              /* PETIGA_FORM_BRATU also provides RHSFunction/RHSJacobian (its explicit form)            */
 };
 
 /* built-in Scalar callbacks of petiga_cuda_compute_scalar (IGAComputeScalar, src/petigacomp.c:35-96) */
@@ -284,7 +289,9 @@ int petiga_cuda_comm_destroy(void *nccl_comm);
 
 /* exchange plan introspection (host logic; usable without a GPU run): for this rank, the neighbours and
    the ghost-row / halo lists.  kind = 0: ghost rows sent to owners (matrix/vector assembly),
-   kind = 1: rows received from lower neighbours.  Returns the count; when out != NULL fills
+   kind = 1: rows received from lower neighbours; collocation plans (no ghost rows, kinds 0 and 1 empty) have the state halo
+   instead: kind = 2: the run of foreign ghost-box nodes each owner sends (first state row, count), kind = 3: the owned rows each
+   neighbour reads (first row, count).  Returns the count; when out != NULL fills
    out[3*i+0] = peer rank, out[3*i+1] = first row (local id), out[3*i+2] = number of rows. */
 int petiga_cuda_plan_exchange_info(petiga_cuda_plan *plan, int kind, int *count, int *out, int capacity);
 
@@ -301,10 +308,14 @@ int petiga_layout_rowbase(const petiga_layout *layout, int64_t *rowbase);  /* [n
 int petiga_layout_pattern(const petiga_layout *layout, int block, int *rowptr, int *colidx);
 /* closed-form position of column node (unwrapped ghost coordinates hb) in the row of ghost node ga */
 int petiga_layout_position(const petiga_layout *layout, const int ga[3], const int hb[3], int64_t *pos);
-/* kind 0: ghost rows I send (peer, first local row, nrows, nblocks); kind 1: rows I receive.
-   out[4*i..]; for kind 1 the row list of peer i is returned by petiga_layout_recv_rows. */
+/* kind 0: ghost rows I send (peer, first local row, nrows, nblocks); kind 1: rows I receive; kinds 2 and 3: the collocation state
+   halo as in petiga_cuda_plan_exchange_info (nblocks 0).  out[4*i..]; the row list of peer i of kind 1 (Galerkin layouts) or
+   kind 3 (collocation layouts) is returned by petiga_layout_recv_rows. */
 int petiga_layout_exchange(const petiga_layout *layout, int kind, int *count, int64_t *out, int capacity);
 int petiga_layout_recv_rows(const petiga_layout *layout, int peer_index, int *rows, int capacity);
+/* collocation layouts only (PETIGA_CUDA_ERR_ARG otherwise): the state numbering of the ghost box, [nghostbox]: an owned node maps
+   to its row, a node of another rank to nown + t (t in ascending global id); *nstate = nown + the number of such nodes */
+int petiga_layout_staterow(const petiga_layout *layout, int *nstate, int *staterow);
 
 #ifdef __cplusplus
 }

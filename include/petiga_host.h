@@ -96,6 +96,12 @@ PetscErrorCode IGADeviceForm_ConvTest_Galerkin(IGAPoint, PetscScalar *, PetscSca
 /* collocation forms (IGASetUseCollocation): the strong form at each Greville point, K[a] and F of one row per node */
 PetscErrorCode IGADeviceForm_Laplace_SystemCollocation(IGAPoint, PetscScalar *, PetscScalar *, void *);  /* demo/Laplace.c SystemCollocation: -Lap N_a */
 PetscErrorCode IGADeviceForm_ConvTest_Collocation(IGAPoint, PetscScalar *, PetscScalar *, void *);      /* c N_a - k Lap N_a, F = (c + k dim pi^2) prod sin(pi x_i); ctx: {c, k} */
+/* Bratu by collocation (the strong form of IGADeviceForm_Bratu_*), ctx: {lambda}: F_a = [v] - Lap u - lambda e^u at x_a, the Jacobian row
+   [shift R_b] - Lap R_b - lambda e^u R_b; a node with a boundary value has F_a = U_a - value and an identity row */
+PetscErrorCode IGADeviceForm_Bratu_FunctionCollocation(IGAPoint, const PetscScalar *, PetscScalar *, void *);
+PetscErrorCode IGADeviceForm_Bratu_JacobianCollocation(IGAPoint, const PetscScalar *, PetscScalar *, void *);
+PetscErrorCode IGADeviceForm_Bratu_IFunctionCollocation(IGAPoint, PetscReal, const PetscScalar *, PetscReal, const PetscScalar *, PetscScalar *, void *);
+PetscErrorCode IGADeviceForm_Bratu_IJacobianCollocation(IGAPoint, PetscReal, const PetscScalar *, PetscReal, const PetscScalar *, PetscScalar *, void *);
 PetscErrorCode IGADeviceForm_Elasticity3D_System(IGAPoint, PetscScalar *, PetscScalar *, void *);       /* ctx: {lambda, mu}                   */
 PetscErrorCode IGADeviceForm_Elasticity_System(IGAPoint, PetscScalar *, PetscScalar *, void *);         /* ctx: {mu, lambda} as demo/Elasticity.c:10-13 */
 PetscErrorCode IGADeviceForm_CahnHilliard2D_Residual(IGAPoint, PetscReal, const PetscScalar *, PetscReal, const PetscScalar *, PetscScalar *, void *); /* ctx: {theta, alpha} */

@@ -291,6 +291,10 @@ const FormEntry* lookup_form(const void* fn, int slot) {
       {FN(IGADeviceForm_ConvTest_Galerkin), PETIGA_SLOT_SYSTEM, PETIGA_FORM_CONVTEST, 2, 0},
       {FN(IGADeviceForm_Laplace_SystemCollocation), PETIGA_SLOT_SYSTEM, PETIGA_FORM_LAPLACE_COLLOCATION, 0, 0},
       {FN(IGADeviceForm_ConvTest_Collocation), PETIGA_SLOT_SYSTEM, PETIGA_FORM_CONVTEST_COLLOCATION, 2, 0},
+      {FN(IGADeviceForm_Bratu_FunctionCollocation), PETIGA_SLOT_FUNCTION, PETIGA_FORM_BRATU_COLLOCATION, 1, 0},
+      {FN(IGADeviceForm_Bratu_JacobianCollocation), PETIGA_SLOT_JACOBIAN, PETIGA_FORM_BRATU_COLLOCATION, 1, 0},
+      {FN(IGADeviceForm_Bratu_IFunctionCollocation), PETIGA_SLOT_IFUNCTION, PETIGA_FORM_BRATU_COLLOCATION, 1, 0},
+      {FN(IGADeviceForm_Bratu_IJacobianCollocation), PETIGA_SLOT_IJACOBIAN, PETIGA_FORM_BRATU_COLLOCATION, 1, 0},
       {FN(IGADeviceForm_Mass_Matrix), PETIGA_SLOT_MATRIX, PETIGA_FORM_MASS, 0, 0},
       {FN(IGADeviceForm_Mass_Vector), PETIGA_SLOT_VECTOR, PETIGA_FORM_MASS, 0, 0},
       {FN(IGADeviceForm_Elasticity3D_System), PETIGA_SLOT_SYSTEM, PETIGA_FORM_ELASTICITY3D, 2, 0},
@@ -353,6 +357,8 @@ SENT4(IGADeviceForm_Laplace_System) SENT4(IGADeviceForm_L2Projection_System) SEN
 SENT3(IGADeviceForm_Mass_Matrix) SENT3(IGADeviceForm_Mass_Vector)
 SENT4(IGADeviceForm_BoundaryIntegral_System) SENT4(IGADeviceForm_Neumann_SystemGalerkin) SENT4(IGADeviceForm_ConvTest_Galerkin)
 SENT4(IGADeviceForm_Laplace_SystemCollocation) SENT4(IGADeviceForm_ConvTest_Collocation)
+SENTF(IGADeviceForm_Bratu_FunctionCollocation) SENTF(IGADeviceForm_Bratu_JacobianCollocation)
+SENTI(IGADeviceForm_Bratu_IFunctionCollocation) SENTI(IGADeviceForm_Bratu_IJacobianCollocation)
 PetscErrorCode IGADeviceExact_ConvTest(IGAPoint, PetscInt, PetscScalar*, void*) { return host_sentinel(); }
 PetscErrorCode IGADeviceExact_Neumann(IGAPoint, PetscInt, PetscScalar*, void*) { return host_sentinel(); }
 SENT4(IGADeviceForm_Elasticity3D_System) SENT4(IGADeviceForm_Elasticity_System)
@@ -861,13 +867,14 @@ PetscErrorCode VecGetArrayDevice(Vec v, PetscScalar** d) { if (!v || !d) return 
 // what the collocation kernel supports, checked before any device work (the library repeats the checks for direct callers)
 static PetscErrorCode check_collocation(IGA g, int slot) {
   const int f = g->slots[slot].form;
-  const bool cform = f == PETIGA_FORM_LAPLACE_COLLOCATION || f == PETIGA_FORM_CONVTEST_COLLOCATION;
+  const bool cform = f == PETIGA_FORM_LAPLACE_COLLOCATION || f == PETIGA_FORM_CONVTEST_COLLOCATION || f == PETIGA_FORM_BRATU_COLLOCATION;
   if (!g->collocation) {
     if (cform) return fail(PETSC_ERR_SUP, "a collocation form needs IGASetUseCollocation(iga, PETSC_TRUE)");
     return 0;
   }
-  if (slot != PETIGA_SLOT_VECTOR && slot != PETIGA_SLOT_MATRIX && slot != PETIGA_SLOT_SYSTEM)
-    return fail(PETSC_ERR_SUP, "collocation: only IGAComputeVector/Matrix/System run on the device");
+  if (slot != PETIGA_SLOT_VECTOR && slot != PETIGA_SLOT_MATRIX && slot != PETIGA_SLOT_SYSTEM && slot != PETIGA_SLOT_FUNCTION &&
+      slot != PETIGA_SLOT_JACOBIAN && slot != PETIGA_SLOT_IFUNCTION && slot != PETIGA_SLOT_IJACOBIAN)
+    return fail(PETSC_ERR_SUP, "collocation: only IGAComputeVector/Matrix/System/Function/Jacobian/IFunction/IJacobian run on the device");
   if (!cform) return fail(PETSC_ERR_SUP, "collocation: pass one of the IGADeviceForm_*Collocation sentinels (Galerkin forms integrate)");
   if (g->dof != 1) return fail(PETSC_ERR_SUP, "collocation: the device forms have dof 1");
   for (int d = 0; d < g->dim; d++)

@@ -332,16 +332,17 @@ int petiga_cuda_plan_create(petiga_cuda_plan** plan, const petiga_cuda_space* sp
   if ((rc = upload(P, L.localrow.data(), L.localrow.size(), &P->d_localrow))) return bail(rc);
   if ((rc = upload(P, L.rowbase.data(), L.rowbase.size(), &P->d_rowbase))) return bail(rc);
   if ((rc = upload(P, L.rank_start.data(), L.rank_start.size(), &P->d_rank_start))) return bail(rc);
+  if (L.collocation && (rc = upload(P, L.staterow.data(), L.staterow.size(), &P->d_staterow))) return bail(rc);
   if (L.nranks > 1) {
-    const size_t nl = (size_t)L.nloc * L.dof;
+    const size_t nl = (size_t)L.nloc * L.dof, ns = (size_t)(L.collocation ? L.nstate : L.nloc) * L.dof;
     if ((rc = upload<double>(P, nullptr, nl, &P->d_rhs_loc))) return bail(rc);
-    if ((rc = upload<double>(P, nullptr, nl, &P->d_U_loc))) return bail(rc);
-    if ((rc = upload<double>(P, nullptr, nl, &P->d_V_loc))) return bail(rc);
+    if ((rc = upload<double>(P, nullptr, ns, &P->d_U_loc))) return bail(rc);
+    if ((rc = upload<double>(P, nullptr, ns, &P->d_V_loc))) return bail(rc);
     if ((rc = upload<double>(P, nullptr, nl, &P->d_W_loc))) return bail(rc);
     std::vector<int> rows;
     std::vector<int64_t> offs;      // prefix sum of the row lengths inside each peer's slab (the sender packs rows back to back)
     P->recv_row_off.clear();
-    for (auto& r : L.recv) {
+    for (auto& r : L.collocation ? L.state_recv : L.recv) {   // collocation: what the state halo packs (no ghost rows)
       P->recv_row_off.push_back(rows.size());
       rows.insert(rows.end(), r.rows.begin(), r.rows.end());
       int64_t o = 0;
@@ -481,7 +482,7 @@ int petiga_cuda_set_fixtable_device(petiga_cuda_plan* P, const double* table_own
   double* tmp = nullptr;
   if (L.nranks > 1) {                     // ghost nodes carry their owner's table value (VecScatter g2l)
     PC_CUDA(cudaMalloc(&tmp, (size_t)L.nloc * L.dof * sizeof(double)));
-    int rc = halo_state(P, table_own, tmp);
+    int rc = halo_state(P, L.send, L.recv, table_own, tmp);
     if (rc) { cudaFree(tmp); return rc; }
     loc = tmp;
   }
@@ -615,10 +616,24 @@ int petiga_cuda_compute_ext(petiga_cuda_plan* P, int slot, int block, double shi
     if (P->d_fixtable) { set_error("compute: IGASetFixTable is not supported with collocation"); return PETIGA_CUDA_ERR_SUP; }
     PC_CUDA(cudaSetDevice(P->device));
     nvtx_push(slot);
+    struct Pop { ~Pop() { nvtx_pop(); } } pop_on_exit;
     cudaEventRecord(P->ev0, P->stream);
-    const int rc = launch_collocation(P, slot, form, values, rhs);
+    int rc;
+    if (state) {   // Bratu collocation: U (and V) on the collocation ghost box, then the state kernel
+      const double *U_k = U, *V_k = V;
+      if (L.nranks > 1) {
+        if ((rc = halo_state(P, L.state_send, L.state_recv, U, P->d_U_loc))) return rc;
+        U_k = P->d_U_loc;
+        if (slot == PETIGA_SLOT_IFUNCTION) {
+          if ((rc = halo_state(P, L.state_send, L.state_recv, V, P->d_V_loc))) return rc;
+          V_k = P->d_V_loc;
+        }
+      }
+      rc = launch_collocation_state(P, slot, U_k, V_k, shift, values, rhs);
+    } else {
+      rc = launch_collocation(P, slot, form, values, rhs);
+    }
     cudaEventRecord(P->ev1, P->stream);
-    nvtx_pop();
     if (rc) return rc;
     P->last_path = PETIGA_PATH_COLLOCATION;
     P->last_impl = -1;
@@ -668,11 +683,11 @@ int petiga_cuda_compute_ext(petiga_cuda_plan* P, int slot, int block, double shi
   // IGAGetLocalVecArray: G2L halo of the state vectors (petigavec.c:256-269)
   const double *U_k = U, *V_k = V, *W_k = W;
   if (multi && state) {
-    int rc = halo_state(P, U, P->d_U_loc);
+    int rc = halo_state(P, L.send, L.recv, U, P->d_U_loc);
     if (rc) return rc;
     U_k = P->d_U_loc;
-    if (has_v) { rc = halo_state(P, V, P->d_V_loc); if (rc) return rc; V_k = P->d_V_loc; }
-    if (has_w) { rc = halo_state(P, W, P->d_W_loc); if (rc) return rc; W_k = P->d_W_loc; }
+    if (has_v) { rc = halo_state(P, L.send, L.recv, V, P->d_V_loc); if (rc) return rc; V_k = P->d_V_loc; }
+    if (has_w) { rc = halo_state(P, L.send, L.recv, W, P->d_W_loc); if (rc) return rc; W_k = P->d_W_loc; }
   }
 
   KParams kp;
@@ -937,12 +952,15 @@ int petiga_cuda_host_free(void* ptr) { PC_CUDA(cudaFreeHost(ptr)); return 0; }
 int petiga_cuda_plan_exchange_info(petiga_cuda_plan* P, int kind, int* count, int* out, int capacity) {
   if (!P || !count) return PETIGA_CUDA_ERR_ARG;
   const Layout& L = P->L;
-  if (kind == 0) {
-    *count = (int)L.send.size();
-    if (out) for (int i = 0; i < *count && i < capacity; i++) { out[3 * i] = L.send[i].rank; out[3 * i + 1] = L.send[i].first_row; out[3 * i + 2] = L.send[i].nrows; }
+  if (kind < 0 || kind > 3) return PETIGA_CUDA_ERR_ARG;
+  if (kind == 0 || kind == 2) {
+    const auto& S = kind == 0 ? L.send : L.state_send;
+    *count = (int)S.size();
+    if (out) for (int i = 0; i < *count && i < capacity; i++) { out[3 * i] = S[i].rank; out[3 * i + 1] = S[i].first_row; out[3 * i + 2] = S[i].nrows; }
   } else {
-    *count = (int)L.recv.size();
-    if (out) for (int i = 0; i < *count && i < capacity; i++) { out[3 * i] = L.recv[i].rank; out[3 * i + 1] = L.recv[i].rows.empty() ? -1 : L.recv[i].rows[0]; out[3 * i + 2] = (int)L.recv[i].rows.size(); }
+    const auto& R = kind == 1 ? L.recv : L.state_recv;
+    *count = (int)R.size();
+    if (out) for (int i = 0; i < *count && i < capacity; i++) { out[3 * i] = R[i].rank; out[3 * i + 1] = R[i].rows.empty() ? -1 : R[i].rows[0]; out[3 * i + 2] = (int)R[i].rows.size(); }
   }
   return 0;
 }

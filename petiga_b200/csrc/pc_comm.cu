@@ -3,7 +3,8 @@
 //        (src/petigaksp.c:197-200): every rank ships the rows it integrated but does not own to their
 //        owner, who adds them.  Here the ghost rows are laid out exactly like the owner's CSR rows, so a
 //        message is one contiguous slab per owner and the receive side is a streaming add.
-//   (ii) state halo:     VecScatter g2l of IGAGetLocalVecArray (src/petigavec.c:147-169,256-269).
+//   (ii) state halo:     VecScatter g2l of IGAGetLocalVecArray (src/petigavec.c:147-169,256-269), on the Galerkin ghost rows or
+//        on the collocation ghost box (the list pair the caller passes).
 // NCCL is loaded with dlopen so that the library also loads on hosts without it (single-rank use).
 #include <dlfcn.h>
 #include <nccl.h>
@@ -165,7 +166,8 @@ int exchange_ghost_rows(petiga_cuda_plan* P, int block, double* values, double* 
   return 0;
 }
 
-int halo_state(petiga_cuda_plan* P, const double* U_own, double* U_loc) {
+int halo_state(petiga_cuda_plan* P, const std::vector<Layout::Peer>& ghost, const std::vector<Layout::Recv>& owned, const double* U_own,
+               double* U_loc) {
   const Layout& L = P->L;
   if (!P->nccl) { set_error("multi-rank plan without an NCCL communicator"); return PETIGA_CUDA_ERR_ORDER; }
   int rc = nccl_load();
@@ -174,21 +176,21 @@ int halo_state(petiga_cuda_plan* P, const double* U_own, double* U_loc) {
   const int dof = L.dof;
   PC_CUDA(cudaMemcpyAsync(U_loc, U_own, (size_t)L.nown * dof * sizeof(double), cudaMemcpyDeviceToDevice, P->stream));
   size_t total = 0;
-  std::vector<size_t> off(L.recv.size());
-  for (size_t i = 0; i < L.recv.size(); i++) { off[i] = total; total += L.recv[i].rows.size() * dof; }
+  std::vector<size_t> off(owned.size());
+  for (size_t i = 0; i < owned.size(); i++) { off[i] = total; total += owned[i].rows.size() * dof; }
   if ((rc = ensure_recv(P, total))) return rc;
-  for (size_t i = 0; i < L.recv.size(); i++) {   // owners pack the rows their neighbours see as ghosts
-    const int n = (int)L.recv[i].rows.size();
+  for (size_t i = 0; i < owned.size(); i++) {   // owners pack the rows their neighbours see as ghosts
+    const int n = (int)owned[i].rows.size();
     gather_vec_rows_kernel<<<(n * dof + 255) / 256, 256, 0, P->stream>>>(P->d_recv_rows + P->recv_row_off[i], n, dof, U_own, P->d_recv + off[i]);
     PC_CUDA(cudaGetLastError());
     P->launches++;
   }
   ncclResult_t gr = g_nccl.GroupStart();
   if (gr != ncclSuccess) return nccl_fail(gr, "ncclGroupStart");
-  for (size_t i = 0; i < L.recv.size() && gr == ncclSuccess; i++)
-    gr = g_nccl.Send(P->d_recv + off[i], L.recv[i].rows.size() * dof, ncclDouble, L.recv[i].rank, comm, P->stream);
-  for (size_t i = 0; i < L.send.size() && gr == ncclSuccess; i++)
-    gr = g_nccl.Recv(U_loc + (size_t)L.send[i].first_row * dof, (size_t)L.send[i].nrows * dof, ncclDouble, L.send[i].rank, comm, P->stream);
+  for (size_t i = 0; i < owned.size() && gr == ncclSuccess; i++)
+    gr = g_nccl.Send(P->d_recv + off[i], owned[i].rows.size() * dof, ncclDouble, owned[i].rank, comm, P->stream);
+  for (size_t i = 0; i < ghost.size() && gr == ncclSuccess; i++)
+    gr = g_nccl.Recv(U_loc + (size_t)ghost[i].first_row * dof, (size_t)ghost[i].nrows * dof, ncclDouble, ghost[i].rank, comm, P->stream);
   ncclResult_t ge = g_nccl.GroupEnd();
   if (gr != ncclSuccess) return nccl_fail(gr, "ncclSend/ncclRecv (state halo)");
   if (ge != ncclSuccess) return nccl_fail(ge, "ncclGroupEnd");

@@ -140,6 +140,10 @@ __host__ __device__ inline FormInfo form_info(int form, int slot, int dim, int d
       if (dof != 1 || !lin) break;
       f.valid = 1; f.colloc = 1; f.order = 2; f.needs_x = 1;
       break;
+    case PETIGA_FORM_BRATU_COLLOCATION:      // strong form of PETIGA_FORM_BRATU (pc_colloc.cu colloc_state_kernel)
+      if (dof != 1 || !(fun || jac)) break;
+      f.valid = 1; f.colloc = 1; f.per_qp = 1; f.needs_state = 1; f.order = 2;
+      break;
     case PETIGA_FORM_NITSCHE:           // demo/NitscheMethod.c:70-119: interior Poisson (f = -2 dim) + face terms
       if (dof != 1 || slot != PETIGA_SLOT_SYSTEM) break;
       f.valid = 1; f.mc0 = 0; f.mc1 = 1 + dim; f.vc0 = 0; f.vc1 = 1 + dim; f.per_qp = 1; f.needs_x = 1; f.order = 1; f.bnd_mat = 1; f.bnd_vec = 1;

@@ -180,7 +180,8 @@ int build_layout(const petiga_cuda_space& sp, int rank, int nranks, Layout& L) {
       }
   std::sort(ghosts.begin(), ghosts.end());
   ghosts.erase(std::unique(ghosts.begin(), ghosts.end()), ghosts.end());
-  if (L.collocation) ghosts.clear();   // every row is computed by the rank that owns its point
+  std::vector<int> foreign;   // collocation: every row is computed by the rank that owns its point, so the nodes of other
+  if (L.collocation) foreign.swap(ghosts);   // ranks are state only (the halo), never rows
   L.nghostrows = (int)ghosts.size();
   L.nloc = L.nown + L.nghostrows;
   for (int g = 0; g < ng; g++) {
@@ -188,6 +189,15 @@ int build_layout(const petiga_cuda_space& sp, int rank, int nranks, Layout& L) {
     if (gid >= my_lo && gid < my_hi) L.localrow[g] = gid - my_lo;
     else if (L.collocation) L.localrow[g] = -1;
     else L.localrow[g] = L.nown + (int)(std::lower_bound(ghosts.begin(), ghosts.end(), gid) - ghosts.begin());
+  }
+  if (L.collocation) {
+    L.nstate = L.nown + (int)foreign.size();
+    L.staterow.resize(ng);
+    for (int g = 0; g < ng; g++) {
+      const int gid = L.lgmap[g];
+      L.staterow[g] = (gid >= my_lo && gid < my_hi) ? gid - my_lo
+                                                    : L.nown + (int)(std::lower_bound(foreign.begin(), foreign.end(), gid) - foreign.begin());
+    }
   }
   // per-row node coordinates and widths, row bases
   for (int d = 0; d < 3; d++) { L.rowW[d].assign(L.nloc, 0); L.rowG[d].assign(L.nloc, 0); }
@@ -207,19 +217,25 @@ int build_layout(const petiga_cuda_space& sp, int rank, int nranks, Layout& L) {
   }
   L.nnz_own = L.rowbase[L.nown];
   L.nnz_loc = L.rowbase[L.nloc];
-  // ghost rows -> owners (contiguous runs because ghost rows are sorted by global id)
-  for (int t = 0; t < L.nghostrows;) {
-    int q = (int)(std::upper_bound(L.rank_start.begin(), L.rank_start.end(), ghosts[t]) - L.rank_start.begin()) - 1;
-    int t1 = t;
-    while (t1 < L.nghostrows && ghosts[t1] < L.rank_start[q + 1]) t1++;
-    Layout::Peer pr;
-    pr.rank = q; pr.first_row = L.nown + t; pr.nrows = t1 - t;
-    pr.first_block = L.rowbase[L.nown + t]; pr.nblocks = L.rowbase[L.nown + t1] - pr.first_block;
-    L.send.push_back(pr);
-    t = t1;
-  }
-  // rows other ranks hold for me, in *their* order (ascending global id == ascending local index here)
-  for (int s = 0; s < nranks && !L.collocation; s++) {
+  // ghost rows (collocation: foreign state nodes) -> owners (contiguous runs because both lists are sorted by global id)
+  auto owner_runs = [&](const std::vector<int>& ids, bool rows, std::vector<Layout::Peer>& out) {
+    const int n = (int)ids.size();
+    for (int t = 0; t < n;) {
+      int q = (int)(std::upper_bound(L.rank_start.begin(), L.rank_start.end(), ids[t]) - L.rank_start.begin()) - 1;
+      int t1 = t;
+      while (t1 < n && ids[t1] < L.rank_start[q + 1]) t1++;
+      Layout::Peer pr;
+      pr.rank = q; pr.first_row = L.nown + t; pr.nrows = t1 - t;
+      pr.first_block = rows ? L.rowbase[L.nown + t] : 0; pr.nblocks = rows ? L.rowbase[L.nown + t1] - pr.first_block : 0;
+      out.push_back(pr);
+      t = t1;
+    }
+  };
+  owner_runs(ghosts, true, L.send);
+  owner_runs(foreign, false, L.state_send);
+  // rows other ranks hold for me (collocation: read as state), in *their* order (ascending global id == ascending local index here)
+  std::vector<Layout::Recv>& held = L.collocation ? L.state_recv : L.recv;
+  for (int s = 0; s < nranks; s++) {
     if (s == rank) continue;
     int c[3] = {s % A0.P, (s / A0.P) % A1.P, s / (A0.P * A1.P)};
     std::vector<int> mine[3];
@@ -240,9 +256,9 @@ int build_layout(const petiga_cuda_space& sp, int rank, int nranks, Layout& L) {
     for (int w2 : mine[2]) for (int w1 : mine[1]) for (int w0 : mine[0]) {
       int row = (w0 - A0.ls) + A0.lw * ((w1 - A1.ls) + A1.lw * (w2 - A2.ls));
       rv.rows.push_back(row);
-      rv.nblocks += L.rowbase[row + 1] - L.rowbase[row];
+      if (!L.collocation) rv.nblocks += L.rowbase[row + 1] - L.rowbase[row];
     }
-    L.recv.push_back(std::move(rv));
+    held.push_back(std::move(rv));
   }
   return 0;
 }

@@ -6,7 +6,8 @@
 //   * box partition            src/petigapart.c:170-202 (IGA_Distribute), src/petiga.c:1160-1209
 //   * global numbering / lgmap src/petigagrid.c:98-171,185-228
 //   * row stencil              src/petigamat.c:197-267 (Stencil, ColumnIndices), both branches
-//   * collocation boxes        the element box is the owned node box, the ghost box the union of the owned rows' stencils
+//   * collocation boxes        the element box is the owned node box, the ghost box the union of the owned rows' stencils;
+//                              the state halo of that ghost box (staterow, state_send, state_recv)
 // What is new: instead of searching a sorted row per inserted value (MatSetValues), the position of
 // column B inside row A is computed in closed form from three per-axis tables (see col_position()).
 #pragma once
@@ -61,6 +62,12 @@ struct Layout {
   std::vector<Peer> send;                 // ghost rows I hold for `rank`  (contiguous local rows)
   struct Recv { int rank; std::vector<int> rows; int64_t nblocks; };
   std::vector<Recv> recv;                 // my owned rows that `rank` holds as ghost rows, in its order
+  // collocation state halo (empty on Galerkin layouts, whose halo uses send/recv): the kernels read U at every node of the
+  // ghost box, and the nodes of other ranks are numbered after the owned rows, ascending global id (one run per owner)
+  std::vector<int> staterow;              // [gw0*gw1*gw2] ghost-box node -> state row (owned: its row; foreign: nown + t)
+  int nstate = 0;                         // nown + foreign nodes of the ghost box
+  std::vector<Peer> state_send;           // the run of foreign nodes that `rank` owns (first_row, nrows; no blocks)
+  std::vector<Recv> state_recv;           // my owned rows inside `rank`'s ghost box, in its order (nblocks 0)
   std::string error;
 };
 

@@ -57,19 +57,31 @@ int petiga_layout_position(const petiga_layout* l, const int ga[3], const int hb
 int petiga_layout_exchange(const petiga_layout* l, int kind, int* count, int64_t* out, int capacity) {
   if (!l || !count) return PETIGA_CUDA_ERR_ARG;
   const pc::Layout& L = l->L;
-  if (kind == 0) {
-    *count = (int)L.send.size();
-    if (out) for (int i = 0; i < *count && i < capacity; i++) { out[4*i] = L.send[i].rank; out[4*i+1] = L.send[i].first_row; out[4*i+2] = L.send[i].nrows; out[4*i+3] = L.send[i].nblocks; }
+  if (kind < 0 || kind > 3) return PETIGA_CUDA_ERR_ARG;
+  if (kind == 0 || kind == 2) {
+    const auto& S = kind == 0 ? L.send : L.state_send;
+    *count = (int)S.size();
+    if (out) for (int i = 0; i < *count && i < capacity; i++) { out[4*i] = S[i].rank; out[4*i+1] = S[i].first_row; out[4*i+2] = S[i].nrows; out[4*i+3] = S[i].nblocks; }
   } else {
-    *count = (int)L.recv.size();
-    if (out) for (int i = 0; i < *count && i < capacity; i++) { out[4*i] = L.recv[i].rank; out[4*i+1] = L.recv[i].rows.empty() ? -1 : L.recv[i].rows[0]; out[4*i+2] = (int64_t)L.recv[i].rows.size(); out[4*i+3] = L.recv[i].nblocks; }
+    const auto& R = kind == 1 ? L.recv : L.state_recv;
+    *count = (int)R.size();
+    if (out) for (int i = 0; i < *count && i < capacity; i++) { out[4*i] = R[i].rank; out[4*i+1] = R[i].rows.empty() ? -1 : R[i].rows[0]; out[4*i+2] = (int64_t)R[i].rows.size(); out[4*i+3] = R[i].nblocks; }
   }
   return 0;
 }
 int petiga_layout_recv_rows(const petiga_layout* l, int peer_index, int* rows, int capacity) {
-  if (!l || peer_index < 0 || peer_index >= (int)l->L.recv.size() || !rows) return PETIGA_CUDA_ERR_ARG;
-  const auto& r = l->L.recv[peer_index].rows;
+  if (!l) return PETIGA_CUDA_ERR_ARG;
+  const auto& R = l->L.collocation ? l->L.state_recv : l->L.recv;   // the other list is empty
+  if (peer_index < 0 || peer_index >= (int)R.size() || !rows) return PETIGA_CUDA_ERR_ARG;
+  const auto& r = R[peer_index].rows;
   for (int i = 0; i < (int)r.size() && i < capacity; i++) rows[i] = r[i];
+  return 0;
+}
+int petiga_layout_staterow(const petiga_layout* l, int* nstate, int* out) {
+  if (!l) return PETIGA_CUDA_ERR_ARG;
+  if (!l->L.collocation) { pc::set_error("layout_staterow: only collocation layouts have a state numbering (Galerkin: localrow)"); return PETIGA_CUDA_ERR_ARG; }
+  if (nstate) *nstate = l->L.nstate;
+  if (out) memcpy(out, l->L.staterow.data(), l->L.staterow.size() * sizeof(int));
   return 0;
 }
 

@@ -23,6 +23,7 @@ struct petiga_cuda_plan {
   pc::DevAxis dax[3];
   std::vector<void*> allocs;      // everything cudaMalloc'ed by the plan (freed on destroy)
   int* d_localrow = nullptr;
+  int* d_staterow = nullptr;      // collocation plans: ghost box -> state row (Layout::staterow)
   int64_t* d_rowbase = nullptr;
   int* d_rowG[3] = {nullptr, nullptr, nullptr};
   int* d_first[3] = {nullptr, nullptr, nullptr};
@@ -58,11 +59,11 @@ struct petiga_cuda_plan {
   // unified local buffers (multi-rank) and exchange staging
   double* d_ghost_values = nullptr; size_t ghost_values_cap = 0;
   double* d_rhs_loc = nullptr;     // [nloc*dof]
-  double* d_U_loc = nullptr;       // [nloc*dof]
+  double* d_U_loc = nullptr;       // [nloc*dof] (collocation: [nstate*dof])
   double* d_V_loc = nullptr;
   double* d_W_loc = nullptr;
   double* d_recv = nullptr; size_t recv_cap = 0;
-  int* d_recv_rows = nullptr;      // concatenated recv row lists
+  int* d_recv_rows = nullptr;      // concatenated recv row lists (collocation: the state_recv lists)
   int64_t* d_recv_off = nullptr;   // same indexing: block offset of each listed row inside its peer's slab
   std::vector<size_t> recv_row_off;
   // host staging for *_host entry points
@@ -117,7 +118,10 @@ bool kron_applicable(const petiga_cuda_plan* P, int slot, int form);
 int launch_kronecker(petiga_cuda_plan* P, int slot, int block, double* values, double* rhs);
 // ghost exchange (pc_comm.cu)
 int exchange_ghost_rows(petiga_cuda_plan* P, int block, double* values, double* rhs, bool mat, bool vec);
-int halo_state(petiga_cuda_plan* P, const double* U_own, double* U_loc);
+// state halo: U_loc = the owned part, then the runs of `ghost` received from their owners; `owned` lists what each neighbour reads
+// and must be the lists uploaded to d_recv_rows (Galerkin plans: L.send / L.recv; collocation plans: L.state_send / L.state_recv)
+int halo_state(petiga_cuda_plan* P, const std::vector<Layout::Peer>& ghost, const std::vector<Layout::Recv>& owned, const double* U_own,
+               double* U_loc);
 int nccl_load();
 int allgather_owned(petiga_cuda_plan* P, const double* owned, double* full);
 int allreduce_sum(petiga_cuda_plan* P, double* d_buf, int n);
@@ -127,6 +131,8 @@ void nvtx_push(const char* name);
 void fill_fix_sides(const petiga_cuda_plan* P, bool loads, FixSide out[3][2]);
 // collocation rows (pc_colloc.cu): every value of the owned rows and the owned right-hand side, written once
 int launch_collocation(petiga_cuda_plan* P, int slot, int form, double* values, double* rhs);
+// the Bratu collocation slots (Function/Jacobian, IFunction/IJacobian); U, V in the state numbering (Layout::staterow)
+int launch_collocation_state(petiga_cuda_plan* P, int slot, const double* U, const double* V, double shift, double* values, double* rhs);
 // boundary-integral pass (pc_bnd.cu)
 int launch_boundary_pass(petiga_cuda_plan* P, int slot, int form, const double* prm, double* rhs, bool apply_fix);
 }  // namespace pc

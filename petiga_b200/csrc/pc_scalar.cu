@@ -330,7 +330,7 @@ extern "C" int petiga_cuda_compute_scalar(petiga_cuda_plan* P, int scalar_id, co
   PC_CUDA(cudaSetDevice(P->device));
   const double* U_k = U;
   if (L.nranks > 1 && U) {   // IGAGetLocalVecArray: G2L halo (petigavec.c:256-269)
-    int rc = halo_state(P, U, P->d_U_loc);
+    int rc = halo_state(P, L.send, L.recv, U, P->d_U_loc);
     if (rc) return rc;
     U_k = P->d_U_loc;
   }

@@ -23,6 +23,8 @@ FORMS = {
     # collocation forms (SetUseCollocation(True)): the strong form at the Greville points
     "LAPLACE_COLLOCATION": {"SYSTEM": "IGADeviceForm_Laplace_SystemCollocation"},
     "CONVTEST_COLLOCATION": {"SYSTEM": "IGADeviceForm_ConvTest_Collocation"},
+    "BRATU_COLLOCATION": {"FUNCTION": "IGADeviceForm_Bratu_FunctionCollocation", "JACOBIAN": "IGADeviceForm_Bratu_JacobianCollocation",
+                          "IFUNCTION": "IGADeviceForm_Bratu_IFunctionCollocation", "IJACOBIAN": "IGADeviceForm_Bratu_IJacobianCollocation"},
     "MASS": {"SYSTEM": "IGADeviceForm_Mass_System", "MATRIX": "IGADeviceForm_Mass_Matrix", "VECTOR": "IGADeviceForm_Mass_Vector"},
     "ELASTICITY3D": {"SYSTEM": "IGADeviceForm_Elasticity3D_System"},
     "ELASTICITY": {"SYSTEM": "IGADeviceForm_Elasticity_System"},
@@ -537,6 +539,14 @@ class Layout:
         out = np.zeros((max(n.value, 1), 4), dtype=np.int64)
         assert self.L.petiga_layout_exchange(self.h, kind, C.byref(n), out.ctypes.data_as(C.POINTER(C.c_int64)), n.value) == 0
         return out[:n.value]
+
+    def staterow(self):
+        """collocation layouts: (state row of every ghost-box node, nstate)"""
+        out = np.empty(self.sizes()["nghostbox"], dtype=np.int32)
+        n = C.c_int()
+        rc = self.L.petiga_layout_staterow(self.h, C.byref(n), out.ctypes.data_as(_ip))
+        assert rc == 0, rc
+        return out, n.value
 
     def recv_rows(self, peer_index, n):
         rows = np.empty(n, dtype=np.int32)
