@@ -51,18 +51,6 @@ int cuda_fail(cudaError_t e, const char* what) {
   return PETIGA_CUDA_ERR_CUDA;
 }
 
-template <typename T>
-static int upload(petiga_cuda_plan* P, const T* src, size_t n, T** dst) {
-  *dst = nullptr;
-  if (n == 0) n = 1;
-  void* d = nullptr;
-  PC_CUDA(cudaMalloc(&d, n * sizeof(T)));
-  P->allocs.push_back(d);
-  if (src) PC_CUDA(cudaMemcpyAsync(d, src, n * sizeof(T), cudaMemcpyHostToDevice, P->stream));
-  *dst = static_cast<T*>(d);
-  return 0;
-}
-
 // ---- pattern kernel: one warp per owned row, closed-form positions (IGACreateMat: petigamat.c:448-537) ----
 struct PatParams {
   const int* rowG[3]; const int* W[3]; const uint32_t* seg[3]; const int* first[3]; const int* own[3];
@@ -304,41 +292,43 @@ int petiga_cuda_plan_create(petiga_cuda_plan** plan, const petiga_cuda_space* sp
   cudaEventCreate(&P->ev0);
   cudaEventCreate(&P->ev1);
   const Layout& L = P->L;
+  cudaStream_t st = P->stream;
   for (int d = 0; d < 3; d++) {
     const AxisLayout& a = L.ax[d];
+    petiga_cuda_plan::AxisTables& t = P->d_ax[d];
     DevAxis& da = P->dax[d];
     const size_t nq = (size_t)a.nel * a.nqp;
     if (!sp->value[d] || !sp->weight[d] || !sp->point[d] || !sp->detJac[d]) { set_error("missing basis tables"); return bail(PETIGA_CUDA_ERR_ARG); }
-    double *v, *w, *pt, *dj; int *off, *W, *lo, *simp; uint32_t* seg;
-    if ((rc = upload(P, sp->value[d], nq * (a.p + 1) * 5, &v))) return bail(rc);
-    if ((rc = upload(P, sp->weight[d], nq, &w))) return bail(rc);
-    if ((rc = upload(P, sp->point[d], nq, &pt))) return bail(rc);
-    if ((rc = upload(P, sp->detJac[d], (size_t)a.nel, &dj))) return bail(rc);
-    if ((rc = upload(P, sp->offset[d], (size_t)a.nel, &off))) return bail(rc);
-    if ((rc = upload(P, a.W.data(), a.W.size(), &W))) return bail(rc);
-    if ((rc = upload(P, a.lo.data(), a.lo.size(), &lo))) return bail(rc);
-    if ((rc = upload(P, a.seg.data(), a.seg.size(), &seg))) return bail(rc);
-    if ((rc = upload(P, a.simple.data(), a.simple.size(), &simp))) return bail(rc);
-    da.value = v; da.weight = w; da.point = pt; da.detJac = dj; da.offset = off; da.W = W; da.lo = lo; da.seg = seg; da.simple = simp;
+    if ((rc = t.value.upload(sp->value[d], nq * (a.p + 1) * 5, st))) return bail(rc);
+    if ((rc = t.weight.upload(sp->weight[d], nq, st))) return bail(rc);
+    if ((rc = t.point.upload(sp->point[d], nq, st))) return bail(rc);
+    if ((rc = t.detJac.upload(sp->detJac[d], (size_t)a.nel, st))) return bail(rc);
+    if ((rc = t.offset.upload(sp->offset[d], (size_t)a.nel, st))) return bail(rc);
+    if ((rc = t.W.upload(a.W.data(), a.W.size(), st))) return bail(rc);
+    if ((rc = t.lo.upload(a.lo.data(), a.lo.size(), st))) return bail(rc);
+    if ((rc = t.seg.upload(a.seg.data(), a.seg.size(), st))) return bail(rc);
+    if ((rc = t.simple.upload(a.simple.data(), a.simple.size(), st))) return bail(rc);
+    da.value = t.value.get(); da.weight = t.weight.get(); da.point = t.point.get(); da.detJac = t.detJac.get(); da.offset = t.offset.get();
+    da.W = t.W.get(); da.lo = t.lo.get(); da.seg = t.seg.get(); da.simple = t.simple.get();
     da.nel = a.nel; da.nqp = a.nqp; da.nen = a.p + 1; da.p = a.p; da.gs = a.gs; da.gw = a.gw; da.es = a.es; da.ew = a.ew;
     da.periodic = a.periodic; da.nnp = a.nnp;
     P->detJac_h[d].assign(sp->detJac[d], sp->detJac[d] + a.nel);
-    if ((rc = upload(P, L.rowG[d].data(), L.rowG[d].size(), &P->d_rowG[d]))) return bail(rc);
-    if ((rc = upload(P, a.first.data(), a.first.size(), &P->d_first[d]))) return bail(rc);
-    if ((rc = upload(P, a.own.data(), a.own.size(), &P->d_own[d]))) return bail(rc);
-    if ((rc = upload(P, a.box_ls.data(), a.box_ls.size(), &P->d_box_ls[d]))) return bail(rc);
-    if ((rc = upload(P, a.box_lw.data(), a.box_lw.size(), &P->d_box_lw[d]))) return bail(rc);
+    if ((rc = t.rowG.upload(L.rowG[d].data(), L.rowG[d].size(), st))) return bail(rc);
+    if ((rc = t.first.upload(a.first.data(), a.first.size(), st))) return bail(rc);
+    if ((rc = t.own.upload(a.own.data(), a.own.size(), st))) return bail(rc);
+    if ((rc = t.box_ls.upload(a.box_ls.data(), a.box_ls.size(), st))) return bail(rc);
+    if ((rc = t.box_lw.upload(a.box_lw.data(), a.box_lw.size(), st))) return bail(rc);
   }
-  if ((rc = upload(P, L.localrow.data(), L.localrow.size(), &P->d_localrow))) return bail(rc);
-  if ((rc = upload(P, L.rowbase.data(), L.rowbase.size(), &P->d_rowbase))) return bail(rc);
-  if ((rc = upload(P, L.rank_start.data(), L.rank_start.size(), &P->d_rank_start))) return bail(rc);
-  if (L.collocation && (rc = upload(P, L.staterow.data(), L.staterow.size(), &P->d_staterow))) return bail(rc);
+  if ((rc = P->d_localrow.upload(L.localrow.data(), L.localrow.size(), st))) return bail(rc);
+  if ((rc = P->d_rowbase.upload(L.rowbase.data(), L.rowbase.size(), st))) return bail(rc);
+  if ((rc = P->d_rank_start.upload(L.rank_start.data(), L.rank_start.size(), st))) return bail(rc);
+  if (L.collocation && (rc = P->d_staterow.upload(L.staterow.data(), L.staterow.size(), st))) return bail(rc);
   if (L.nranks > 1) {
     const size_t nl = (size_t)L.nloc * L.dof, ns = (size_t)(L.collocation ? L.nstate : L.nloc) * L.dof;
-    if ((rc = upload<double>(P, nullptr, nl, &P->d_rhs_loc))) return bail(rc);
-    if ((rc = upload<double>(P, nullptr, ns, &P->d_U_loc))) return bail(rc);
-    if ((rc = upload<double>(P, nullptr, ns, &P->d_V_loc))) return bail(rc);
-    if ((rc = upload<double>(P, nullptr, nl, &P->d_W_loc))) return bail(rc);
+    if ((rc = P->d_rhs_loc.reserve(nl))) return bail(rc);
+    if ((rc = P->d_U_loc.reserve(ns))) return bail(rc);
+    if ((rc = P->d_V_loc.reserve(ns))) return bail(rc);
+    if ((rc = P->d_W_loc.reserve(nl))) return bail(rc);
     std::vector<int> rows;
     std::vector<int64_t> offs;      // prefix sum of the row lengths inside each peer's slab (the sender packs rows back to back)
     P->recv_row_off.clear();
@@ -349,8 +339,8 @@ int petiga_cuda_plan_create(petiga_cuda_plan** plan, const petiga_cuda_space* sp
       for (int row : r.rows) { offs.push_back(o); o += L.rowbase[row + 1] - L.rowbase[row]; }
     }
     P->recv_row_off.push_back(rows.size());
-    if ((rc = upload(P, rows.data(), rows.size(), &P->d_recv_rows))) return bail(rc);
-    if ((rc = upload(P, offs.data(), offs.size(), &P->d_recv_off))) return bail(rc);
+    if ((rc = P->d_recv_rows.upload(rows.data(), rows.size(), st))) return bail(rc);
+    if ((rc = P->d_recv_off.upload(offs.data(), offs.size(), st))) return bail(rc);
   }
   cudaError_t e = cudaStreamSynchronize(P->stream);
   if (e != cudaSuccess) return bail(cuda_fail(e, "plan upload"));
@@ -362,15 +352,10 @@ int petiga_cuda_plan_destroy(petiga_cuda_plan* P) {
   if (!P) return 0;
   cudaSetDevice(P->device);
   if (P->stream) cudaStreamSynchronize(P->stream);
-  for (void* d : P->allocs) cudaFree(d);
-  for (int b = 0; b < 2; b++) { cudaFree(P->d_rowptr[b]); cudaFree(P->d_colidx[b]); }
-  cudaFree(P->d_X); cudaFree(P->d_W); cudaFree(P->d_fixtable); cudaFree(P->d_ghost_values); cudaFree(P->d_recv);
-  cudaFree(P->d_scalar); cudaFree(P->d_sf3_dprime); cudaFree(P->d_solve_work); cudaFree(P->d_solve_xfull); cudaFree(P->d_gmres_work); cudaFree(P->d_values_own); cudaFree(P->d_rhs_own); cudaFree(P->d_U_own); cudaFree(P->d_V_own);
-  if (P->h_pinned) cudaFreeHost(P->h_pinned);
   if (P->ev0) cudaEventDestroy(P->ev0);
   if (P->ev1) cudaEventDestroy(P->ev1);
   if (P->own_stream && P->stream) cudaStreamDestroy(P->stream);
-  delete P;
+  delete P;   // the DevBuf members free the plan's device memory, with its device current
   return 0;
 }
 
@@ -406,18 +391,20 @@ int petiga_cuda_set_geometry(petiga_cuda_plan* P, int nsd, const double* X, cons
   if (!P) return PETIGA_CUDA_ERR_ARG;
   PC_CUDA(cudaSetDevice(P->device));
   PC_CUDA(cudaStreamSynchronize(P->stream));
-  cudaFree(P->d_X); cudaFree(P->d_W);
-  P->d_X = P->d_W = nullptr;
+  P->d_X.reset(); P->d_W.reset();
   P->config_version++;
   if (!X) return 0;
   if (nsd != P->L.dim) { set_error("geometry: nsd must equal dim on the device path (manifolds unsupported)"); return PETIGA_CUDA_ERR_SUP; }
   const size_t ng = P->L.localrow.size();
-  PC_CUDA(cudaMalloc(&P->d_X, ng * nsd * sizeof(double)));
-  PC_CUDA(cudaMemcpy(P->d_X, X, ng * nsd * sizeof(double), cudaMemcpyHostToDevice));
+  DevBuf<double> dX, dW;   // published only when both are complete
+  int rc = dX.reserve(ng * nsd);
+  if (rc) return rc;
+  PC_CUDA(cudaMemcpy(dX.get(), X, ng * nsd * sizeof(double), cudaMemcpyHostToDevice));
   if (W) {
-    PC_CUDA(cudaMalloc(&P->d_W, ng * sizeof(double)));
-    PC_CUDA(cudaMemcpy(P->d_W, W, ng * sizeof(double), cudaMemcpyHostToDevice));
+    if ((rc = dW.reserve(ng))) return rc;
+    PC_CUDA(cudaMemcpy(dW.get(), W, ng * sizeof(double), cudaMemcpyHostToDevice));
   }
+  P->d_X = std::move(dX); P->d_W = std::move(dW);
   return 0;
 }
 
@@ -425,8 +412,7 @@ int petiga_cuda_set_bc(petiga_cuda_plan* P, const petiga_cuda_bc* bc) {
   if (!P) return PETIGA_CUDA_ERR_ARG;
   PC_CUDA(cudaSetDevice(P->device));
   PC_CUDA(cudaStreamSynchronize(P->stream));
-  cudaFree(P->d_fixtable);
-  P->d_fixtable = nullptr;
+  P->d_fixtable.reset();
   P->has_bc = false;
   P->config_version++;
   memset(&P->bc, 0, sizeof(P->bc));
@@ -460,8 +446,11 @@ int petiga_cuda_set_bc(petiga_cuda_plan* P, const petiga_cuda_bc* bc) {
   P->bc.fixtableU = nullptr;
   if (bc->fixtableU) {
     const size_t n = P->L.localrow.size() * P->L.dof;
-    PC_CUDA(cudaMalloc(&P->d_fixtable, n * sizeof(double)));
-    PC_CUDA(cudaMemcpy(P->d_fixtable, bc->fixtableU, n * sizeof(double), cudaMemcpyHostToDevice));
+    DevBuf<double> table;
+    int rc = table.reserve(n);
+    if (rc) return rc;
+    PC_CUDA(cudaMemcpy(table.get(), bc->fixtableU, n * sizeof(double), cudaMemcpyHostToDevice));
+    P->d_fixtable = std::move(table);
   }
   return 0;
 }
@@ -471,27 +460,26 @@ int petiga_cuda_set_fixtable_device(petiga_cuda_plan* P, const double* table_own
   if (P->L.collocation && table_own) { set_error("set_fixtable_device: IGASetFixTable is not supported on a collocation plan"); return PETIGA_CUDA_ERR_SUP; }
   PC_CUDA(cudaSetDevice(P->device));
   PC_CUDA(cudaStreamSynchronize(P->stream));
-  cudaFree(P->d_fixtable);
-  P->d_fixtable = nullptr;
+  P->d_fixtable.reset();
   P->config_version++;
   if (!table_own) return 0;
   const Layout& L = P->L;
   const size_t ng = L.localrow.size();
-  PC_CUDA(cudaMalloc(&P->d_fixtable, ng * L.dof * sizeof(double)));
+  DevBuf<double> table, tmp;              // the table is published only once it has been written
+  int rc = table.reserve(ng * L.dof);
+  if (rc) return rc;
   const double* loc = table_own;          // one rank: local rows == owned rows
-  double* tmp = nullptr;
   if (L.nranks > 1) {                     // ghost nodes carry their owner's table value (VecScatter g2l)
-    PC_CUDA(cudaMalloc(&tmp, (size_t)L.nloc * L.dof * sizeof(double)));
-    int rc = halo_state(P, L.send, L.recv, table_own, tmp);
-    if (rc) { cudaFree(tmp); return rc; }
-    loc = tmp;
+    if ((rc = tmp.reserve((size_t)L.nloc * L.dof))) return rc;
+    if ((rc = halo_state(P, L.send, L.recv, table_own, tmp.get()))) return rc;
+    loc = tmp.get();
   }
   const int blocks = (int)std::min<size_t>((ng * L.dof + 255) / 256, (size_t)P->num_sms * 8);
-  fixtable_scatter_kernel<<<std::max(blocks, 1), 256, 0, P->stream>>>(P->d_localrow, loc, P->d_fixtable, ng, L.dof);
+  fixtable_scatter_kernel<<<std::max(blocks, 1), 256, 0, P->stream>>>(P->d_localrow.get(), loc, table.get(), ng, L.dof);
   PC_CUDA(cudaGetLastError());
   P->launches++;
   PC_CUDA(cudaStreamSynchronize(P->stream));
-  cudaFree(tmp);
+  P->d_fixtable = std::move(table);
   return 0;
 }
 
@@ -535,32 +523,35 @@ int petiga_cuda_plan_pattern(petiga_cuda_plan* P, int block, int* nrows, int64_t
   const int64_t n = L.nnz_own * bs * bs;
   if (n > INT32_MAX) { set_error("pattern: more than 2^31-1 nonzeros on one rank; use the block (BAIJ) layout or more ranks"); return PETIGA_CUDA_ERR_SUP; }
   PC_CUDA(cudaSetDevice(P->device));
-  if (!P->d_rowptr[block]) {
+  if (!P->d_rowptr[block]) {   // built into local buffers and published once complete, so a set rowptr means a filled colidx
     std::vector<int> rp((size_t)L.nown * bs + 1);
     rp[0] = 0;
     for (int r = 0; r < L.nown; r++) {
       int W = L.rowW[0][r] * L.rowW[1][r] * L.rowW[2][r];
       for (int k = 0; k < bs; k++) rp[(size_t)r * bs + k + 1] = (int)(L.rowbase[r] * bs * bs + (int64_t)(k + 1) * W * bs);
     }
-    PC_CUDA(cudaMalloc(&P->d_rowptr[block], rp.size() * sizeof(int)));
-    PC_CUDA(cudaMemcpyAsync(P->d_rowptr[block], rp.data(), rp.size() * sizeof(int), cudaMemcpyHostToDevice, P->stream));
-    PC_CUDA(cudaMalloc(&P->d_colidx[block], (size_t)(n > 0 ? n : 1) * sizeof(int)));
+    DevBuf<int> rowptr, colidx;
+    int rc = rowptr.upload(rp.data(), rp.size(), P->stream);
+    if (rc) return rc;
+    if ((rc = colidx.reserve((size_t)n))) return rc;
     PatParams pp;
     for (int d = 0; d < 3; d++) {
-      pp.rowG[d] = P->d_rowG[d]; pp.W[d] = P->dax[d].W; pp.seg[d] = P->dax[d].seg; pp.first[d] = P->d_first[d]; pp.own[d] = P->d_own[d];
-      pp.box_ls[d] = P->d_box_ls[d]; pp.box_lw[d] = P->d_box_lw[d]; pp.gs[d] = L.ax[d].gs; pp.nnp[d] = L.ax[d].nnp; pp.Pn[d] = L.ax[d].P;
+      const petiga_cuda_plan::AxisTables& t = P->d_ax[d];
+      pp.rowG[d] = t.rowG.get(); pp.W[d] = P->dax[d].W; pp.seg[d] = P->dax[d].seg; pp.first[d] = t.first.get(); pp.own[d] = t.own.get();
+      pp.box_ls[d] = t.box_ls.get(); pp.box_lw[d] = t.box_lw.get(); pp.gs[d] = L.ax[d].gs; pp.nnp[d] = L.ax[d].nnp; pp.Pn[d] = L.ax[d].P;
     }
-    pp.rank_start = P->d_rank_start; pp.rowbase = P->d_rowbase; pp.nown = L.nown; pp.bs = bs; pp.colidx = P->d_colidx[block];
+    pp.rank_start = P->d_rank_start.get(); pp.rowbase = P->d_rowbase.get(); pp.nown = L.nown; pp.bs = bs; pp.colidx = colidx.get();
     const int blocks = std::max(1, std::min((L.nown + 7) / 8, P->num_sms * 16));
     pattern_kernel<<<blocks, 256, 0, P->stream>>>(pp);
     PC_CUDA(cudaGetLastError());
     P->launches++;
     PC_CUDA(cudaStreamSynchronize(P->stream));
+    P->d_rowptr[block] = std::move(rowptr); P->d_colidx[block] = std::move(colidx);
   }
   if (nrows) *nrows = L.nown * bs;
   if (nnz) *nnz = n;
-  if (d_rowptr) *d_rowptr = P->d_rowptr[block];
-  if (d_colidx) *d_colidx = P->d_colidx[block];
+  if (d_rowptr) *d_rowptr = P->d_rowptr[block].get();
+  if (d_colidx) *d_colidx = P->d_colidx[block].get();
   return 0;
 }
 
@@ -574,15 +565,6 @@ int petiga_cuda_plan_pattern_host(petiga_cuda_plan* P, int block, int* rowptr, i
 }
 
 // ---------------------------------------------------------------------------------------------
-static int ensure(double** buf, size_t* cap, size_t n) {
-  if (*cap >= n && *buf) return 0;
-  cudaFree(*buf);
-  *buf = nullptr; *cap = 0;
-  PC_CUDA(cudaMalloc(buf, (n ? n : 1) * sizeof(double)));
-  *cap = n;
-  return 0;
-}
-
 int petiga_cuda_compute(petiga_cuda_plan* P, int slot, int block, double shift, const double* V, double t, const double* U,
                         double* values, double* rhs) {
   return petiga_cuda_compute_ext(P, slot, block, shift, V, t, U, 0.0, nullptr, 0.0, values, rhs);
@@ -622,11 +604,11 @@ int petiga_cuda_compute_ext(petiga_cuda_plan* P, int slot, int block, double shi
     if (state) {   // Bratu collocation: U (and V) on the collocation ghost box, then the state kernel
       const double *U_k = U, *V_k = V;
       if (L.nranks > 1) {
-        if ((rc = halo_state(P, L.state_send, L.state_recv, U, P->d_U_loc))) return rc;
-        U_k = P->d_U_loc;
+        if ((rc = halo_state(P, L.state_send, L.state_recv, U, P->d_U_loc.get()))) return rc;
+        U_k = P->d_U_loc.get();
         if (slot == PETIGA_SLOT_IFUNCTION) {
-          if ((rc = halo_state(P, L.state_send, L.state_recv, V, P->d_V_loc))) return rc;
-          V_k = P->d_V_loc;
+          if ((rc = halo_state(P, L.state_send, L.state_recv, V, P->d_V_loc.get()))) return rc;
+          V_k = P->d_V_loc.get();
         }
       }
       rc = launch_collocation_state(P, slot, U_k, V_k, shift, values, rhs);
@@ -673,21 +655,21 @@ int petiga_cuda_compute_ext(petiga_cuda_plan* P, int slot, int block, double shi
   double* rhs_k = rhs;
   if (multi) {
     if (quad_mat) {
-      int rc = ensure(&P->d_ghost_values, &P->ghost_values_cap, (size_t)(L.nnz_loc - L.nnz_own) * bs2);
+      int rc = P->d_ghost_values.reserve((size_t)(L.nnz_loc - L.nnz_own) * bs2);
       if (rc) return rc;
-      PC_CUDA(cudaMemsetAsync(P->d_ghost_values, 0, (size_t)(L.nnz_loc - L.nnz_own) * bs2 * sizeof(double), P->stream));
+      PC_CUDA(cudaMemsetAsync(P->d_ghost_values.get(), 0, (size_t)(L.nnz_loc - L.nnz_own) * bs2 * sizeof(double), P->stream));
     }
-    if (want_vec) { rhs_k = P->d_rhs_loc; PC_CUDA(cudaMemsetAsync(rhs_k, 0, (size_t)L.nloc * L.dof * sizeof(double), P->stream)); }
+    if (want_vec) { rhs_k = P->d_rhs_loc.get(); PC_CUDA(cudaMemsetAsync(rhs_k, 0, (size_t)L.nloc * L.dof * sizeof(double), P->stream)); }
   } else if (want_vec) PC_CUDA(cudaMemsetAsync(rhs, 0, nvec * sizeof(double), P->stream));
 
   // IGAGetLocalVecArray: G2L halo of the state vectors (petigavec.c:256-269)
   const double *U_k = U, *V_k = V, *W_k = W;
   if (multi && state) {
-    int rc = halo_state(P, L.send, L.recv, U, P->d_U_loc);
+    int rc = halo_state(P, L.send, L.recv, U, P->d_U_loc.get());
     if (rc) return rc;
-    U_k = P->d_U_loc;
-    if (has_v) { rc = halo_state(P, L.send, L.recv, V, P->d_V_loc); if (rc) return rc; V_k = P->d_V_loc; }
-    if (has_w) { rc = halo_state(P, L.send, L.recv, W, P->d_W_loc); if (rc) return rc; W_k = P->d_W_loc; }
+    U_k = P->d_U_loc.get();
+    if (has_v) { rc = halo_state(P, L.send, L.recv, V, P->d_V_loc.get()); if (rc) return rc; V_k = P->d_V_loc.get(); }
+    if (has_w) { rc = halo_state(P, L.send, L.recv, W, P->d_W_loc.get()); if (rc) return rc; W_k = P->d_W_loc.get(); }
   }
 
   KParams kp;
@@ -696,16 +678,16 @@ int petiga_cuda_compute_ext(petiga_cuda_plan* P, int slot, int block, double shi
   kp.dim = L.dim; kp.dof = L.dof;
   kp.nelem = L.ax[0].ew * L.ax[1].ew * L.ax[2].ew;
   kp.nown = L.nown; kp.nnz_own = L.nnz_own;
-  kp.localrow = P->d_localrow; kp.rowbase = P->d_rowbase;
-  kp.values = values; kp.ghost_values = P->d_ghost_values; kp.rhs = rhs_k;
+  kp.localrow = P->d_localrow.get(); kp.rowbase = P->d_rowbase.get();
+  kp.values = values; kp.ghost_values = P->d_ghost_values.get(); kp.rhs = rhs_k;
   kp.U = state ? U_k : nullptr; kp.V = has_v ? V_k : nullptr; kp.Wv = has_w ? W_k : nullptr;
   kp.shift2 = shift2; kp.t0 = t0;
   kp.face_axis = kp.face_side = -1;
   for (int d = 0; d < 3; d++) {
     kp.maxdeg = std::max(kp.maxdeg, d < L.dim ? L.ax[d].p : 0);
-    for (int s2 = 0; s2 < 2; s2++) { kp.bnd_value[d][s2] = P->d_bnd_value[d][s2]; kp.bnd_point[d][s2] = P->bnd_point[d][s2]; }
+    for (int s2 = 0; s2 < 2; s2++) { kp.bnd_value[d][s2] = P->d_bnd_value[d][s2].get(); kp.bnd_point[d][s2] = P->bnd_point[d][s2]; }
   }
-  kp.X = P->d_X; kp.Wt = P->d_W; kp.fixtable = P->d_fixtable;
+  kp.X = P->d_X.get(); kp.Wt = P->d_W.get(); kp.fixtable = P->d_fixtable.get();
   kp.any_bc = 0;
   const bool apply_bc = (slot != PETIGA_SLOT_VECTOR && slot != PETIGA_SLOT_MATRIX);   // IGAComputeVector/Matrix never fix (petigaksp.c:33-139)
   if (apply_bc) {
@@ -720,25 +702,22 @@ int petiga_cuda_compute_ext(petiga_cuda_plan* P, int slot, int block, double shi
           int fa[2] = {0, 0}, nfa = 0;
           for (int i = 0; i < L.dim; i++) if (i != d) fa[nfa++] = i;
           const int n0 = L.ax[fa[0]].ew, n1 = (L.dim > 2) ? L.ax[fa[1]].ew : 1;
-          if (!P->d_face_dS[d][s]) {
-            void* buf = nullptr;
-            PC_CUDA(cudaMalloc(&buf, (size_t)n0 * n1 * sizeof(double)));
-            P->allocs.push_back(buf);
-            P->d_face_dS[d][s] = (double*)buf;
-            P->face_version[d][s] = -1;
-          }
-          if (P->face_version[d][s] != P->config_version) {
+          DevBuf<double>& dS = P->d_face_dS[d][s];   // recomputed in place when the geometry changes; empty after a failed build
+          if (!dS || P->face_version[d][s] != P->config_version) {
+            int rc = dS.reserve((size_t)n0 * n1);
+            if (rc) return rc;
             FaceParams fp;
             for (int i = 0; i < 3; i++) fp.ax[i] = P->dax[i];
-            fp.dir = d; fp.side = s; fp.n0 = n0; fp.n1 = n1; fp.X = P->d_X; fp.Wt = P->d_W; fp.out = P->d_face_dS[d][s];
+            fp.dir = d; fp.side = s; fp.n0 = n0; fp.n1 = n1; fp.X = P->d_X.get(); fp.Wt = P->d_W.get(); fp.out = dS.get();
             const int nb = (n0 * n1 + 127) / 128;
             if (L.dim == 2) face_area_kernel<2><<<nb, 128, 0, P->stream>>>(fp);
             else face_area_kernel<3><<<nb, 128, 0, P->stream>>>(fp);
-            PC_CUDA(cudaGetLastError());
+            const cudaError_t e = cudaGetLastError();
+            if (e != cudaSuccess) { dS.reset(); return cuda_fail(e, "face_area_kernel"); }
             P->launches++;
             P->face_version[d][s] = P->config_version;
           }
-          kp.face_dS[d][s] = P->d_face_dS[d][s];
+          kp.face_dS[d][s] = dS.get();
         }
       }
   }
@@ -828,18 +807,16 @@ int petiga_cuda_compute_host(petiga_cuda_plan* P, int slot, int block, double sh
   const Layout& L = P->L;
   PC_CUDA(cudaSetDevice(P->device));
   const size_t nval = (size_t)L.nnz_own * L.dof * L.dof, nvec = (size_t)L.nown * L.dof;
-  size_t cap;
-  if (values_host) { int rc = ensure(&P->d_values_own, &P->values_own_cap, nval); if (rc) return rc; }
-  cap = P->d_rhs_own ? nvec : 0; { int rc = ensure(&P->d_rhs_own, &cap, nvec); if (rc) return rc; }
-  if (U_host) { cap = P->d_U_own ? nvec : 0; int rc = ensure(&P->d_U_own, &cap, nvec); if (rc) return rc;
-    PC_CUDA(cudaMemcpyAsync(P->d_U_own, U_host, nvec * sizeof(double), cudaMemcpyHostToDevice, P->stream)); }
-  if (V_host) { cap = P->d_V_own ? nvec : 0; int rc = ensure(&P->d_V_own, &cap, nvec); if (rc) return rc;
-    PC_CUDA(cudaMemcpyAsync(P->d_V_own, V_host, nvec * sizeof(double), cudaMemcpyHostToDevice, P->stream)); }
-  int rc = petiga_cuda_compute(P, slot, block, shift, V_host ? P->d_V_own : nullptr, t, U_host ? P->d_U_own : nullptr,
-                               values_host ? P->d_values_own : nullptr, rhs_host ? P->d_rhs_own : nullptr);
+  int rc = 0;
+  if (values_host && (rc = P->d_values_own.reserve(nval))) return rc;
+  if ((rc = P->d_rhs_own.reserve(nvec))) return rc;
+  if (U_host && (rc = P->d_U_own.upload(U_host, nvec, P->stream))) return rc;
+  if (V_host && (rc = P->d_V_own.upload(V_host, nvec, P->stream))) return rc;
+  rc = petiga_cuda_compute(P, slot, block, shift, V_host ? P->d_V_own.get() : nullptr, t, U_host ? P->d_U_own.get() : nullptr,
+                           values_host ? P->d_values_own.get() : nullptr, rhs_host ? P->d_rhs_own.get() : nullptr);
   if (rc) return rc;
-  if (values_host) PC_CUDA(cudaMemcpyAsync(values_host, P->d_values_own, nval * sizeof(double), cudaMemcpyDeviceToHost, P->stream));
-  if (rhs_host) PC_CUDA(cudaMemcpyAsync(rhs_host, P->d_rhs_own, nvec * sizeof(double), cudaMemcpyDeviceToHost, P->stream));
+  if (values_host) PC_CUDA(cudaMemcpyAsync(values_host, P->d_values_own.get(), nval * sizeof(double), cudaMemcpyDeviceToHost, P->stream));
+  if (rhs_host) PC_CUDA(cudaMemcpyAsync(rhs_host, P->d_rhs_own.get(), nvec * sizeof(double), cudaMemcpyDeviceToHost, P->stream));
   return petiga_cuda_finish(P);
 }
 
@@ -852,10 +829,15 @@ int petiga_cuda_measure_fp64(int device, double seconds, double* tflops_burst, d
   PC_CUDA(cudaSetDevice(device));
   int sms = 0;
   PC_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
-  double* d = nullptr;
-  PC_CUDA(cudaMalloc(&d, 8));
-  cudaEvent_t e0, e1;
-  cudaEventCreate(&e0); cudaEventCreate(&e1);
+  DevBuf<double> out;
+  if ((rc = out.reserve(1))) return rc;
+  double* d = out.get();
+  struct Events {   // destroyed on every return
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    ~Events() { if (e0) cudaEventDestroy(e0); if (e1) cudaEventDestroy(e1); }
+  } ev;
+  cudaEventCreate(&ev.e0); cudaEventCreate(&ev.e1);
+  const cudaEvent_t e0 = ev.e0, e1 = ev.e1;
   const int blocks = sms * 4, iters = 4096;
   const double flop = 2.0 * 64.0 * iters * 256.0 * blocks;      // 64 DFMA per iteration per thread
   double best = 0.0, sus_flop = 0.0;
@@ -878,20 +860,18 @@ int petiga_cuda_measure_fp64(int device, double seconds, double* tflops_burst, d
   PC_CUDA(cudaGetLastError());
   if (tflops_burst) *tflops_burst = best;
   if (tflops_sustained) *tflops_sustained = sus_flop / (ms * 1e-3) / 1e12;
-  cudaEventDestroy(e0); cudaEventDestroy(e1);
-  cudaFree(d);
   return 0;
 }
 
 int petiga_cuda_diff_norm2(const double* d_a, const double* d_b, size_t n, double* diff2, double* ref2) {
   if (!d_a || !d_b || !diff2 || !ref2) return PETIGA_CUDA_ERR_ARG;
   const int blocks = 1184;
-  double* part = nullptr;
-  PC_CUDA(cudaMalloc(&part, 2 * blocks * sizeof(double)));
-  diff_norm_kernel<<<blocks, 256>>>(d_a, d_b, n, part);
+  DevBuf<double> part;
+  int rc = part.reserve(2 * blocks);
+  if (rc) return rc;
+  diff_norm_kernel<<<blocks, 256>>>(d_a, d_b, n, part.get());
   std::vector<double> h(2 * blocks);
-  cudaError_t e = cudaMemcpy(h.data(), part, h.size() * sizeof(double), cudaMemcpyDeviceToHost);
-  cudaFree(part);
+  cudaError_t e = cudaMemcpy(h.data(), part.get(), h.size() * sizeof(double), cudaMemcpyDeviceToHost);
   if (e != cudaSuccess) return cuda_fail(e, "diff_norm2");
   double x = 0.0, y = 0.0;
   for (int b = 0; b < blocks; b++) { x += h[2 * b]; y += h[2 * b + 1]; }

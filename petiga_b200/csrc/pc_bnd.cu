@@ -202,13 +202,13 @@ int launch_boundary_pass(petiga_cuda_plan* P, int slot, int form, const double* 
       memset(&bp, 0, sizeof(bp));
       for (int i = 0; i < 3; i++) {
         bp.ax[i] = P->dax[i];
-        for (int t = 0; t < 2; t++) { bp.bnd_value[i][t] = P->d_bnd_value[i][t]; bp.bnd_point[i][t] = P->bnd_point[i][t]; }
+        for (int t = 0; t < 2; t++) { bp.bnd_value[i][t] = P->d_bnd_value[i][t].get(); bp.bnd_point[i][t] = P->bnd_point[i][t]; }
       }
       int fa[2] = {0, 0}, nfa = 0;
       for (int i = 0; i < L.dim; i++) if (i != d) fa[nfa++] = i;
       bp.dim = L.dim; bp.dof = L.dof; bp.dir = d; bp.side = s;
       bp.n0 = (L.dim > 1) ? L.ax[fa[0]].ew : 1; bp.n1 = (L.dim > 2) ? L.ax[fa[1]].ew : 1;
-      bp.localrow = P->d_localrow; bp.X = P->d_X; bp.Wt = P->d_W; bp.rhs = rhs;
+      bp.localrow = P->d_localrow.get(); bp.X = P->d_X.get(); bp.Wt = P->d_W.get(); bp.rhs = rhs;
       bp.apply_fix = apply_fix ? 1 : 0; bp.form = form; bp.slot = slot;
       memcpy(bp.prm, prm, sizeof(bp.prm));
       int nqf = 1;
@@ -235,14 +235,12 @@ extern "C" int petiga_cuda_set_boundary_tables(petiga_cuda_plan* P, int axis, co
   PC_CUDA(cudaSetDevice(P->device));
   const size_t n = (size_t)(P->L.ax[axis].p + 1) * 5;
   const double* src[2] = {bnd_value0, bnd_value1};
-  for (int s = 0; s < 2; s++) {
-    if (!P->d_bnd_value[axis][s]) {
-      void* buf = nullptr;
-      PC_CUDA(cudaMalloc(&buf, n * sizeof(double)));
-      P->allocs.push_back(buf);
-      P->d_bnd_value[axis][s] = (double*)buf;
-    }
-    PC_CUDA(cudaMemcpy(P->d_bnd_value[axis][s], src[s], n * sizeof(double), cudaMemcpyHostToDevice));
+  for (int s = 0; s < 2; s++) {   // a table whose copy failed is dropped, so the face passes report it as not set
+    DevBuf<double>& b = P->d_bnd_value[axis][s];
+    int rc = b.reserve(n);
+    if (rc) return rc;
+    const cudaError_t e = cudaMemcpy(b.get(), src[s], n * sizeof(double), cudaMemcpyHostToDevice);
+    if (e != cudaSuccess) { b.reset(); return cuda_fail(e, "set_boundary_tables"); }
   }
   P->bnd_point[axis][0] = bnd_point0; P->bnd_point[axis][1] = bnd_point1;
   return 0;

@@ -389,10 +389,10 @@ static void colloc_params(petiga_cuda_plan* P, int slot, double* values, double*
   memset(&cp, 0, sizeof(cp));
   for (int d = 0; d < 3; d++) { cp.ax[d] = P->dax[d]; cp.ls[d] = L.ax[d].ls; cp.lw[d] = L.ax[d].lw; }
   cp.nown = L.nown;
-  cp.rowbase = P->d_rowbase;
+  cp.rowbase = P->d_rowbase.get();
   cp.values = slot_has_mat(slot) ? values : nullptr;
   cp.rhs = slot_has_vec(slot) ? rhs : nullptr;
-  cp.X = P->d_X; cp.Wt = P->d_W;
+  cp.X = P->d_X.get(); cp.Wt = P->d_W.get();
   cp.fix = 0;
   if (slot_fix_kind(slot) && P->has_bc) {   // IGAComputeVector/Matrix never fix (petigaksp.c:33-139)
     FixSide fs[3][2];
@@ -444,7 +444,7 @@ int launch_collocation(petiga_cuda_plan* P, int slot, int form, double* values, 
 int launch_collocation_state(petiga_cuda_plan* P, int slot, const double* U, const double* V, double shift, double* values, double* rhs) {
   CollocParams cp;
   colloc_params(P, slot, values, rhs, cp);
-  cp.staterow = P->d_staterow;
+  cp.staterow = P->d_staterow.get();
   cp.U = U;
   cp.V = slot == PETIGA_SLOT_IFUNCTION ? V : nullptr;
   cp.lambda = P->slots[slot].prm[0];

@@ -75,15 +75,6 @@ int nccl_load() {
   return 0;
 }
 
-static int ensure_recv(petiga_cuda_plan* P, size_t n) {
-  if (P->recv_cap >= n && P->d_recv) return 0;
-  cudaFree(P->d_recv);
-  P->d_recv = nullptr; P->recv_cap = 0;
-  PC_CUDA(cudaMalloc(&P->d_recv, (n ? n : 1) * sizeof(double)));
-  P->recv_cap = n;
-  return 0;
-}
-
 // MPI_Allreduce(SUM) of IGAComputeScalar (src/petigacomp.c:90), in place on the plan's stream
 int allreduce_sum(petiga_cuda_plan* P, double* d_buf, int n) {
   if (!P->nccl) { set_error("multi-rank plan without an NCCL communicator"); return PETIGA_CUDA_ERR_ORDER; }
@@ -128,19 +119,19 @@ int exchange_ghost_rows(petiga_cuda_plan* P, int block, double* values, double* 
   std::vector<size_t> moff(L.recv.size()), voff(L.recv.size());
   for (size_t i = 0; i < L.recv.size(); i++) { moff[i] = total; if (mat) total += (size_t)L.recv[i].nblocks * bs2; }
   for (size_t i = 0; i < L.recv.size(); i++) { voff[i] = total; if (vec) total += L.recv[i].rows.size() * dof; }
-  if ((rc = ensure_recv(P, total))) return rc;
+  if ((rc = P->d_recv.reserve(total))) return rc;
   // a failed Send/Recv must not leave the NCCL group open (ADVICE r1): close it, then report
   ncclResult_t gr = g_nccl.GroupStart();
   if (gr != ncclSuccess) return nccl_fail(gr, "ncclGroupStart");
   auto post = [&](ncclResult_t r) { if (gr == ncclSuccess && r != ncclSuccess) gr = r; };
   for (const auto& s : L.send) {
-    if (mat) post(g_nccl.Send(P->d_ghost_values + (size_t)(s.first_block - L.nnz_own) * bs2, (size_t)s.nblocks * bs2, ncclDouble, s.rank, comm, P->stream));
-    if (vec) post(g_nccl.Send(P->d_rhs_loc + (size_t)s.first_row * dof, (size_t)s.nrows * dof, ncclDouble, s.rank, comm, P->stream));
+    if (mat) post(g_nccl.Send(P->d_ghost_values.get() + (size_t)(s.first_block - L.nnz_own) * bs2, (size_t)s.nblocks * bs2, ncclDouble, s.rank, comm, P->stream));
+    if (vec) post(g_nccl.Send(P->d_rhs_loc.get() + (size_t)s.first_row * dof, (size_t)s.nrows * dof, ncclDouble, s.rank, comm, P->stream));
   }
   for (size_t i = 0; i < L.recv.size(); i++) {
     const auto& r = L.recv[i];
-    if (mat) post(g_nccl.Recv(P->d_recv + moff[i], (size_t)r.nblocks * bs2, ncclDouble, r.rank, comm, P->stream));
-    if (vec) post(g_nccl.Recv(P->d_recv + voff[i], r.rows.size() * dof, ncclDouble, r.rank, comm, P->stream));
+    if (mat) post(g_nccl.Recv(P->d_recv.get() + moff[i], (size_t)r.nblocks * bs2, ncclDouble, r.rank, comm, P->stream));
+    if (vec) post(g_nccl.Recv(P->d_recv.get() + voff[i], r.rows.size() * dof, ncclDouble, r.rank, comm, P->stream));
   }
   ncclResult_t ge = g_nccl.GroupEnd();
   if (gr != ncclSuccess) return nccl_fail(gr, "ncclSend/ncclRecv (ghost rows)");
@@ -149,20 +140,20 @@ int exchange_ghost_rows(petiga_cuda_plan* P, int block, double* values, double* 
   for (size_t i = 0; i < L.recv.size(); i++) {
     const auto& r = L.recv[i];
     const int n = (int)r.rows.size();
-    const int* rows = P->d_recv_rows + P->recv_row_off[i];
+    const int* rows = P->d_recv_rows.get() + P->recv_row_off[i];
     if (mat) {   // per-row offsets inside the slab were uploaded once by petiga_cuda_plan_create: no host work, no sync here
-      add_rows_kernel<<<std::max(1, std::min((n + 7) / 8, P->num_sms * 8)), 256, 0, P->stream>>>(rows, P->d_recv_off + P->recv_row_off[i], n, P->d_rowbase, bs2,
-                                                                                               values, P->d_recv + moff[i]);
+      add_rows_kernel<<<std::max(1, std::min((n + 7) / 8, P->num_sms * 8)), 256, 0, P->stream>>>(rows, P->d_recv_off.get() + P->recv_row_off[i], n, P->d_rowbase.get(), bs2,
+                                                                                               values, P->d_recv.get() + moff[i]);
       PC_CUDA(cudaGetLastError());
       P->launches++;
     }
     if (vec) {
-      add_vec_rows_kernel<<<(n * dof + 255) / 256, 256, 0, P->stream>>>(rows, n, dof, (int64_t)voff[i], P->d_rhs_loc, P->d_recv);
+      add_vec_rows_kernel<<<(n * dof + 255) / 256, 256, 0, P->stream>>>(rows, n, dof, (int64_t)voff[i], P->d_rhs_loc.get(), P->d_recv.get());
       PC_CUDA(cudaGetLastError());
       P->launches++;
     }
   }
-  if (vec) PC_CUDA(cudaMemcpyAsync(rhs, P->d_rhs_loc, (size_t)L.nown * dof * sizeof(double), cudaMemcpyDeviceToDevice, P->stream));
+  if (vec) PC_CUDA(cudaMemcpyAsync(rhs, P->d_rhs_loc.get(), (size_t)L.nown * dof * sizeof(double), cudaMemcpyDeviceToDevice, P->stream));
   return 0;
 }
 
@@ -178,17 +169,17 @@ int halo_state(petiga_cuda_plan* P, const std::vector<Layout::Peer>& ghost, cons
   size_t total = 0;
   std::vector<size_t> off(owned.size());
   for (size_t i = 0; i < owned.size(); i++) { off[i] = total; total += owned[i].rows.size() * dof; }
-  if ((rc = ensure_recv(P, total))) return rc;
+  if ((rc = P->d_recv.reserve(total))) return rc;
   for (size_t i = 0; i < owned.size(); i++) {   // owners pack the rows their neighbours see as ghosts
     const int n = (int)owned[i].rows.size();
-    gather_vec_rows_kernel<<<(n * dof + 255) / 256, 256, 0, P->stream>>>(P->d_recv_rows + P->recv_row_off[i], n, dof, U_own, P->d_recv + off[i]);
+    gather_vec_rows_kernel<<<(n * dof + 255) / 256, 256, 0, P->stream>>>(P->d_recv_rows.get() + P->recv_row_off[i], n, dof, U_own, P->d_recv.get() + off[i]);
     PC_CUDA(cudaGetLastError());
     P->launches++;
   }
   ncclResult_t gr = g_nccl.GroupStart();
   if (gr != ncclSuccess) return nccl_fail(gr, "ncclGroupStart");
   for (size_t i = 0; i < owned.size() && gr == ncclSuccess; i++)
-    gr = g_nccl.Send(P->d_recv + off[i], owned[i].rows.size() * dof, ncclDouble, owned[i].rank, comm, P->stream);
+    gr = g_nccl.Send(P->d_recv.get() + off[i], owned[i].rows.size() * dof, ncclDouble, owned[i].rank, comm, P->stream);
   for (size_t i = 0; i < ghost.size() && gr == ncclSuccess; i++)
     gr = g_nccl.Recv(U_loc + (size_t)ghost[i].first_row * dof, (size_t)ghost[i].nrows * dof, ncclDouble, ghost[i].rank, comm, P->stream);
   ncclResult_t ge = g_nccl.GroupEnd();

@@ -876,22 +876,21 @@ int launch_kronecker(petiga_cuda_plan* P, int slot, int block, double* values, d
   const Layout& L = P->L;
   const int form = P->slots[slot].form;
   FormInfo fi = form_info(form, slot, L.dim, L.dof);
-  if (!P->d_kronrow[0]) {   // 1-D tables, once per plan
-    for (int d = 0; d < 3; d++) {
-      const int nnp = L.ax[d].nnp;
-      void* buf = nullptr;
-      const size_t nM = (size_t)4 * nnp * kMaxW, nmv = (size_t)2 * nnp;
-      PC_CUDA(cudaMalloc(&buf, (nM + nmv + nnp + (size_t)4 * nnp) * sizeof(double) + (size_t)nnp * sizeof(int)));
-      P->allocs.push_back(buf);
-      P->d_kronrow[d] = (double*)buf;
-      double* M = (double*)buf; double* mv = M + nM; double* lsum = mv + nmv; double* rsum = lsum + nnp; int* nsup = (int*)(rsum + (size_t)4 * nnp);
-      const int total = (int)nM;
-      kron_1d_kernel<<<(total + 127) / 128, 128, 0, P->stream>>>(P->dax[d], P->d_first[d], M, mv, nsup, lsum);
-      PC_CUDA(cudaGetLastError());
-      kron_rowsum_kernel<<<(4 * nnp + 127) / 128, 128, 0, P->stream>>>(M, rsum, nnp);
-      PC_CUDA(cudaGetLastError());
-      P->launches += 2;
-    }
+  for (int d = 0; d < 3; d++) {   // 1-D tables, once per plan and axis (into a local buffer, kept once the build has been launched)
+    if (P->d_ax[d].kronrow) continue;
+    const int nnp = L.ax[d].nnp;
+    const size_t nM = (size_t)4 * nnp * kMaxW, nmv = (size_t)2 * nnp;
+    DevBuf<double> buf;   // M, mv, lsum, rsum, then the nnp ints of nsup in (nnp + 1) / 2 doubles
+    int rc = buf.reserve(nM + nmv + nnp + (size_t)4 * nnp + (size_t)(nnp + 1) / 2);
+    if (rc) return rc;
+    double* M = buf.get(); double* mv = M + nM; double* lsum = mv + nmv; double* rsum = lsum + nnp; int* nsup = (int*)(rsum + (size_t)4 * nnp);
+    const int total = (int)nM;
+    kron_1d_kernel<<<(total + 127) / 128, 128, 0, P->stream>>>(P->dax[d], P->d_ax[d].first.get(), M, mv, nsup, lsum);
+    PC_CUDA(cudaGetLastError());
+    kron_rowsum_kernel<<<(4 * nnp + 127) / 128, 128, 0, P->stream>>>(M, rsum, nnp);
+    PC_CUDA(cudaGetLastError());
+    P->launches += 2;
+    P->d_ax[d].kronrow = std::move(buf);
   }
   // the parameter block only depends on (slot, form, parameters, block layout, boundary conditions): build it once and
   // reuse it, so that a repeated assembly costs one kernel launch on the host side
@@ -908,12 +907,12 @@ int launch_kronecker(petiga_cuda_plan* P, int slot, int block, double* values, d
   for (int d = 0; d < 3; d++) {
     const int nnp = L.ax[d].nnp;
     const size_t nM = (size_t)4 * nnp * kMaxW, nmv = (size_t)2 * nnp;
-    kp.M[d] = P->d_kronrow[d]; kp.mv[d] = kp.M[d] + nM; kp.lsum[d] = kp.mv[d] + nmv; kp.rsum[d] = kp.lsum[d] + nnp; kp.nsup[d] = (const int*)(kp.rsum[d] + (size_t)4 * nnp);
-    kp.first[d] = P->d_first[d]; kp.Wg[d] = P->dax[d].W; kp.lo[d] = P->dax[d].lo; kp.seg[d] = P->dax[d].seg; kp.simp[d] = P->dax[d].simple;
+    kp.M[d] = P->d_ax[d].kronrow.get(); kp.mv[d] = kp.M[d] + nM; kp.lsum[d] = kp.mv[d] + nmv; kp.rsum[d] = kp.lsum[d] + nnp; kp.nsup[d] = (const int*)(kp.rsum[d] + (size_t)4 * nnp);
+    kp.first[d] = P->d_ax[d].first.get(); kp.Wg[d] = P->dax[d].W; kp.lo[d] = P->dax[d].lo; kp.seg[d] = P->dax[d].seg; kp.simp[d] = P->dax[d].simple;
     kp.ls[d] = L.ax[d].ls; kp.lw[d] = L.ax[d].lw; kp.gs[d] = L.ax[d].gs; kp.gw[d] = L.ax[d].gw; kp.nnp[d] = nnp; kp.periodic[d] = L.ax[d].periodic;
     if (L.ax[d].periodic) simple = false;
   }
-  kp.rowbase = P->d_rowbase; kp.localrow = P->d_localrow; kp.fixtable = P->d_fixtable;
+  kp.rowbase = P->d_rowbase.get(); kp.localrow = P->d_localrow.get(); kp.fixtable = P->d_fixtable.get();
   kp.dim = L.dim; kp.dof = L.dof; kp.block = block; kp.slot = slot; kp.simple = simple; kp.wfull0 = 2 * L.ax[0].p + 1;
   kp.bulk = P->kron_bulk;
   kp.minb_rows = P->kron_minb_rows;

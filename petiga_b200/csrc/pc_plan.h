@@ -7,6 +7,62 @@
 
 #include "pc_device.h"
 
+namespace pc {
+void set_error(const std::string& msg);
+int cuda_fail(cudaError_t e, const char* what);
+#define PC_CUDA(call)                                              \
+  do {                                                             \
+    cudaError_t _e = (call);                                       \
+    if (_e != cudaSuccess) return pc::cuda_fail(_e, #call);        \
+  } while (0)
+
+// Sole owner of one device allocation of n elements of T; non-empty means allocated.  It frees on the current device, so whoever
+// drops one makes the owning device current first.  reserve() is grow-only: it frees before it allocates, so a regrow never holds
+// two buffers at once, and the contents are undefined after it.  A failed reserve() leaves the buffer empty.
+template <typename T>
+class DevBuf {
+ public:
+  DevBuf() = default;
+  DevBuf(DevBuf&& o) noexcept : p_(o.p_), n_(o.n_) { o.p_ = nullptr; o.n_ = 0; }
+  DevBuf& operator=(DevBuf&& o) noexcept {
+    if (this != &o) { reset(); p_ = o.p_; n_ = o.n_; o.p_ = nullptr; o.n_ = 0; }
+    return *this;
+  }
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  ~DevBuf() { reset(); }
+  T* get() const { return p_; }
+  size_t size() const { return n_; }
+  explicit operator bool() const { return p_ != nullptr; }
+  void reset() {
+    if (p_) cudaFree(p_);
+    p_ = nullptr;
+    n_ = 0;
+  }
+  int reserve(size_t n) {
+    if (p_ && n <= n_) return 0;
+    reset();
+    if (n == 0) n = 1;
+    void* d = nullptr;
+    PC_CUDA(cudaMalloc(&d, n * sizeof(T)));
+    p_ = static_cast<T*>(d);
+    n_ = n;
+    return 0;
+  }
+  // reserve(n), then n elements from the host on `stream` (none when src is NULL)
+  int upload(const T* src, size_t n, cudaStream_t stream) {
+    int rc = reserve(n);
+    if (rc) return rc;
+    if (src) PC_CUDA(cudaMemcpyAsync(p_, src, n * sizeof(T), cudaMemcpyHostToDevice, stream));
+    return 0;
+  }
+
+ private:
+  T* p_ = nullptr;
+  size_t n_ = 0;
+};
+}  // namespace pc
+
 struct petiga_cuda_plan {
   pc::Layout L;
   int device = 0;
@@ -19,60 +75,57 @@ struct petiga_cuda_plan {
   std::vector<double> detJac_h[3];
   std::vector<int> first_h[3];
 
-  // device tables
-  pc::DevAxis dax[3];
-  std::vector<void*> allocs;      // everything cudaMalloc'ed by the plan (freed on destroy)
-  int* d_localrow = nullptr;
-  int* d_staterow = nullptr;      // collocation plans: ghost box -> state row (Layout::staterow)
-  int64_t* d_rowbase = nullptr;
-  int* d_rowG[3] = {nullptr, nullptr, nullptr};
-  int* d_first[3] = {nullptr, nullptr, nullptr};
-  int* d_own[3] = {nullptr, nullptr, nullptr};
-  int* d_box_ls[3] = {nullptr, nullptr, nullptr};
-  int* d_box_lw[3] = {nullptr, nullptr, nullptr};
-  int* d_rank_start = nullptr;
-  // 1-D element matrices for the separable path: [comp pair][nel][nen][nen]
-  double* d_kron1d[3] = {nullptr, nullptr, nullptr};
-  double* d_kronrow[3] = {nullptr, nullptr, nullptr};   // 1-D global banded matrices [4][nnp][kMaxW]
-  double* d_sfpp[3] = {nullptr, nullptr, nullptr};      // pair-product tables of the sum-factorised kernel
-  double* d_sf3pp[3] = {nullptr, nullptr, nullptr};     // the same products in the fragment layout of the third-generation kernel
-  double* d_solve_work = nullptr; size_t solve_work_cap = 0;     // pc_solve.cu: r, z, p, Ap, 1/diag, reduction partials, scalars
-  double* d_solve_xfull = nullptr; size_t solve_xfull_cap = 0;   // full-length operand of a distributed matrix-vector product
-  double* d_gmres_work = nullptr; size_t gmres_work_cap = 0;     // pc_solve.cu GMRES: Krylov basis, w, z, 1/diag, partials, Hessenberg, rotations
-  double* d_sf3_dprime = nullptr; size_t sf3_dprime_cap = 0;   // D'[element][pair][64] of the geometry pre-pass (mapped geometry)
+  // device tables; every buffer the plan allocates is owned by one DevBuf member and freed with the plan.  Tables built on first
+  // use (kronrow, sfpp, sf3pp, the pattern) are complete when non-empty and never move: kron_cache keeps pointers into kronrow.
+  struct AxisTables {
+    pc::DevBuf<double> value, weight, point, detJac;
+    pc::DevBuf<int> offset, W, lo, simple;
+    pc::DevBuf<uint32_t> seg;
+    pc::DevBuf<int> rowG, first, own, box_ls, box_lw;
+    pc::DevBuf<double> kronrow;   // 1-D global banded matrices [4][nnp][kMaxW] of the separable path, then mv, lsum, rsum, nsup
+    pc::DevBuf<double> sfpp;      // pair-product tables of the sum-factorised kernel
+    pc::DevBuf<double> sf3pp;     // the same products in the fragment layout of the third-generation kernel
+  } d_ax[3];
+  pc::DevAxis dax[3];             // kernel view of d_ax[d]
+  pc::DevBuf<int> d_localrow;
+  pc::DevBuf<int> d_staterow;     // collocation plans: ghost box -> state row (Layout::staterow)
+  pc::DevBuf<int64_t> d_rowbase;
+  pc::DevBuf<int> d_rank_start;
+  pc::DevBuf<double> d_solve_work;    // pc_solve.cu: r, z, p, Ap, 1/diag, reduction partials, scalars
+  pc::DevBuf<double> d_solve_xfull;   // full-length operand of a distributed matrix-vector product
+  pc::DevBuf<double> d_gmres_work;    // pc_solve.cu GMRES: Krylov basis, w, z, 1/diag, partials, Hessenberg, rotations
+  pc::DevBuf<double> d_sf3_dprime;    // D'[element][pair][64] of the geometry pre-pass (mapped geometry)
 
   // pattern (owned by the plan), per block mode
-  int* d_rowptr[2] = {nullptr, nullptr};
-  int* d_colidx[2] = {nullptr, nullptr};
+  pc::DevBuf<int> d_rowptr[2];
+  pc::DevBuf<int> d_colidx[2];
 
   // geometry / bc / state
-  double* d_X = nullptr;
-  double* d_W = nullptr;
-  double* d_fixtable = nullptr;
-  double* d_bnd_value[3][2] = {{nullptr, nullptr}, {nullptr, nullptr}, {nullptr, nullptr}};   // IGABasis.bnd_value on the device
+  pc::DevBuf<double> d_X;
+  pc::DevBuf<double> d_W;
+  pc::DevBuf<double> d_fixtable;
+  pc::DevBuf<double> d_bnd_value[3][2];   // IGABasis.bnd_value on the device
   double bnd_point[3][2] = {{0, 0}, {0, 0}, {0, 0}};
   int visit[3][2] = {{0, 0}, {0, 0}, {0, 0}};            // IGASetBoundaryForm flags
-  double* d_face_dS[3][2] = {{nullptr, nullptr}, {nullptr, nullptr}, {nullptr, nullptr}};   // BoundaryArea factors of mapped faces with loads
+  pc::DevBuf<double> d_face_dS[3][2];     // BoundaryArea factors of mapped faces with loads
   long face_version[3][2] = {{-1, -1}, {-1, -1}, {-1, -1}};
   petiga_cuda_bc bc;
   bool has_bc = false;
   // unified local buffers (multi-rank) and exchange staging
-  double* d_ghost_values = nullptr; size_t ghost_values_cap = 0;
-  double* d_rhs_loc = nullptr;     // [nloc*dof]
-  double* d_U_loc = nullptr;       // [nloc*dof] (collocation: [nstate*dof])
-  double* d_V_loc = nullptr;
-  double* d_W_loc = nullptr;
-  double* d_recv = nullptr; size_t recv_cap = 0;
-  int* d_recv_rows = nullptr;      // concatenated recv row lists (collocation: the state_recv lists)
-  int64_t* d_recv_off = nullptr;   // same indexing: block offset of each listed row inside its peer's slab
+  pc::DevBuf<double> d_ghost_values;
+  pc::DevBuf<double> d_rhs_loc;   // [nloc*dof]
+  pc::DevBuf<double> d_U_loc;     // [nloc*dof] (collocation: [nstate*dof])
+  pc::DevBuf<double> d_V_loc;
+  pc::DevBuf<double> d_W_loc;
+  pc::DevBuf<double> d_recv;
+  pc::DevBuf<int> d_recv_rows;        // concatenated recv row lists (collocation: the state_recv lists)
+  pc::DevBuf<int64_t> d_recv_off;     // same indexing: block offset of each listed row inside its peer's slab
   std::vector<size_t> recv_row_off;
-  // host staging for *_host entry points
-  double* h_pinned = nullptr; size_t h_pinned_cap = 0;
-  double* d_values_own = nullptr; size_t values_own_cap = 0;   // device arrays used by compute_host
-  double* d_rhs_own = nullptr;
-  double* d_U_own = nullptr;
-  double* d_V_own = nullptr;
-  double* d_scalar = nullptr; size_t scalar_cap = 0;   // [0,8): result, then per-CTA partials of compute_scalar
+  pc::DevBuf<double> d_values_own;   // device arrays used by compute_host
+  pc::DevBuf<double> d_rhs_own;
+  pc::DevBuf<double> d_U_own;
+  pc::DevBuf<double> d_V_own;
+  pc::DevBuf<double> d_scalar;       // [0,8): result, then per-CTA partials of compute_scalar
 
   struct Slot { int form = -1; double prm[pc::kMaxPrm] = {0}; } slots[PETIGA_NSLOTS];
   int path = PETIGA_PATH_AUTO;
@@ -97,15 +150,8 @@ struct petiga_cuda_plan {
 };
 
 namespace pc {
-void set_error(const std::string& msg);
 void nvtx_push(int slot);   // NVTX range named after the IGACompute* driver the slot stands for (no-op without libnvToolsExt)
 void nvtx_pop();
-int cuda_fail(cudaError_t e, const char* what);
-#define PC_CUDA(call)                                              \
-  do {                                                             \
-    cudaError_t _e = (call);                                       \
-    if (_e != cudaSuccess) return pc::cuda_fail(_e, #call);        \
-  } while (0)
 
 // quadrature path (pc_quad.cu)
 int launch_quadrature(petiga_cuda_plan* P, const KParams& base);      // v1: pair loop as one register-tiled contraction

@@ -202,19 +202,18 @@ int launch_sf(petiga_cuda_plan* Pl, const KParams& base, const FormInfo& fi) {
   host_matrix_pattern<DIM, DOF>(base.form, base.slot, base.prm, fi, cpat, ijmask, Cc);
   int rc = build_sf_lists(base, fi, mapped, rational, state, transient, cpat, ijmask, sp.l);
   if (rc) { set_error("sum-factorised kernel: too many components for this form"); return rc; }
-  // per-axis pair-product tables, built once per plan
+  // per-axis pair-product tables, built once per plan (into a local buffer, kept once the build has been launched)
   for (int d = 0; d < 3; d++) {
-    if (!Pl->d_sfpp[d]) {
+    if (!Pl->d_ax[d].sfpp) {
       const size_t n = (size_t)base.ax[d].nel * 9 * base.ax[d].nqp * base.ax[d].nen * base.ax[d].nen;
-      void* buf = nullptr;
-      PC_CUDA(cudaMalloc(&buf, n * sizeof(double)));
-      Pl->allocs.push_back(buf);
-      Pl->d_sfpp[d] = (double*)buf;
-      sf_pp_kernel<<<(int)std::min<size_t>((n + 255) / 256, 4096), 256, 0, Pl->stream>>>(base.ax[d], Pl->d_sfpp[d]);
+      DevBuf<double> pp;
+      if ((rc = pp.reserve(n))) return rc;
+      sf_pp_kernel<<<(int)std::min<size_t>((n + 255) / 256, 4096), 256, 0, Pl->stream>>>(base.ax[d], pp.get());
       PC_CUDA(cudaGetLastError());
       Pl->launches++;
+      Pl->d_ax[d].sfpp = std::move(pp);
     }
-    sp.pp[d] = Pl->d_sfpp[d];
+    sp.pp[d] = Pl->d_ax[d].sfpp.get();
   }
   // identity geometry + constant coefficients: D'[ij][pair] is a constant times JW
   const int NA = base.mc1 - base.mc0;

@@ -105,19 +105,18 @@ int launch_quadrature_sf3(petiga_cuda_plan* Pl, const KParams& base) {
   if (rc) return nope("component lists");
   if (sp.l.NT > 4 || sp.l.npairs > k3MaxPairs || sp.l.ng2 > 4) return nope("too many tensor components");
   sp.vslots = vector_slots(base, sp.l, sp.f4);
-  // per-axis pair-product tables in the fragment layout, once per plan
+  // per-axis pair-product tables in the fragment layout, once per plan (into a local buffer, kept once the build has been launched)
   for (int d = 0; d < 3; d++) {
-    if (!Pl->d_sf3pp[d]) {
+    if (!Pl->d_ax[d].sf3pp) {
       const size_t n = (size_t)base.ax[d].nel * 576;
-      void* buf = nullptr;
-      PC_CUDA(cudaMalloc(&buf, n * sizeof(double)));
-      Pl->allocs.push_back(buf);
-      Pl->d_sf3pp[d] = (double*)buf;
-      sf3_pp_kernel<<<(int)std::min<size_t>((n + 255) / 256, 4096), 256, 0, Pl->stream>>>(base.ax[d], Pl->d_sf3pp[d]);
+      DevBuf<double> pp;
+      if ((rc = pp.reserve(n))) return rc;
+      sf3_pp_kernel<<<(int)std::min<size_t>((n + 255) / 256, 4096), 256, 0, Pl->stream>>>(base.ax[d], pp.get());
       PC_CUDA(cudaGetLastError());
       Pl->launches++;
+      Pl->d_ax[d].sf3pp = std::move(pp);
     }
-    sp.pp[d] = Pl->d_sf3pp[d];
+    sp.pp[d] = Pl->d_ax[d].sf3pp.get();
   }
   sp.const_dp = 0;
   if (!mapped && NA > 0) {   // identity geometry: D'[pair] = JW * C[phys(s)][phys(t)]
@@ -148,13 +147,8 @@ int launch_quadrature_sf3(petiga_cuda_plan* Pl, const KParams& base) {
   if (base.nelem <= 0) return 0;
   if (mapped && sp.want_mat) {   // D' scratch of the geometry pre-pass: [local element][pair][64]
     const size_t need = (size_t)base.nelem * sp.l.npairs * 64;
-    if (Pl->sf3_dprime_cap < need) {
-      cudaFree(Pl->d_sf3_dprime);
-      Pl->d_sf3_dprime = nullptr; Pl->sf3_dprime_cap = 0;
-      PC_CUDA(cudaMalloc(&Pl->d_sf3_dprime, need * sizeof(double)));
-      Pl->sf3_dprime_cap = need;
-    }
-    sp.dprime = Pl->d_sf3_dprime;
+    if ((rc = Pl->d_sf3_dprime.reserve(need))) return rc;
+    sp.dprime = Pl->d_sf3_dprime.get();
   }
   const dim3 ggrid((unsigned)base.ax[0].ew, (unsigned)base.ax[1].ew, (unsigned)base.ax[2].ew);
   if (base.ax[1].ew > 65535 || base.ax[2].ew > 65535) return nope("element box too large for a 3-D grid");

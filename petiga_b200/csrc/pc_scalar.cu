@@ -330,25 +330,20 @@ extern "C" int petiga_cuda_compute_scalar(petiga_cuda_plan* P, int scalar_id, co
   PC_CUDA(cudaSetDevice(P->device));
   const double* U_k = U;
   if (L.nranks > 1 && U) {   // IGAGetLocalVecArray: G2L halo (petigavec.c:256-269)
-    int rc = halo_state(P, L.send, L.recv, U, P->d_U_loc);
+    int rc = halo_state(P, L.send, L.recv, U, P->d_U_loc.get());
     if (rc) return rc;
-    U_k = P->d_U_loc;
+    U_k = P->d_U_loc.get();
   }
   for (int d = 0; d < 3; d++) sp.ax[d] = P->dax[d];
   sp.dim = L.dim; sp.dof = L.dof; sp.nelem = L.ax[0].ew * L.ax[1].ew * L.ax[2].ew;
-  sp.localrow = P->d_localrow; sp.U = U_k; sp.X = P->d_X; sp.Wt = P->d_W;
+  sp.localrow = P->d_localrow.get(); sp.U = U_k; sp.X = P->d_X.get(); sp.Wt = P->d_W.get();
   sp.sid = scalar_id; sp.n = n; sp.kmax = kmax;
   const int nen = (L.ax[0].p + 1) * (L.ax[1].p + 1) * (L.ax[2].p + 1);
   const size_t smem = (size_t)nen * (L.dof + L.dim + 1) * sizeof(double);
   if (smem > 200 * 1024) { set_error("compute_scalar: element does not fit shared memory"); return PETIGA_CUDA_ERR_SUP; }
   const int blocks = std::max(1, std::min(sp.nelem, P->num_sms * 8));
-  if (P->scalar_cap < (size_t)(blocks + 1) * kMaxS) {
-    cudaFree(P->d_scalar);
-    P->d_scalar = nullptr; P->scalar_cap = 0;
-    PC_CUDA(cudaMalloc(&P->d_scalar, (size_t)(blocks + 1) * kMaxS * sizeof(double)));
-    P->scalar_cap = (size_t)(blocks + 1) * kMaxS;
-  }
-  sp.partial = P->d_scalar + kMaxS;
+  if (int rc = P->d_scalar.reserve((size_t)(blocks + 1) * kMaxS)) return rc;
+  sp.partial = P->d_scalar.get() + kMaxS;
   cudaEventRecord(P->ev0, P->stream);
 #define SK(DIM_)                                                                                                        \
   if (L.dim == DIM_) {                                                                                                  \
@@ -358,14 +353,14 @@ extern "C" int petiga_cuda_compute_scalar(petiga_cuda_plan* P, int scalar_id, co
   SK(1) SK(2) SK(3)
 #undef SK
   PC_CUDA(cudaGetLastError());
-  scalar_reduce_kernel<<<n, 32, 0, P->stream>>>(sp.partial, blocks, n, P->d_scalar);
+  scalar_reduce_kernel<<<n, 32, 0, P->stream>>>(sp.partial, blocks, n, P->d_scalar.get());
   PC_CUDA(cudaGetLastError());
   P->launches += 2;
   cudaEventRecord(P->ev1, P->stream);
   if (L.nranks > 1) {   // MPI_Allreduce(localS, S, n, SUM) (petigacomp.c:90)
-    int rc = allreduce_sum(P, P->d_scalar, n);
+    int rc = allreduce_sum(P, P->d_scalar.get(), n);
     if (rc) return rc;
   }
-  PC_CUDA(cudaMemcpyAsync(S_host, P->d_scalar, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, P->stream));
+  PC_CUDA(cudaMemcpyAsync(S_host, P->d_scalar.get(), (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, P->stream));
   return petiga_cuda_finish(P);
 }

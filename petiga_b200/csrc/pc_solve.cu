@@ -267,15 +267,11 @@ int full_operand(petiga_cuda_plan* P, const double* x_owned, const double** xful
   const Layout& L = P->L;
   if (L.nranks == 1) { *xfull = x_owned; return 0; }
   const size_t ntot = (size_t)L.rank_start[L.nranks] * L.dof;
-  if (P->solve_xfull_cap < ntot) {
-    cudaFree(P->d_solve_xfull);
-    P->d_solve_xfull = nullptr; P->solve_xfull_cap = 0;
-    PC_CUDA(cudaMalloc(&P->d_solve_xfull, ntot * sizeof(double)));
-    P->solve_xfull_cap = ntot;
-  }
-  int rc = allgather_owned(P, x_owned, P->d_solve_xfull);
+  int rc = P->d_solve_xfull.reserve(ntot);
   if (rc) return rc;
-  *xfull = P->d_solve_xfull;
+  rc = allgather_owned(P, x_owned, P->d_solve_xfull.get());
+  if (rc) return rc;
+  *xfull = P->d_solve_xfull.get();
   return 0;
 }
 
@@ -325,13 +321,8 @@ extern "C" int petiga_cuda_solve_cg(petiga_cuda_plan* P, int block, const double
   const int n = pt.nrows * pt.bs;                       // owned scalar rows
   // work vectors r, z, p, Ap, dinv + partials + scalars, kept with the plan
   const size_t need = (size_t)5 * std::max(n, 1) + 4 * kDotBlocks + 16;
-  if (P->solve_work_cap < need) {
-    cudaFree(P->d_solve_work);
-    P->d_solve_work = nullptr; P->solve_work_cap = 0;
-    PC_CUDA(cudaMalloc(&P->d_solve_work, need * sizeof(double)));
-    P->solve_work_cap = need;
-  }
-  double *r = P->d_solve_work, *z = r + n, *p = z + n, *Ap = p + n, *dinv = Ap + n, *part = dinv + n, *s = part + 4 * kDotBlocks;
+  if ((rc = P->d_solve_work.reserve(need))) return rc;
+  double *r = P->d_solve_work.get(), *z = r + n, *p = z + n, *Ap = p + n, *dinv = Ap + n, *part = dinv + n, *s = part + 4 * kDotBlocks;
   cudaStream_t st = P->stream;
   const int gb = std::max(1, std::min((n + 255) / 256, kDotBlocks));
   const bool multi = L.nranks > 1;
@@ -403,13 +394,8 @@ extern "C" int petiga_cuda_solve_gmres(petiga_cuda_plan* P, int block, const dou
   // basis V[m+1], w, z, 1/diag, partials [npass*32][blocks], H[m][m+1], cs, sn, g, y, h, state; kept with the plan
   const size_t nsmall = (size_t)m * (m + 1) + 2 * (size_t)m + 2 * (size_t)(m + 1) + (size_t)npass * kc + kStateLen;
   const size_t need = (size_t)(m + 4) * ld + (size_t)npass * kc * kDotBlocks + nsmall;
-  if (P->gmres_work_cap < need) {
-    cudaFree(P->d_gmres_work);
-    P->d_gmres_work = nullptr; P->gmres_work_cap = 0;
-    PC_CUDA(cudaMalloc(&P->d_gmres_work, need * sizeof(double)));
-    P->gmres_work_cap = need;
-  }
-  double *V = P->d_gmres_work, *w = V + (size_t)(m + 1) * ld, *z = w + ld, *dinv = z + ld, *part = dinv + ld;
+  if ((rc = P->d_gmres_work.reserve(need))) return rc;
+  double *V = P->d_gmres_work.get(), *w = V + (size_t)(m + 1) * ld, *z = w + ld, *dinv = z + ld, *part = dinv + ld;
   double *H = part + (size_t)npass * kc * kDotBlocks, *cs = H + (size_t)m * (m + 1), *sn = cs + m, *g = sn + m, *y = g + m + 1;
   double *hd = y + m + 1, *st = hd + (size_t)npass * kc;
   cudaStream_t s = P->stream;
